@@ -3,14 +3,22 @@
 factor-edge evaluations / s and variable samples / s per sweep).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workloads c2,c4,c3] [--blocks R]
+                    [--workloads c2,c4,c3] [--dump-outputs DIR]
 
 Headline workload (``value``, ``e2e``, ``roofline``): BASELINE config 2, the
 4096 x 4096 Boolean Ising grid with EQUAL pairwise factors, inference only; a
-"step" is one full chromatic Gibbs sweep (every colour once).  The timed block
-of K steps is repeated R times back to back (each bracketed by CUDA events on
-the library's stream, barrier + synchronize on both sides) and the MEDIAN block
-is reported -- one 3.6 ms block is too fragile a sample.
+"step" is one full chromatic Gibbs sweep (every colour once).  After W warm-up
+steps the K timed steps run back to back in one call of the library, bracketed
+by CUDA events on its stream (barrier + synchronize on both sides).  Every
+workload times exactly K of its steps; the ``e2e`` calls through the public API
+that follow are timed separately, min(max(K, 3), 10) of them.
+
+``--dump-outputs DIR`` writes what the timed steps computed, as a caller of
+that path receives it, to ``DIR/<name>.npy`` (float32 / float64): the sampled
+values and the marginals of the K timed sweeps (``c2_*``, ``c4_*``) and the
+learned weights (``learn_weights``).  Per-variable arrays hold a fixed, seeded
+sample of DUMP_SAMPLE variables.  The inputs depend on the arguments alone, so
+two builds run with the same arguments can be compared output for output.
 
 With N = 1 two more blocks ride in the same JSON line:
   ``c4``     BASELINE config 4 at full size (200 M Boolean variables / 1 B edges,
@@ -50,6 +58,7 @@ GRID = int(os.environ.get("NB_BENCH_GRID", 4096))          # rows per GPU and co
 CPU_GRID = int(os.environ.get("NB_BENCH_CPU_GRID", 1024))   # bounded sample for the cpu_baseline leg
 C4_VARS = int(os.environ.get("NB_BENCH_C4_VARS", 200_000_000))
 C3_COPIES = int(os.environ.get("NB_BENCH_C3_COPIES", 1_000_000))
+DUMP_SAMPLE = 1 << 20                                       # variables per dumped array (<= 8 MB each)
 METRIC = "factor_edge_evals_per_sec"
 UNIT = "factor-edge evals/s"
 SEED = 20261017
@@ -109,6 +118,7 @@ class ClockSampler(object):
         self.rows, self.stop = [], False
         self.index = index
         self.t = threading.Thread(target=self._run, daemon=True)
+        self.first = threading.Event()
 
     def _run(self):
         while not self.stop:
@@ -120,10 +130,14 @@ class ClockSampler(object):
                     self.rows.append([x.strip() for x in out.split(",")])
             except Exception:
                 pass
+            self.first.set()
             time.sleep(0.1)
 
     def __enter__(self):
+        # the first query's Python start-up holds the GIL: waiting for it keeps the main thread from
+        # stalling between the timer's start event and the launches that follow
         self.t.start()
+        self.first.wait(timeout=10)
         return self
 
     def __exit__(self, *a):
@@ -177,7 +191,7 @@ def _ref_ising_arrays(n, m, types, coupling=0.1):
 def _import_reference():
     ref = os.path.join(REPO, "baseline", "_ref")
     if not os.path.isdir(os.path.join(ref, "numbskull")):
-        raise RuntimeError("baseline/_ref is missing: run baseline/install_ref.sh where /root/reference exists")
+        raise RuntimeError("baseline/_ref is missing: run baseline/install_ref.sh <numbskull source checkout>")
     sys.path[:0] = [ref, os.path.join(REPO, "baseline", "shims")]
     import numbskull
     assert os.path.abspath(numbskull.__file__).startswith(ref), numbskull.__file__
@@ -269,8 +283,8 @@ def run_reference(args):
     try:
         r = reference_throughput(steps, warmup, grid=args.ref_grid or None)
     except Exception as exc:  # noqa: BLE001
-        # no baseline/_ref on this box (it is installed where /root/reference exists and travels with the
-        # snapshot): the oracle port always exists -- the C restatement of gibbsthread, all host threads
+        # no baseline/_ref here (baseline/install_ref.sh installs it from a numbskull checkout): the oracle
+        # port always exists -- the C restatement of gibbsthread, all host threads
         try:
             grid = args.ref_grid or 2048
             r = cpu_port_throughput(steps, warmup, grid=grid)
@@ -380,23 +394,44 @@ class Dev(object):
         self.L.nb_launch_count(self.g, C.byref(n))
         return n.value
 
-    def timed_blocks(self, fn, steps, blocks):
-        """`blocks` back-to-back blocks of `steps` steps; per block: barrier + sync, CUDA events on
-        the launching stream, max over ranks.  Returns the per-block milliseconds."""
-        out = []
-        for _ in range(blocks):
-            self.barrier()
-            self.lib.check(self.L.nb_timer_start(self.g))
-            fn(steps)
-            ms = C.c_float(0)
-            self.lib.check(self.L.nb_timer_stop(self.g, C.byref(ms)))
-            self.barrier()
-            out.append(self.max_over_ranks(ms.value))
-        return out
+    def timed(self, fn, steps):
+        """fn(steps) between CUDA events on the launching stream, barrier + sync on both sides;
+        milliseconds, max over ranks."""
+        self.barrier()
+        self.lib.check(self.L.nb_timer_start(self.g))
+        fn(steps)
+        ms = C.c_float(0)
+        self.lib.check(self.L.nb_timer_stop(self.g, C.byref(ms)))
+        self.barrier()
+        return self.max_over_ranks(ms.value)
+
+    def state(self, prefix, n_vars, epochs, seed):
+        """The chain-0 values and the marginals (tallies / epochs) of a seeded sample of the first
+        n_vars variables, as a caller of FactorGraph.inference receives them (Boolean variables:
+        one tally each)."""
+        fg = self.fg
+        vals = np.empty(len(fg.variable), np.int64)
+        self.lib.check(self.L.nb_get_var_values(self.g, 0, self.lib.ptr(vals)))
+        marg = np.empty(int(fg.cstart[-1]), np.float64)
+        self.lib.check(self.L.nb_get_marginals(self.g, self.lib.ptr(marg), float(epochs)))
+        if n_vars > DUMP_SAMPLE:
+            ids = np.sort(np.random.default_rng(seed).choice(n_vars, DUMP_SAMPLE, replace=False))
+        else:
+            ids = np.arange(n_vars)
+        return {prefix + "var_value": vals[ids].astype(np.float32), prefix + "marginals": marg[fg.cstart[ids]]}
 
 
-def block_c4(args, local_rank):
-    """BASELINE config 4 at full size on one GPU."""
+def write_dump(out_dir, arrays):
+    """DIR/<name>.npy for every array (float32 / float64, 64 MB at most in all)."""
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def block_c4(args, local_rank, dump):
+    """BASELINE config 4 at full size on one GPU; its outputs go into `dump` unless it is None."""
     import numbskull_b200 as nb
     from numbskull_b200 import _lib, synth
     t0 = time.perf_counter()
@@ -418,19 +453,22 @@ def block_c4(args, local_rank):
     bytes_sweep = 16.0 * nvar + float((ar * (20 + 5 * ar)).sum())
     del ar
     L = dev.L
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
 
     def sweeps(n):
         _lib.check(L.nb_gibbs_sweeps(dev.g, n, 0, 1, fg.seed))
     sweeps(3)
+    _lib.check(L.nb_reset_counts(dev.g))        # the marginals of the timed sweeps alone
     import torch
     rt = torch.cuda.cudart()
     l0 = dev.launches()
     rt.cudaProfilerStart()
-    ms = dev.timed_blocks(sweeps, steps, 3)
+    ms = dev.timed(sweeps, steps)
     rt.cudaProfilerStop()
     l1 = dev.launches()
-    med = float(np.median(ms)) / steps
+    if dump is not None:
+        dump.update(dev.state("c4_", nvar, steps, 4))
+    per_step = ms / steps
     bad = C.c_int64(-1)
     _lib.check(L.nb_graph_check_coloring(dev.g, C.byref(bad)))
     _lib.check(L.nb_reset_counts(dev.g))
@@ -440,13 +478,13 @@ def block_c4(args, local_rank):
     e2e_ms = 1e3 * (time.perf_counter() - t4)
     out = {"workload": "kbc_%d_vars_%d_edges_mixed_istrue_imply_and_or_inference (BASELINE config 4%s)"
                        % (nvar, edges, "" if C4_VARS == 200_000_000 else ", scaled"),
-           "metric": METRIC, "value": edges / (med * 1e-3), "unit": UNIT, "ms_per_step": med,
-           "var_samples_per_sec": nvar / (med * 1e-3), "steps": steps, "timed_blocks_ms": ms,
+           "metric": METRIC, "value": edges / (per_step * 1e-3), "unit": UNIT, "ms_per_step": per_step,
+           "var_samples_per_sec": nvar / (per_step * 1e-3), "steps": steps, "timed_ms": ms,
            "variables": nvar, "factor_edge_evals_per_sweep": edges, "colors": int(info["n_colors"]),
            "color_conflicts": int(bad.value), "device_GB": round(info["device_bytes"] / 1e9, 2),
            "gpu_launches": int(l1 - l0),
            "rows": {"pair": int(info["n_pair_rows"]), "fast": int(info["n_fast_rows"]), "warp": int(info["n_warp_rows"])},
-           "roofline": roofline(bytes_sweep, med, "k_gibbs_tt (FAST rows: 16-byte truth-table quads with the weight "
+           "roofline": roofline(bytes_sweep, per_step, "k_gibbs_tt (FAST rows: 16-byte truth-table quads with the weight "
                                 "inlined, member gathers from the bit-packed value mirror; one launch per colour; "
                                 "traffic = all launches of one sweep)", "k_gibbs_tt_c4_bytes_per_sweep"),
            "e2e_first_call_ms": e2e_ms, "mean_marginal": float(m.mean()),
@@ -456,9 +494,9 @@ def block_c4(args, local_rank):
     return out
 
 
-def block_learn(args, local_rank):
+def block_learn(args, local_rank, dump):
     """BASELINE config 3 shape: weight learning on the labelling-function model (L1, learn_non_evidence,
-    step 1e-4 as test_lf_learning.py:129-137)."""
+    step 1e-4 as test_lf_learning.py:129-137); the learned weights go into `dump` unless it is None."""
     import numbskull_b200 as nb
     from numbskull_b200 import _lib, synth
     n_lf = 100
@@ -488,18 +526,20 @@ def block_learn(args, local_rank):
     rt = torch.cuda.cudart()
     l0 = dev.launches()
     rt.cudaProfilerStart()
-    ms = dev.timed_blocks(epochs, 3, 3)
+    ms = dev.timed(epochs, args.steps)
     rt.cudaProfilerStop()
     l1 = dev.launches()
-    med = float(np.median(ms)) / 3
+    per_step = ms / args.steps
     fg._stale.add("weight_value")
     w = fg.weight_value[0]
+    if dump is not None:
+        dump["learn_weights"] = w.copy()
     out = {"workload": "lf_model_%dx%d_learning_L1_learn_non_evidence_step1e-4 (BASELINE config 3 shape, %s of its size)"
                        % (copies, n_lf, "%.0f%%" % (100.0 * copies / 1e7)),
-           "metric": METRIC, "value": edges / (med * 1e-3), "unit": UNIT, "ms_per_step": med, "step": "one learning epoch",
-           "timed_blocks_ms": ms, "variables": int(len(fg.variable)), "factor_edge_evals_per_epoch": int(edges),
-           "gpu_launches_per_epoch": (l1 - l0) / 9.0,
-           "roofline": roofline(b_learn, med, "learning epoch (both chains + gradient reduction by weight id)",
+           "metric": METRIC, "value": edges / (per_step * 1e-3), "unit": UNIT, "ms_per_step": per_step, "step": "one learning epoch",
+           "steps": args.steps, "timed_ms": ms, "variables": int(len(fg.variable)),
+           "factor_edge_evals_per_epoch": int(edges), "gpu_launches_per_epoch": (l1 - l0) / args.steps,
+           "roofline": roofline(b_learn, per_step, "learning epoch (both chains + gradient reduction by weight id)",
                                 "learn_c3_bytes_per_epoch"),
            "weights_head": [round(float(x), 4) for x in w[:6]], "weights_finite": bool(np.isfinite(w).all())}
     fg.clear()
@@ -526,11 +566,11 @@ def block_c4_strong(args, rank, world, local_rank):
     dev = Dev(fg, world)
     fg._sync_device(0, 0, evid=False)
     run.sweeps(2, True, True)
-    steps = max(3, min(args.steps, 10))
-    ms = dev.timed_blocks(lambda n: run.sweeps(n, False, True), steps, 3)
+    steps = args.steps
+    ms = dev.timed(lambda n: run.sweeps(n, False, True), steps)
     if run.p2p:
         _lib.check(dev.L.nb_p2p_check(dev.g))
-    med = float(np.median(ms)) / steps
+    per_step = ms / steps
     tot = torch.tensor([float(fg.color_edges().sum()), float(run.n_owned), float(n_ghost), float(run.halo_bytes_per_sweep),
                         t1 - t0, t2 - t1], device="cuda", dtype=torch.float64)
     mx = tot.clone()
@@ -541,8 +581,8 @@ def block_c4_strong(args, rank, world, local_rank):
         edges = tot[0].item()
         out = {"workload": "kbc_%d_vars_%d_edges_block_partitioned_over_%d_gpus (BASELINE config 4, strong scaling)"
                            % (C4_VARS, int(edges), world),
-               "metric": METRIC, "value": edges / (med * 1e-3), "unit": UNIT, "ms_per_step": med, "scaling": "strong",
-               "steps": steps, "timed_blocks_ms": ms, "colors": run.n_colors, "phases_per_sweep": run.n_phases,
+               "metric": METRIC, "value": edges / (per_step * 1e-3), "unit": UNIT, "ms_per_step": per_step, "scaling": "strong",
+               "steps": steps, "timed_ms": ms, "colors": run.n_colors, "phases_per_sweep": run.n_phases,
                "ghost_copies_total": int(tot[2].item()), "ghost_copies_per_owned_variable": tot[2].item() / max(tot[1].item(), 1),
                "halo_values_per_sweep_total": int(tot[3].item()), "halo_values_per_sweep_max_rank": int(mx[3].item()),
                "transport": "NVLink peer stores + in-kernel flag barrier" if run.p2p else "NCCL point-to-point",
@@ -603,8 +643,9 @@ def run_ours(args):
     if not torch.cuda.is_available():
         raise RuntimeError("bench.py needs a CUDA device (no CPU fallback); use --impl reference for the CPU arm")
     L = _lib.lib()
-    steps, warmup, blocks = max(1, args.steps), max(3, args.warmup), max(1, args.blocks)
+    steps, warmup = args.steps, max(3, args.warmup)
     workloads = [w for w in args.workloads.split(",") if w]
+    dump = None if args.dump_outputs is None else {}
 
     identical = None
     if world > 1:
@@ -630,30 +671,33 @@ def run_ours(args):
     if world == 1:
         assert edges == info["n_edges"], (edges, info["n_edges"])
 
-    def sweeps(n):
+    def sweeps(n, burnin=False):
         if runner is None:
-            _lib.check(L.nb_gibbs_sweeps(g, n, 0, 1, fg.seed))
+            _lib.check(L.nb_gibbs_sweeps(g, n, int(burnin), 1, fg.seed))
         else:
-            runner.sweeps(n, burnin=False, sample_evidence=True)
+            runner.sweeps(n, burnin=burnin, sample_evidence=True)
 
     fg._sync_device(0, 0)
-    sweeps(warmup)
-    dev.barrier()
+    _lib.check(L.nb_reset_counts(g))
     # `ncu --profile-from-start off` then lists exactly the launches of the timed region and of the
     # end-to-end steps (no-ops without a profiler)
     cudart = torch.cuda.cudart()
     with ClockSampler(local_rank) as clocks:
+        # warm-up right before the timed sweeps, as burn-in: the marginals are those of the timed sweeps
+        sweeps(warmup, burnin=True)
+        dev.barrier()
         l0 = dev.launches()
         cudart.cudaProfilerStart()
         t0 = time.perf_counter()
-        block_ms = dev.timed_blocks(sweeps, steps, blocks)
+        dev_ms = dev.timed(sweeps, steps)
         wall = time.perf_counter() - t0
         cudart.cudaProfilerStop()
         l1 = dev.launches()
-        dev_ms = float(np.median(block_ms))
+        if dump is not None and rank == 0:     # rank 0's own strip when partitioned
+            dump.update(dev.state("c2_", len(fg.variable) if runner is None else runner.n_owned, steps, 2))
         # keep the GPUs busy a little longer so that the sampler sees clocks under load
         # (same count on every rank: it is derived from the rank-agreed dev_ms)
-        if sum(block_ms) < 1500:
+        if dev_ms < 1500:
             sweeps(max(1, int(steps * 1500 / max(dev_ms, 1e-3)) // 4))
             dev.barrier()
 
@@ -712,12 +756,12 @@ def run_ours(args):
         del dev
         if "c4" in workloads:
             try:
-                c4 = block_c4(args, local_rank)
+                c4 = block_c4(args, local_rank, dump)
             except Exception as exc:  # noqa: BLE001
                 c4 = {"unavailable": "%s: %s" % (type(exc).__name__, exc)}
         if "c3" in workloads:
             try:
-                learn = block_learn(args, local_rank)
+                learn = block_learn(args, local_rank, dump)
             except Exception as exc:  # noqa: BLE001
                 learn = {"unavailable": "%s: %s" % (type(exc).__name__, exc)}
 
@@ -754,10 +798,10 @@ def run_ours(args):
                    "partition": "single GPU" if world == 1 else
                    ("row strips; per colour a boundary phase + NVLink halo push on a side stream, concurrent with "
                     "the interior phase" if runner.p2p and runner.split else "row strips, per-colour halo exchange")},
-        "timed_blocks": blocks, "timed_blocks_ms": block_ms, "block_statistic": "median",
+        "timed_ms": dev_ms,
         "var_samples_per_sec": total_vars * steps / (dev_ms * 1e-3),
         "roofline": roofline(bytes_sweep, ms_per_step, "k_gibbs_tt2 (PAIR rows, uniform slices: 4-byte records; one launch "
-                             "per colour; duration = CUDA-event time of the median block / sweeps)",
+                             "per colour; duration = CUDA-event time of the timed sweeps / sweeps)",
                              "k_gibbs_tt2_bytes_per_sweep"),
         "gpu_launches": int(l1 - l0),
         "clocks": clocks.summary(),
@@ -780,7 +824,15 @@ def run_ours(args):
         line["cpu_baseline"] = cpu_baselines()
         if learn is not None and "unavailable" not in learn:
             learn["cpu_baseline"] = reference_child("learn")       # the reference's learnthread on the same model shape
+    missing = []
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
+        # a workload that failed wrote nothing: say so, rather than leave a comparison of fewer outputs
+        missing = [name for name, blk in (("c4", c4), ("learn", learn)) if blk is not None and "unavailable" in blk]
+        line["dump_outputs"] = {"dir": args.dump_outputs, "arrays": sorted(dump), "missing_workloads": missing}
     OUT.emit(json.dumps(line))
+    if missing:
+        sys.exit("--dump-outputs: no outputs of %s (the workload failed, see the JSON line)" % ", ".join(missing))
     if world > 1:
         import torch.distributed as dist
         dist.barrier()
@@ -812,9 +864,8 @@ def main():
     OUT = _QuietStdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every workload")
     ap.add_argument("--warmup", type=int, default=5)
-    ap.add_argument("--blocks", type=int, default=7, help="timed blocks of --steps steps (median reported)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workloads", default=os.environ.get("NB_BENCH_WORKLOADS", "c2,c4,c3"),
                     help="N = 1 only: extra blocks next to the c2 headline")
@@ -822,7 +873,12 @@ def main():
     ap.add_argument("--ref-mode", default="inference", choices=["inference", "single", "learn"],
                     help="reference arm: the headline inference line, or a bounded single-thread / learning sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the timed steps to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,12 +1,12 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in this directory from the REAL reference.
 
-Run in the build container only (needs /root/reference and numba):
+Needs a source checkout of HazyResearch/numbskull and numba:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <numbskull checkout>
 
 The reference package is copied to a temp dir (its ``@jit(cache=True)``
-functions write next to their sources and /root/reference is read-only), the
+functions write next to their sources, and the checkout may be read-only), the
 missing ``past.builtins`` module is shimmed, and the unmodified numba functions
 are called.  Nothing from the reference is stored in the repo -- only the
 arrays it computes.  ``nthreads=1`` plus a jitted ``np.random.seed /
@@ -31,7 +31,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, REPO)
 
-REF = "/root/reference"
+if len(sys.argv) != 2 or not os.path.isdir(os.path.join(sys.argv[1], "numbskull")):
+    sys.exit("usage: python tests/golden/make_golden.py <numbskull checkout>")
+REF = sys.argv[1]
 tmp = tempfile.mkdtemp(prefix="nbref_")
 shutil.copytree(os.path.join(REF, "numbskull"), os.path.join(tmp, "numbskull"))
 os.makedirs(os.path.join(tmp, "past"))

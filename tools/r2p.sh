@@ -10,10 +10,10 @@ timeout 900 python bench.py > $out/${tag}_bench_n1.json 2> $out/${tag}_bench_n1.
 timeout 600 python bench.py --impl reference > $out/${tag}_bench_reference.json 2> $out/${tag}_bench_reference.err
 # launch list of the timed regions (bench.py brackets them with cudaProfilerStart/Stop)
 timeout 900 $NCU --profile-from-start off --metrics gpu__time_duration.sum -c 4000 --csv \
-    --log-file $out/${tag}_launches_bench_steps2.csv python bench.py --steps 2 --warmup 3 --blocks 1 --no-cpu-baseline > /dev/null 2>&1
+    --log-file $out/${tag}_launches_bench_steps2.csv python bench.py --steps 2 --warmup 3 --no-cpu-baseline > /dev/null 2>&1
 # C2: the two colours of one sweep, full set
 timeout 300 $NCU --profile-from-start off --set full --import-source on -k regex:k_gibbs_tt2 -c 2 -f -o $out/${tag}_tt2 \
-    python bench.py --steps 2 --warmup 3 --blocks 1 --workloads c2 --no-cpu-baseline > /dev/null 2>&1
+    python bench.py --steps 2 --warmup 3 --workloads c2 --no-cpu-baseline > /dev/null 2>&1
 ncu -i $out/${tag}_tt2.ncu-rep --page raw --csv > $out/${tag}_gibbs_tt2_ncu_full.csv 2> /dev/null
 # C4 at the full 200 M variables / 1 B edges: DRAM bytes and time of every launch of one sweep (single pass: no replay backup of 89 GB)
 timeout 600 $NCU --profile-from-start off --metrics dram__bytes_read.sum,dram__bytes_write.sum,gpu__time_duration.sum -k regex:k_gibbs -c 80 --csv \
