@@ -82,6 +82,7 @@ typedef struct {
     int64_t max_arity;                 /* largest factor arity (the natural-order colouring is only tried when <= 2) */
     int64_t n_pair_rows, n_fast_rows, n_cat_rows;   /* padded id ranges of the record row classes */
     int64_t tt_quads, tt2_quads;       /* 16-byte quads in the FAST / PAIR record streams   */
+    int32_t value_bytes;               /* device value width: 1 (every cardinality <= 255) or 2 */
 } nb_graph_info;
 
 const char *nb_last_error(void);

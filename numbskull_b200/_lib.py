@@ -42,6 +42,7 @@ class GraphInfo(C.Structure):
         ("device_bytes", C.c_int64), ("count_entries", C.c_int64), ("jp_rounds", C.c_int64),
         ("max_arity", C.c_int64), ("n_pair_rows", C.c_int64), ("n_fast_rows", C.c_int64),
         ("n_cat_rows", C.c_int64), ("tt_quads", C.c_int64), ("tt2_quads", C.c_int64),
+        ("value_bytes", C.c_int32),
     ]
 
     def as_dict(self):

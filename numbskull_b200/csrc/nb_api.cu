@@ -73,6 +73,7 @@ extern "C" int nb_graph_get_info(const nb_graph *g, nb_graph_info *info)
     info->device_bytes = g->device_bytes; info->count_entries = g->count_entries; info->jp_rounds = g->jp_rounds;
     info->max_arity = g->max_arity; info->n_pair_rows = g->n_prows; info->n_fast_rows = g->n_frows - g->n_prows;
     info->n_cat_rows = g->n_crows - g->n_frows; info->tt_quads = g->n_tt_quads; info->tt2_quads = g->n_tt2_quads;
+    info->value_bytes = g->value_bytes;
     return NB_OK;
 }
 
@@ -96,8 +97,8 @@ extern "C" int nb_graph_color_edges(const nb_graph *g, int64_t *edges_per_color)
 //
 // The caller's arrays keep the reference's types (int64 values and counts,
 // float64 weights).  They are narrowed / widened on the host by a few threads
-// next to pinned staging buffers, so only 1 byte per variable and 4 bytes per
-// count entry cross PCIe.
+// next to pinned staging buffers, so only 1 byte per variable (2 on graphs with
+// cardinalities above 255) and 4 bytes per count entry cross PCIe.
 // ---------------------------------------------------------------------------
 // The host conversion runs chunk by chunk on a few threads and overlaps with the PCIe copies:
 // uploads are copied as soon as a chunk is narrowed, downloads are widened as soon as the chunk's
@@ -242,20 +243,40 @@ static int download_chunks(nb_graph *g, const void *d_src, int64_t n, int elem)
 // An out-of-range value is an error for an evidence variable; for a variable that is sampled
 // anyway (or a ghost, refreshed by its owner) the reference simply overwrites it at the first
 // sample (load_domains leaves a raw initialValue that is not in the explicit domain): mapped to 0.
-__global__ void k_scatter_values_u8(int64_t V, const uint8_t *in, const int32_t *old2new, const int32_t *v_card,
-                                    const int8_t *v_evid, nb_val_t *val, int *bad)
+// (T = the graph's value element type; the staged values have the same width)
+template <class T>
+__global__ void k_scatter_values(int64_t V, const T *in, const int32_t *old2new, const int32_t *v_card,
+                                 const int8_t *v_evid, T *val, int *bad)
 {
     int64_t v = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (v >= V) return;
     int x = in[v];
     if (x >= v_card[v]) { if (v_evid[v] == 1) *bad = 1; x = 0; }
-    val[old2new[v]] = (nb_val_t)x;
+    val[old2new[v]] = (T)x;
 }
 
-__global__ void k_gather_values_u8(int64_t V, const nb_val_t *val, const int32_t *old2new, uint8_t *out)
+template <class T>
+__global__ void k_gather_values(int64_t V, const T *val, const int32_t *old2new, T *out)
 {
     int64_t v = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (v < V) out[v] = val[old2new[v]];
+}
+
+// Narrow to the value width on the host: anything outside [0, max value] becomes the largest
+// value, which is >= every cardinality of the graph, so the device judges it out of range.
+template <class T>
+static int stage_values(nb_graph *g, const int64_t *values)
+{
+    const int64_t V = g->V;
+    const int64_t top = (int64_t)(T)~(T)0;   // 255 / 65535
+    T *stage = (T *)g->h_pinned;
+    return host_chunks(g, V, [&](int64_t, int64_t a, int64_t b) {
+        for (int64_t i = a; i < b; i++) {
+            int64_t x = values[i];
+            stage[i] = (x < 0 || x > top) ? (T)top : (T)x;
+        }
+        return cudaMemcpyAsync((T *)g->d_xfer + a, stage + a, (size_t)(b - a) * sizeof(T), cudaMemcpyHostToDevice, g->stream);
+    });
 }
 
 extern "C" int nb_set_var_values(nb_graph *g, int chain, const int64_t *values)
@@ -265,28 +286,22 @@ extern "C" int nb_set_var_values(nb_graph *g, int chain, const int64_t *values)
     NB_CUDA(cudaSetDevice(g->device));
     const int64_t V = g->V;
     if (V == 0) return NB_OK;
-    NB_TRY(nb_ensure_pinned(g, (size_t)V + 64));
-    NB_TRY(nb_ensure_xfer(g, (size_t)V + 64));
-    uint8_t *stage = (uint8_t *)g->h_pinned;
-    std::atomic<int> out_of_range(0);
-    int rc = host_chunks(g, V, [&](int64_t, int64_t a, int64_t b) {
-        int bad = 0;
-        for (int64_t i = a; i < b; i++) {
-            int64_t x = values[i];
-            stage[i] = (x < 0 || x > NB_MAX_CARD) ? (uint8_t)NB_MAX_CARD : (uint8_t)x;   // 255 >= every cardinality: judged on the device
-        }
-        (void)bad;
-        return cudaMemcpyAsync((uint8_t *)g->d_xfer + a, stage + a, (size_t)(b - a), cudaMemcpyHostToDevice, g->stream);
-    });
-    if (rc != NB_OK || out_of_range.load()) {
+    const size_t vb = (size_t)g->value_bytes;
+    NB_TRY(nb_ensure_pinned(g, (size_t)V * vb + 64));
+    NB_TRY(nb_ensure_xfer(g, (size_t)V * vb + 64));
+    int rc = vb == 1 ? stage_values<nb_val_t>(g, values) : stage_values<nb_val16_t>(g, values);
+    if (rc != NB_OK) {
         cudaStreamSynchronize(g->stream);
-        if (rc != NB_OK) return rc;
-        NB_FAIL(NB_ERR_INVALID, "var_value holds entries outside [0, cardinality)");
+        return rc;
     }
-    int *d_bad = (int *)((char *)g->d_xfer + (((size_t)V + 15) & ~(size_t)15));
+    int *d_bad = (int *)((char *)g->d_xfer + (((size_t)V * vb + 15) & ~(size_t)15));
     NB_CUDA(cudaMemsetAsync(d_bad, 0, 4, g->stream));
-    k_scatter_values_u8<<<grid_for(V), 256, 0, g->stream>>>(V, (const uint8_t *)g->d_xfer, g->d_old2new, g->d_v_card,
-                                                            g->d_v_evid, g->d_val[chain], d_bad);
+    if (vb == 1)
+        k_scatter_values<<<grid_for(V), 256, 0, g->stream>>>(V, (const nb_val_t *)g->d_xfer, g->d_old2new, g->d_v_card,
+                                                             g->d_v_evid, nb_vals<nb_val_t>(g, chain), d_bad);
+    else
+        k_scatter_values<<<grid_for(V), 256, 0, g->stream>>>(V, (const nb_val16_t *)g->d_xfer, g->d_old2new, g->d_v_card,
+                                                             g->d_v_evid, nb_vals<nb_val16_t>(g, chain), d_bad);
     int bad = 0;
     NB_CUDA(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, g->stream));
     NB_CUDA(cudaStreamSynchronize(g->stream));
@@ -301,15 +316,24 @@ extern "C" int nb_get_var_values(nb_graph *g, int chain, int64_t *values)
     NB_CUDA(cudaSetDevice(g->device));
     const int64_t V = g->V;
     if (V == 0) return NB_OK;
-    NB_TRY(nb_ensure_pinned(g, (size_t)V + 64));
-    NB_TRY(nb_ensure_xfer(g, (size_t)V + 64));
-    k_gather_values_u8<<<grid_for(V), 256, 0, g->stream>>>(V, g->d_val[chain], g->d_old2new, (uint8_t *)g->d_xfer);
-    int rc = download_chunks(g, g->d_xfer, V, 1);
+    const int vb = g->value_bytes;
+    NB_TRY(nb_ensure_pinned(g, (size_t)V * vb + 64));
+    NB_TRY(nb_ensure_xfer(g, (size_t)V * vb + 64));
+    if (vb == 1)
+        k_gather_values<<<grid_for(V), 256, 0, g->stream>>>(V, nb_vals<nb_val_t>(g, chain), g->d_old2new, (nb_val_t *)g->d_xfer);
+    else
+        k_gather_values<<<grid_for(V), 256, 0, g->stream>>>(V, nb_vals<nb_val16_t>(g, chain), g->d_old2new, (nb_val16_t *)g->d_xfer);
+    int rc = download_chunks(g, g->d_xfer, V, vb);
     if (rc != NB_OK) { cudaStreamSynchronize(g->stream); return rc; }
-    const uint8_t *stage = (const uint8_t *)g->h_pinned;
     rc = host_chunks(g, V, [&](int64_t k, int64_t a, int64_t b) {
         cudaError_t e = cudaEventSynchronize(g->xfer_events[(size_t)k]);
         if (e != cudaSuccess) return e;
+        if (vb == 2) {
+            const nb_val16_t *stage16 = (const nb_val16_t *)g->h_pinned;
+            for (int64_t i = a; i < b; i++) values[i] = (int64_t)stage16[i];
+            return cudaSuccess;
+        }
+        const uint8_t *stage = (const uint8_t *)g->h_pinned;
 #if NB_HAVE_AVX2_PATH
         if (nb_use_nt()) { widen_u8_nt(stage, values, a, b); return cudaSuccess; }
 #endif
@@ -691,9 +715,10 @@ __global__ void k_scatter_u8(int64_t n, const int32_t *ids, const int32_t *old2n
 extern "C" int nb_gather_values_dev(nb_graph *g, int chain, const int32_t *dev_local_ids, int64_t n, uint8_t *dev_out)
 {
     if (chain < 0 || chain > 1) NB_FAIL(NB_ERR_INVALID, "chain must be 0 or 1");
+    if (g->value_bytes != 1) NB_FAIL(NB_ERR_UNSUPPORTED, "byte-valued halo transfers need a graph whose cardinalities are all <= 255");
     if (n == 0) return NB_OK;
     NB_CUDA(cudaSetDevice(g->device));
-    k_gather_u8<<<grid_for(n), 256, 0, g->stream>>>(n, dev_local_ids, g->d_old2new, g->d_val[chain], dev_out);
+    k_gather_u8<<<grid_for(n), 256, 0, g->stream>>>(n, dev_local_ids, g->d_old2new, nb_vals<nb_val_t>(g, chain), dev_out);
     g->launches++;
     NB_CUDA(cudaGetLastError());
     return NB_OK;
@@ -702,9 +727,10 @@ extern "C" int nb_gather_values_dev(nb_graph *g, int chain, const int32_t *dev_l
 extern "C" int nb_scatter_values_dev(nb_graph *g, int chain, const int32_t *dev_local_ids, int64_t n, const uint8_t *dev_in)
 {
     if (chain < 0 || chain > 1) NB_FAIL(NB_ERR_INVALID, "chain must be 0 or 1");
+    if (g->value_bytes != 1) NB_FAIL(NB_ERR_UNSUPPORTED, "byte-valued halo transfers need a graph whose cardinalities are all <= 255");
     if (n == 0) return NB_OK;
     NB_CUDA(cudaSetDevice(g->device));
-    k_scatter_u8<<<grid_for(n), 256, 0, g->stream>>>(n, dev_local_ids, g->d_old2new, g->d_val[chain], dev_in);
+    k_scatter_u8<<<grid_for(n), 256, 0, g->stream>>>(n, dev_local_ids, g->d_old2new, nb_vals<nb_val_t>(g, chain), dev_in);
     g->launches++;
     NB_CUDA(cudaGetLastError());
     return NB_OK;

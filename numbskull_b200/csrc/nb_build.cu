@@ -99,6 +99,7 @@ struct RawGraph {
     const int32_t *m_eq;
     const int64_t *gid;
     bool wide;
+    bool val16;     // 2-byte value graph (some cardinality above 255)
 };
 
 __device__ __forceinline__ int nbuckets(const RawGraph &G, int64_t v) { return G.v_dtype[v] == 0 ? 1 : G.v_card[v]; }
@@ -124,6 +125,11 @@ __global__ void k_row_size(RawGraph G, uint32_t *rowlen, uint32_t *ninc, uint8_t
             int code = G.f_code[f], a = G.f_arity[f];
             words += nb_incidence_words(G.wide, code, a, G.f_feat[f] != 1.0);
             if (catok) catok = (code == C_AND_CAT || code == C_EQUAL_CAT_CONST) && a <= 3 && G.f_feat[f] == 1.0;
+            // the records hold the other members' dense_equal_to in 8 bits; on a 2-byte graph a member
+            // value of 255 or more would compare against a truncated one: such rows stay generic
+            if (catok && G.val16)
+                for (int j = 0; j < a; j++)
+                    catok &= G.m_vid[G.f_off[f] + j] == v || (uint32_t)G.m_eq[G.f_off[f] + j] <= 0xFFu;
             if (ok) {   // truth-table class: arity <= 3, integer-valued function, small member domains
                 if (!nb_code_tt_ok(code) || a > 3 || G.f_feat[f] != 1.0) ok = false;
                 else if (!nb_code_tt_const_compare(code))
@@ -302,12 +308,14 @@ __global__ void k_sort_keys(int64_t V, const int32_t *color, const int8_t *v_evi
     if (!ghost) atomicAdd(&color_edges[c], (unsigned long long)ninc[v]);
 }
 
-// sorted position -> new id, plus all per-variable arrays in the new order
+// sorted position -> new id, plus all per-variable arrays in the new order (T: value element type;
+// vcard: cardinalities of a 2-byte graph, whose vmeta card field is 0 above 255)
+template <class T>
 __global__ void k_assign_ids(int64_t V, const uint64_t *keys, const int32_t *sorted_ids, int n_colors,
                              const int64_t *group_start, const int64_t *group_base, RawGraph G,
                              const int32_t *v_init, const uint32_t *rowlen, const uint8_t *fast, int32_t *old2new,
-                             int32_t *new2old, uint32_t *vmeta, uint32_t *rowlen_new, nb_val_t *vinit,
-                             uint32_t *rng_id, nb_val_t *val0, nb_val_t *val1)
+                             int32_t *new2old, uint32_t *vmeta, uint32_t *rowlen_new, T *vinit,
+                             uint32_t *rng_id, T *val0, T *val1, uint16_t *vcard)
 {
     int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= V) return;
@@ -319,9 +327,11 @@ __global__ void k_assign_ids(int64_t V, const uint64_t *keys, const int32_t *sor
     int v = sorted_ids[i];
     old2new[v] = (int32_t)nid;
     new2old[nid] = v;
-    vmeta[nid] = nb_pack_meta(G.v_card[v], G.v_evid[v], G.v_dtype[v], 1, cls <= NB_CLASS_FAST, rowlen[v]);
+    const int card = G.v_card[v];
+    vmeta[nid] = nb_pack_meta(card <= NB_MAX_CARD ? card : 0, G.v_evid[v], G.v_dtype[v], 1, cls <= NB_CLASS_FAST, rowlen[v]);
+    if (vcard) vcard[nid] = (uint16_t)card;
     rowlen_new[nid] = rowlen[v];
-    nb_val_t init = (nb_val_t)v_init[v];
+    T init = (T)v_init[v];
     vinit[nid] = init;
     val0[nid] = init;
     val1[nid] = init;
@@ -344,12 +354,13 @@ __global__ void k_window_starts(int64_t V, const uint64_t *keys, int n_colors, c
     win_start[(size_t)g * (size_t)(n_win + 1) + (size_t)w] = (int32_t)(group_base[g] + (i - group_start[g]));
 }
 
-__global__ void k_count_entries(int64_t Vn, const uint32_t *vmeta, uint32_t *entries)
+template <class T>
+__global__ void k_count_entries(int64_t Vn, const uint32_t *vmeta, const uint16_t *vcard, uint32_t *entries)
 {
     int64_t n = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (n >= Vn) return;
     uint32_t m = vmeta[n];
-    int card = NB_META_CARD(m);
+    int card = NbCardOf<T>(vcard).card(m, (uint32_t)n);
     entries[n] = NB_META_VALID(m) ? (card == 2 ? 1u : (uint32_t)card) : 0u;
 }
 
@@ -677,6 +688,7 @@ static RawGraph raw_view(const nb_graph *g)
     G.b_off = g->d_b_off; G.b_len = g->d_b_len; G.fi = g->d_fi;
     G.f_code = g->d_f_code; G.f_wid = g->d_f_wid; G.f_feat = g->d_f_feat; G.f_arity = g->d_f_arity;
     G.f_off = g->d_f_off; G.m_vid = g->d_m_vid; G.m_eq = g->d_m_eq; G.gid = g->d_gid; G.wide = g->wide;
+    G.val16 = g->value_bytes == 2;
     return G;
 }
 
@@ -722,7 +734,7 @@ static int extract_and_upload(nb_graph *g, const nb_graph_desc *d)
             for (int64_t i = a; i < b; i++) {
                 const nb_variable_rec &r = d->variable[i];
                 if (r.dataType != 0 && r.dataType != 1) { fail("variable dataType must be 0 or 1", i); continue; }
-                if (r.cardinality < 1 || r.cardinality > NB_MAX_CARD) { fail("variable cardinality outside [1, 255]", i); continue; }
+                if (r.cardinality < 1 || r.cardinality > NB_MAX_CARD_WIDE) { fail("variable cardinality outside [1, 65535]", i); continue; }
                 // the reference accepts such graphs: a sampled variable's value is overwritten at its first
                 // sample (load_domains can leave a raw initialValue that is not in the domain)
                 const bool init_ok = r.initialValue >= 0 && r.initialValue < r.cardinality;
@@ -833,6 +845,7 @@ static int extract_and_upload(nb_graph *g, const nb_graph_desc *d)
 
     g->n_edges = edges.load();
     g->max_card = maxcard.load();
+    g->value_bytes = g->max_card > NB_MAX_CARD ? 2 : 1;   // 1-byte values unless some cardinality needs 2
     g->max_arity = maxarity.load();
     g->any_categorical = need_eq;
     g->wide = (W > (int64_t)NB_COMPACT_MAX_WID + 1) || (maxarity.load() > NB_COMPACT_MAX_ARITY);
@@ -1154,15 +1167,24 @@ int nb_build_finalize(nb_graph *g)
     NB_TRY(nb_alloc(g, &g->d_vmeta, (size_t)Vn));
     uint32_t *d_rowlen_new;
     NB_TRY(nb_alloc(g, &d_rowlen_new, (size_t)Vn));
-    NB_TRY(nb_alloc(g, &g->d_vinit, (size_t)Vn));
+    NB_TRY(nb_dev_alloc(g, &g->d_vinit, (size_t)Vn * g->value_bytes, true));
     NB_TRY(nb_alloc(g, &g->d_rng_id, (size_t)Vn));
     // both chains in one allocation: one L2 access-policy window covers them (nb_set_l2_policy)
     g->val_stride = ((size_t)Vn + 255) & ~(size_t)255;
-    NB_TRY(nb_alloc(g, &g->d_val[0], 2 * g->val_stride));
-    g->d_val[1] = g->d_val[0] + g->val_stride;
-    k_assign_ids<<<grid_for(V), 256, 0, g->stream>>>(V, d_keys_sorted, d_ids_sorted, nc, d_gstart, d_gbase, G,
-                                                     g->d_v_init, d_rowlen, d_fast, g->d_old2new, g->d_new2old, g->d_vmeta,
-                                                     d_rowlen_new, g->d_vinit, g->d_rng_id, g->d_val[0], g->d_val[1]);
+    NB_TRY(nb_dev_alloc(g, &g->d_val[0], 2 * g->val_stride * g->value_bytes, true));
+    g->d_val[1] = (char *)g->d_val[0] + g->val_stride * g->value_bytes;
+    if (g->value_bytes == 1) {
+        k_assign_ids<<<grid_for(V), 256, 0, g->stream>>>(V, d_keys_sorted, d_ids_sorted, nc, d_gstart, d_gbase, G,
+                                                         g->d_v_init, d_rowlen, d_fast, g->d_old2new, g->d_new2old, g->d_vmeta,
+                                                         d_rowlen_new, (nb_val_t *)g->d_vinit, g->d_rng_id, nb_vals<nb_val_t>(g, 0),
+                                                         nb_vals<nb_val_t>(g, 1), (uint16_t *)nullptr);
+    } else {
+        NB_TRY(nb_alloc(g, &g->d_vcard, (size_t)Vn));
+        k_assign_ids<<<grid_for(V), 256, 0, g->stream>>>(V, d_keys_sorted, d_ids_sorted, nc, d_gstart, d_gbase, G,
+                                                         g->d_v_init, d_rowlen, d_fast, g->d_old2new, g->d_new2old, g->d_vmeta,
+                                                         d_rowlen_new, (nb_val16_t *)g->d_vinit, g->d_rng_id,
+                                                         nb_vals<nb_val16_t>(g, 0), nb_vals<nb_val16_t>(g, 1), g->d_vcard);
+    }
 
     // ---- id windows of every (class, colour) group: learning walks the graph window by window ----
     {
@@ -1191,7 +1213,8 @@ int nb_build_finalize(nb_graph *g)
         uint32_t *d_entries;
         NB_TRY(nb_alloc(g, &d_entries, (size_t)Vn + 1));
         NB_TRY(nb_alloc(g, &g->d_cstart, (size_t)Vn + 1));
-        k_count_entries<<<grid_for(Vn), 256, 0, g->stream>>>(Vn, g->d_vmeta, d_entries);
+        if (g->value_bytes == 1) k_count_entries<nb_val_t><<<grid_for(Vn), 256, 0, g->stream>>>(Vn, g->d_vmeta, nullptr, d_entries);
+        else k_count_entries<nb_val16_t><<<grid_for(Vn), 256, 0, g->stream>>>(Vn, g->d_vmeta, g->d_vcard, d_entries);
         NB_TRY(exclusive_scan(g, d_entries, g->d_cstart, Vn + 1));
         int64_t *d_entries_old;
         NB_TRY(nb_alloc(g, &d_entries_old, (size_t)V + 1));
@@ -1255,7 +1278,9 @@ int nb_build_finalize(nb_graph *g)
         }
         task_ptr[(size_t)nw] = (int64_t)task_row.size();
         g->n_wtasks = (int64_t)task_row.size();
-        g->wpart_stride = g->max_card > 4 ? ((g->max_card + 3) & ~3) : 4;
+        // (rows above NB_MAX_CARD -- 2-byte graphs -- write no task partials: nb_warp_sample_wide)
+        const int part_card = std::min(g->max_card, NB_MAX_CARD);
+        g->wpart_stride = part_card > 4 ? ((part_card + 3) & ~3) : 4;
         NB_TRY(upload(g, &g->d_wtask_row, task_row));
         NB_TRY(upload(g, &g->d_wtask_beg, task_beg));
         NB_TRY(upload(g, &g->d_wtask_ptr, task_ptr));
@@ -1374,7 +1399,7 @@ void nb_set_l2_policy(nb_graph *g, cudaStream_t stream)
     cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)max_persist);
     cudaStreamAttrValue attr;
     memset(&attr, 0, sizeof(attr));
-    const size_t bytes = std::min<size_t>(2 * g->val_stride, (size_t)max_window);
+    const size_t bytes = std::min<size_t>(2 * g->val_stride * g->value_bytes, (size_t)max_window);
     attr.accessPolicyWindow.base_ptr = g->d_val[0];
     attr.accessPolicyWindow.num_bytes = bytes;
     attr.accessPolicyWindow.hitRatio = (float)std::min(1.0, 0.9 * (double)max_persist / (double)std::max<size_t>(bytes, 1));

@@ -132,7 +132,9 @@ __host__ __device__ inline int nb_incidence_words(bool wide, int code, int arity
 }
 
 // vmeta word per (new) variable id: card:8 | isEvidence:4 | dataType:1 | valid:1 | fast:1 | row words:17
-// (row words saturate at 2^17-1; warp-path rows take their length from wrow_ptr)
+// (row words saturate at 2^17-1; warp-path rows take their length from wrow_ptr).  card = 0 marks a
+// cardinality above 255 (2-byte graphs only): the real one is in nb_graph::d_vcard.  Device code
+// reads cardinalities through NbCardOf (nb_eval.cuh), never NB_META_CARD directly.
 #define NB_META_CARD(m) ((int)((m) & 0xFFu))
 #define NB_META_EVID(m) ((int)(((m) >> 8) & 0xFu))
 #define NB_META_DTYPE(m) ((int)(((m) >> 12) & 1u))
@@ -168,8 +170,13 @@ __host__ __device__ inline uint32_t nb_pack_meta(int card, int evid, int dtype, 
    back (230 us per colour on the KBC hubs, a tenth of the sweep) */
 #define NB_WARP_TASK 64
 
-typedef uint8_t nb_val_t;  // variable values on the device (cardinality <= 255)
-#define NB_MAX_CARD 255
+// Variable values on the device.  The element width is a property of the graph, chosen at build
+// time (nb_graph::value_bytes): 1 byte when every cardinality is <= 255 (nb_val_t), 2 bytes up to
+// 65535 (nb_val16_t).  Kernels that read or write values are instantiated for both.
+typedef uint8_t nb_val_t;
+typedef uint16_t nb_val16_t;
+#define NB_MAX_CARD 255          /* largest cardinality of a 1-byte graph (and of the vmeta card field) */
+#define NB_MAX_CARD_WIDE 65535   /* largest cardinality of a 2-byte graph */
 
 // ----------------------------------------------------------------------------
 // device graph
@@ -267,7 +274,8 @@ struct nb_graph {
 
     // ---- per new-id variable data ----
     uint32_t *d_vmeta = nullptr;     // [Vn] packed meta incl. row length
-    nb_val_t *d_vinit = nullptr;     // [Vn]
+    void *d_vinit = nullptr;         // [Vn] value_bytes each
+    uint16_t *d_vcard = nullptr;     // [Vn] cardinalities of 2-byte graphs (nullptr on 1-byte graphs)
     uint32_t *d_cstart = nullptr;    // [Vn + 1] new-order count layout
     int64_t *d_cstart_old = nullptr; // [V + 1] reference count layout
 
@@ -309,8 +317,9 @@ struct nb_graph {
     int wpart_stride = 4;
 
     // ---- state ----
-    nb_val_t *d_val[2] = {nullptr, nullptr};  // [Vn] chain 0 = free, 1 = evidence (one allocation, val_stride apart)
+    void *d_val[2] = {nullptr, nullptr};  // [Vn] chain 0 = free, 1 = evidence (one allocation, val_stride elements apart)
     size_t val_stride = 0;
+    int value_bytes = 1;             // element width of d_val / d_vinit: 1 (nb_val_t) or 2 (nb_val16_t)
     int64_t l2_persist_bytes = 0;    // bytes of the value arrays pinned in the persisting part of L2
     int32_t *d_count = nullptr;      // [count_entries] new-order layout
     double *d_weight = nullptr;      // [W]
@@ -342,6 +351,10 @@ struct nb_graph {
     std::vector<NbColorRange> colors;
     std::vector<void *> allocs;
 };
+
+// the value arrays with their element type (T = nb_val_t on 1-byte graphs, nb_val16_t on 2-byte ones)
+template <class T>
+inline T *nb_vals(const nb_graph *g, int chain) { return (T *)g->d_val[chain]; }
 
 // device allocation tracked by the graph
 int nb_dev_alloc(nb_graph *g, void **p, size_t bytes, bool zero);

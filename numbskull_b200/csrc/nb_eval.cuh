@@ -146,8 +146,32 @@ __device__ __forceinline__ double nb_read_feature(const NbRow &r, const NbHdr &h
 // Where member values come from.  The sweeps read the chain's value array; the table builders
 // (nb_build.cu) force the values of the (at most two) other members of an incidence, so that the
 // truth tables of the record streams are tabulated by THIS evaluator and nothing else.
-struct NbValsGlobal {
-    const nb_val_t *__restrict__ v;
+//
+// The accessors are templates on the element type of the value array (nb_val_t or nb_val16_t) and
+// also answer the cardinality of a variable (NbCardOf): on 1-byte graphs that is the card field of
+// its vmeta word and the accessor is a bare pointer, as before; on 2-byte graphs a card field of 0
+// sends the lookup to nb_graph::d_vcard.  SweepArgs / LearnArgs derive from it too: on 1-byte
+// graphs it is an empty base, so their layout (and the kernels' code) is what it was before.
+template <class T>
+struct NbCardOf {
+    __host__ __device__ __forceinline__ NbCardOf(const uint16_t * = nullptr) {}
+    __device__ __forceinline__ int card(uint32_t meta, uint32_t) const { return NB_META_CARD(meta); }
+};
+template <>
+struct NbCardOf<nb_val16_t> {
+    const uint16_t *vcard;
+    __host__ __device__ __forceinline__ NbCardOf(const uint16_t *c = nullptr) : vcard(c) {}
+    __device__ __forceinline__ int card(uint32_t meta, uint32_t id) const
+    {
+        const int c = NB_META_CARD(meta);
+        return c ? c : (int)__ldg(vcard + id);
+    }
+};
+
+template <class T>
+struct NbValsGlobal : NbCardOf<T> {
+    const T *__restrict__ v;
+    __device__ __forceinline__ NbValsGlobal(const T *v_, const NbCardOf<T> &cards = NbCardOf<T>()) : NbCardOf<T>(cards), v(v_) {}
     __device__ __forceinline__ int operator()(uint32_t vid) const { return (int)v[vid]; }
 };
 // Same for the persistent learning kernel, which reads values other CTAs wrote earlier in the same
@@ -156,8 +180,10 @@ struct NbValsGlobal {
 // barrier, whose fence invalidates the SM's L1 (CCTL.IVALL) before anybody reads again.  Bypassing
 // L1 altogether (ld.global.cg) cost the categorical rows a factor of four: their samplers re-read
 // the same few neighbours for every candidate value.
-struct NbValsCG {
-    const nb_val_t *v;
+template <class T>
+struct NbValsCG : NbCardOf<T> {
+    const T *v;
+    __device__ __forceinline__ NbValsCG(const T *v_, const NbCardOf<T> &cards = NbCardOf<T>()) : NbCardOf<T>(cards), v(v_) {}
     __device__ __forceinline__ int operator()(uint32_t vid) const { return (int)__ldca(v + vid); }
 };
 // weight accessors: global (read-only for the launch), global through L2, or a shared-memory copy
@@ -318,10 +344,11 @@ __device__ NB_EVAL_FN double nb_eval_incidence_v(const NbRow &r, const NbHdr &h,
     }
 }
 
+template <class T>
 __device__ __forceinline__ double nb_eval_incidence(const NbRow &r, const NbHdr &h, int mpos, uint32_t self,
-                                                    int k, const nb_val_t *__restrict__ vals)
+                                                    int k, const T *__restrict__ vals)
 {
-    return nb_eval_incidence_v(r, h, mpos, self, k, NbValsGlobal{vals});
+    return nb_eval_incidence_v(r, h, mpos, self, k, NbValsGlobal<T>(vals));
 }
 
 // position of the first member word of the incidence whose header is at `pos`
@@ -391,12 +418,12 @@ __device__ __forceinline__ double nb_row_energy_k_v(const NbRow &r, int len, uin
     return e;
 }
 
-template <bool WIDE>
+template <bool WIDE, class T>
 __device__ __forceinline__ double nb_row_energy_k(const NbRow &r, int len, uint32_t self, int k,
-                                                  const nb_val_t *__restrict__ vals,
+                                                  const T *__restrict__ vals,
                                                   const double *__restrict__ weight)
 {
-    return nb_row_energy_k_v<WIDE>(r, len, self, k, NbValsGlobal{vals}, NbWtsGlobal{weight});
+    return nb_row_energy_k_v<WIDE>(r, len, self, k, NbValsGlobal<T>(vals), NbWtsGlobal{weight});
 }
 
 // j-th value (ascending) of a categorical row that has no bucket marker
@@ -443,7 +470,7 @@ template <bool WIDE, class Vals, class Wts>
 __device__ NB_EVAL_FN int nb_sample_row_v(const NbRow &r, int len, uint32_t self, uint32_t meta,
                                             const Vals &vals, const Wts &weight, NbUniforms &rng)
 {
-    const int card = NB_META_CARD(meta);
+    const int card = vals.card(meta, self);
     if (NB_META_DTYPE(meta) == 0) {
         if (card <= 4) {
             double e[4] = {0.0, 0.0, 0.0, 0.0};
@@ -480,12 +507,12 @@ __device__ NB_EVAL_FN int nb_sample_row_v(const NbRow &r, int len, uint32_t self
     return res.pick;
 }
 
-template <bool WIDE>
+template <bool WIDE, class T>
 __device__ inline int nb_sample_row(const NbRow &r, int len, uint32_t self, uint32_t meta,
-                                    const nb_val_t *__restrict__ vals, const double *__restrict__ weight,
+                                    const T *__restrict__ vals, const NbCardOf<T> &cards, const double *__restrict__ weight,
                                     NbUniforms &rng)
 {
-    return nb_sample_row_v<WIDE>(r, len, self, meta, NbValsGlobal{vals}, NbWtsGlobal{weight}, rng);
+    return nb_sample_row_v<WIDE>(r, len, self, meta, NbValsGlobal<T>(vals, cards), NbWtsGlobal{weight}, rng);
 }
 
 
@@ -494,6 +521,67 @@ __device__ __forceinline__ double nb_warp_sum(double x)
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xFFFFFFFFu, x, o);
     return x;
+}
+
+// Sample a warp row whose cardinality is above 255 (2-byte graphs), one warp, every lane returns
+// the same value.  Such a row's per-value energies do not fit the warp's shared array (and a task
+// partial of card doubles per task would scale with n_tasks x card), so the row is sampled from its
+// incidences directly and needs no memory beyond the row itself:
+//   dataType 1: the incidences are in bucket order, i.e. ascending value order.  The lanes evaluate
+//     32 consecutive incidences at a time; the energies are then folded in incidence order into one
+//     sum per value (shuffles, identical on every lane), and each finished value enters the
+//     reservoir, followed by the single group of empty buckets -- nb_sample_row_v's semantics.
+//   dataType 0: every incidence contributes to every value: one warp reduction per value.
+template <bool WIDE, class Vals, class Wts>
+__device__ NB_EVAL_FN int nb_warp_sample_wide(const NbRow &r, int len, const uint2 *__restrict__ inc, int n_inc,
+                                                uint32_t self, uint32_t meta, int card, const Vals &vals,
+                                                const Wts &weight, NbUniforms &rng)
+{
+    const int lane = threadIdx.x & 31;
+    NbReservoir res;
+    if (NB_META_DTYPE(meta) == 0) {
+        for (int k = 0; k < card; k++) {
+            double e = 0.0;
+            for (int i = lane; i < n_inc; i += 32) {
+                const int pos = (int)inc[i].x;
+                const NbHdr h = nb_read_hdr<WIDE>(r, pos);
+                e += weight(h.wid) * nb_eval_incidence_v(r, h, nb_member_pos<WIDE>(h, pos), self, k, vals);
+            }
+            if (res.add(nb_warp_sum(e), 1.0, rng.next32())) res.pick = k;
+        }
+        return res.pick;
+    }
+    int cur = -1, nonempty = 0;
+    double e = 0.0;
+    for (int base = 0; base < n_inc; base += 32) {
+        int k = -1;
+        double x = 0.0;
+        if (base + lane < n_inc) {
+            const uint2 ent = inc[base + lane];
+            const NbHdr h = nb_read_hdr<WIDE>(r, (int)ent.x);
+            k = (int)ent.y;
+            x = weight(h.wid) * nb_eval_incidence_v(r, h, nb_member_pos<WIDE>(h, (int)ent.x), self, k, vals);
+        }
+        const int m = min(32, n_inc - base);
+        for (int j = 0; j < m; j++) {
+            const int kj = __shfl_sync(0xFFFFFFFFu, k, j);
+            const double xj = __shfl_sync(0xFFFFFFFFu, x, j);
+            if (kj != cur) {
+                if (cur >= 0 && res.add(e, 1.0, rng.next32())) res.pick = cur;
+                cur = kj;
+                e = 0.0;
+                nonempty++;
+            }
+            e += xj;
+        }
+    }
+    if (cur >= 0 && res.add(e, 1.0, rng.next32())) res.pick = cur;
+    const int n_empty = card - nonempty;
+    if (n_empty > 0 && res.add(0.0, (double)n_empty, rng.next32())) {
+        const int j = min(n_empty - 1, (int)(rng.next32() * (double)n_empty));
+        res.pick = nb_nth_empty_value<WIDE>(r, len, j);
+    }
+    return res.pick;
 }
 
 
@@ -593,8 +681,9 @@ __device__ inline NbHdr nb_tabulate(const NbRow &r, int pos, uint32_t self, uint
 #define NB_TT_UNROLL_DEFAULT 4
 // where the record kernels read member values from: the byte array, or (large all-Boolean graphs,
 // see nb_graph::d_valbits) a bit-packed mirror of it that stays L2-resident
+template <class T>
 struct NbValsBytes {
-    const nb_val_t *__restrict__ v;
+    const T *__restrict__ v;
     __device__ __forceinline__ int operator()(uint32_t id) const { return (int)v[id]; }
 };
 struct NbValsBits {
@@ -623,11 +712,11 @@ __device__ __forceinline__ double nb_tt_delta_v(const uint4 *__restrict__ qp, in
     }
     return d;
 }
-template <int NB_TT_UNROLL = NB_TT_UNROLL_DEFAULT>
+template <int NB_TT_UNROLL = NB_TT_UNROLL_DEFAULT, class T>
 __device__ __forceinline__ double nb_tt_delta(const uint4 *__restrict__ qp, int n, uint32_t self,
-                                              const nb_val_t *__restrict__ vals)
+                                              const T *__restrict__ vals)
 {
-    return nb_tt_delta_v<NB_TT_UNROLL>(qp, n, self, NbValsBytes{vals});
+    return nb_tt_delta_v<NB_TT_UNROLL>(qp, n, self, NbValsBytes<T>{vals});
 }
 
 // Pair records (NB_CLASS_PAIR): incidences with at most ONE other member take 8 bytes,
@@ -690,10 +779,11 @@ __device__ __forceinline__ double nb_tt2_delta_v(const uint4 *__restrict__ qp, i
     }
     return d;
 }
+template <class T>
 __device__ __forceinline__ double nb_tt2_delta(const uint4 *__restrict__ qp, int n, uint32_t common, uint32_t self,
-                                               const nb_val_t *__restrict__ vals, const double *__restrict__ weight)
+                                               const T *__restrict__ vals, const double *__restrict__ weight)
 {
-    return nb_tt2_delta_v(qp, n, common, self, NbValsBytes{vals}, weight);
+    return nb_tt2_delta_v(qp, n, common, self, NbValsBytes<T>{vals}, weight);
 }
 
 // Categorical records (NB_CLASS_CAT): one quad per incidence of an AND_CAT / EQUAL_CAT_CONST factor
@@ -702,16 +792,17 @@ __device__ __forceinline__ double nb_tt2_delta(const uint4 *__restrict__ qp, int
 // (like the FAST quads the record inlines the weight VALUE; the ids live in cat_wid for the refresh)
 // The factor is 1 iff every other member equals its dense_equal_to (the variable itself matches by
 // construction of the bucket); n_others == 3 marks "never satisfied" (padding, or the variable
-// occurring twice with different values).
+// occurring twice with different values).  eqA / eqB have 8 bits: on a 2-byte graph a row is a CAT
+// row only if every dense_equal_to it stores is <= 255 (k_row_size); its other members may be wide.
 __host__ __device__ inline uint32_t nb_pack_cat(int k, int eq_a, int eq_b, int n_others, int fixed)
 {
     return (uint32_t)k | ((uint32_t)eq_a << 8) | ((uint32_t)eq_b << 16) | ((uint32_t)n_others << 24) | ((uint32_t)fixed << 26);
 }
 
 // Per-value energies of a CAT row: acc.add(k, w) for every satisfied incidence of bucket k.
-template <class Acc>
+template <class Acc, class T>
 __device__ __forceinline__ void nb_cat_energies(const uint4 *__restrict__ qp, int n, uint32_t self,
-                                                const nb_val_t *__restrict__ vals, Acc &acc)
+                                                const T *__restrict__ vals, Acc &acc)
 {
     for (int j = 0; j < n; j += 2) {
         uint4 q[2];

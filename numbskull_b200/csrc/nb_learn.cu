@@ -35,7 +35,9 @@ namespace cg = cooperative_groups;
 #define NB_GRAD_SHIFT 20
 typedef long long nb_fix_t;
 
-struct LearnArgs {
+// T = element type of the value arrays (nb_val_t or nb_val16_t, see nb_graph::value_bytes)
+template <class T>
+struct LearnArgs : NbCardOf<T> {   // (cardinalities: a.card(meta, nid))
     const uint32_t *vmeta;
     const int64_t *slice_ptr;
     const uint32_t *twords;
@@ -44,9 +46,9 @@ struct LearnArgs {
     const int64_t *inc_ptr;
     const uint2 *inc;
     const uint32_t *rng_id;
-    const nb_val_t *vinit;
-    nb_val_t *val_free;
-    nb_val_t *val_evid;
+    const T *vinit;
+    T *val_free;
+    T *val_evid;
     double *weight;
     const uint8_t *wfixed;
     int64_t n_trows;
@@ -168,7 +170,8 @@ struct CtxWts {
 };
 
 // visit counter increment of one variable (learning.py:90: one truncation draw per variable)
-__device__ __forceinline__ uint32_t nb_cnt_inc(const LearnArgs &a, uint32_t id)
+template <class T>
+__device__ __forceinline__ uint32_t nb_cnt_inc(const LearnArgs<T> &a, uint32_t id)
 {
     if (a.regularization == 1) {
         NbUniforms tr(id, a.epoch, NB_TAG_TRUNC, a.seed);
@@ -178,13 +181,13 @@ __device__ __forceinline__ uint32_t nb_cnt_inc(const LearnArgs &a, uint32_t id)
 }
 
 // second pass over a row: gradient of every visited incidence with a learnable weight
-template <bool WIDE, bool SMEM>
+template <bool WIDE, bool SMEM, class T>
 __device__ NB_EVAL_FN void nb_row_gradient(const NbRow &r, int len, uint32_t self, uint32_t meta, int ev, int prop,
-                                       const LearnArgs &a, uint32_t cnt_inc, const LearnCtx<SMEM> &ctx,
+                                       const LearnArgs<T> &a, uint32_t cnt_inc, const LearnCtx<SMEM> &ctx,
                                        int first_inc, int inc_stride, const uint2 *inc_list, int n_inc)
 {
     const bool cat = NB_META_DTYPE(meta) == 1;
-    const NbValsCG vF{a.val_free}, vE{a.val_evid};
+    const NbValsCG<T> vF(a.val_free), vE(a.val_evid);
     if (inc_list == nullptr) {
         int pos = 0, cur = -1;
         while (pos < len) {
@@ -217,8 +220,8 @@ __device__ NB_EVAL_FN void nb_row_gradient(const NbRow &r, int len, uint32_t sel
 // ---------------------------------------------------------------------------
 // thread path: generic rows (GEN class) and categorical record rows (CAT class), one row per thread
 // ---------------------------------------------------------------------------
-template <bool WIDE, bool SMEM>
-__device__ __noinline__ void learn_thread_rows(const LearnArgs &a, const LearnCtx<SMEM> &ctx, int beg0, int end0, int beg1, int end1)
+template <bool WIDE, bool SMEM, class T>
+__device__ __noinline__ void learn_thread_rows(const LearnArgs<T> &a, const LearnCtx<SMEM> &ctx, int beg0, int end0, int beg1, int end1)
 {
     const int64_t n0 = end0 - beg0, ntot = n0 + (end1 - beg1);
     const CtxWts<SMEM> wts{ctx};
@@ -233,20 +236,21 @@ __device__ __noinline__ void learn_thread_rows(const LearnArgs &a, const LearnCt
         int ev;
         if (evid != 1) {                                                    // :53-57
             NbUniforms rng(id, a.epoch, NB_TAG_EVID, a.seed);
-            ev = nb_sample_row_v<WIDE>(r, len, self, meta, NbValsCG{a.val_evid}, wts, rng);
+            ev = nb_sample_row_v<WIDE>(r, len, self, meta, NbValsCG<T>(a.val_evid, a), wts, rng);
         } else {
             ev = (int)a.vinit[nid];                                         // :60-61
         }
-        a.val_evid[nid] = (nb_val_t)ev;                                     // :63
+        a.val_evid[nid] = (T)ev;                                            // :63
         NbUniforms rng(id, a.epoch, NB_TAG_FREE, a.seed);
-        int prop = nb_sample_row_v<WIDE>(r, len, self, meta, NbValsCG{a.val_free}, wts, rng);   // :65-67
-        a.val_free[nid] = (nb_val_t)prop;                                   // :69
+        int prop = nb_sample_row_v<WIDE>(r, len, self, meta, NbValsCG<T>(a.val_free, a), wts, rng);   // :65-67
+        a.val_free[nid] = (T)prop;                                          // :69
         if (!a.learn_non_evidence && evid != 1) continue;                   // :70-71
         nb_row_gradient<WIDE, SMEM>(r, len, self, meta, ev, prop, a, nb_cnt_inc(a, id), ctx, 0, 1, nullptr, 0);
     }
 }
 
-__device__ __forceinline__ int nb_ldv(const nb_val_t *v, uint32_t i) { return (int)__ldca(v + i); }   // see NbValsCG
+template <class T>
+__device__ __forceinline__ int nb_ldv(const T *v, uint32_t i) { return (int)__ldca(v + i); }   // see NbValsCG
 // ---------------------------------------------------------------------------
 // categorical record rows (CAT class), one row per thread.  Same records as the Gibbs sweep
 // (nb_cat_energies: one 16-byte quad per incidence of an AND_CAT / EQUAL_CAT_CONST factor in its
@@ -275,8 +279,8 @@ __device__ __forceinline__ int nb_cat_draw(float *e, int card, double u)
     return card - 1;
 }
 
-template <bool SMEM>
-__device__ __forceinline__ int nb_cat_sample_l(const uint4 *qp, const uint32_t *wp, int n, int card, const nb_val_t *vals,
+template <bool SMEM, class T>
+__device__ __forceinline__ int nb_cat_sample_l(const uint4 *qp, const uint32_t *wp, int n, int card, const T *vals,
                                                const LearnCtx<SMEM> &ctx, float *e, double u)
 {
     for (int k = 0; k < card; k++) e[k] = 0.0f;
@@ -298,16 +302,16 @@ __device__ __forceinline__ int nb_cat_sample_l(const uint4 *qp, const uint32_t *
     return nb_cat_draw(e, card, u);
 }
 
-template <bool SMEM>
-__device__ __noinline__ void learn_cat_rows(const LearnArgs &a, const LearnCtx<SMEM> &ctx, int beg, int end, uint32_t kf, uint32_t ke)
+template <bool SMEM, class T>
+__device__ __noinline__ void learn_cat_rows(const LearnArgs<T> &a, const LearnCtx<SMEM> &ctx, int beg, int end, uint32_t kf, uint32_t ke)
 {
     float e[NB_CAT_MAX_CARD];
-    const nb_val_t *vF = a.val_free, *vE = a.val_evid;
+    const T *vF = a.val_free, *vE = a.val_evid;
     for (int64_t nid = (int64_t)beg + blockIdx.x * (int64_t)blockDim.x + threadIdx.x; nid < end; nid += (int64_t)gridDim.x * blockDim.x) {
         const uint32_t meta = __ldg(a.vmeta + nid);
         const int evid = NB_META_EVID(meta);
         if (!NB_META_VALID(meta) || evid == 4) continue;                   // learning.py:24-26
-        const int card = NB_META_CARD(meta);
+        const int card = NB_META_CARD(meta);                               // CAT rows: card <= NB_CAT_MAX_CARD
         const uint32_t id = __ldg(a.rng_id + nid);
         const int64_t s = (nid - a.cat_first) >> 5;
         const int64_t q0 = __ldg(a.cat_ptr + s), q1 = __ldg(a.cat_ptr + s + 1);
@@ -317,9 +321,9 @@ __device__ __noinline__ void learn_cat_rows(const LearnArgs &a, const LearnCtx<S
         int ev;
         if (evid != 1) ev = nb_cat_sample_l<SMEM>(qp, wp, n, card, vE, ctx, e, nb_philox2x32_u53(id, (uint32_t)a.epoch, ke));   // :53-57
         else ev = (int)a.vinit[nid];                                        // :60-61
-        a.val_evid[nid] = (nb_val_t)ev;                                     // :63
+        a.val_evid[nid] = (T)ev;                                            // :63
         const int prop = nb_cat_sample_l<SMEM>(qp, wp, n, card, vF, ctx, e, nb_philox2x32_u53(id, (uint32_t)a.epoch, kf));   // :65-67
-        a.val_free[nid] = (nb_val_t)prop;                                   // :69
+        a.val_free[nid] = (T)prop;                                          // :69
         if (!a.learn_non_evidence && evid != 1) continue;                   // :70-71
         // gradient (learning.py:73-108): the incidences of the buckets of the two chains' values
         const uint32_t cinc = nb_cnt_inc(a, id);
@@ -339,13 +343,13 @@ __device__ __noinline__ void learn_cat_rows(const LearnArgs &a, const LearnCtx<S
 // warp path: one long row per warp
 // ---------------------------------------------------------------------------
 // per-value energies of a warp row into e[4] (dataType 0, card <= 4) or the shared array se
-template <bool WIDE, bool SMEM>
+template <bool WIDE, bool SMEM, class T>
 __device__ inline void nb_warp_energies_l(const NbRow &r, const uint2 *inc, int n_inc, uint32_t self, uint32_t meta,
-                                          const nb_val_t *vals, const LearnCtx<SMEM> &ctx, double e[4], double *se)
+                                          const T *vals, const LearnCtx<SMEM> &ctx, double e[4], double *se)
 {
-    const int lane = threadIdx.x & 31, card = NB_META_CARD(meta);
+    const int lane = threadIdx.x & 31, card = NB_META_CARD(meta);   // <= NB_MAX_CARD: wider rows take nb_warp_sample_wide
     const bool small = NB_META_DTYPE(meta) == 0 && card <= 4;
-    const NbValsCG v{vals};
+    const NbValsCG<T> v(vals);
     if (!small) {
         for (int k = lane; k < card; k += 32) se[k] = 0.0;
         __syncwarp();
@@ -374,9 +378,9 @@ __device__ inline void nb_warp_energies_l(const NbRow &r, const uint2 *inc, int 
     }
 }
 
-template <bool WIDE, bool SMEM>
+template <bool WIDE, bool SMEM, class T>
 __device__ NB_EVAL_FN int nb_warp_sample_l(const NbRow &r, const uint2 *inc, int n_inc, uint32_t self, uint32_t meta,
-                                       const nb_val_t *vals, const LearnCtx<SMEM> &ctx, double *se, NbUniforms &rng)
+                                       const T *vals, const LearnCtx<SMEM> &ctx, double *se, NbUniforms &rng)
 {
     const int card = NB_META_CARD(meta);
     double e[4] = {0.0, 0.0, 0.0, 0.0};
@@ -393,8 +397,21 @@ __device__ NB_EVAL_FN int nb_warp_sample_l(const NbRow &r, const uint2 *inc, int
     return k;
 }
 
-template <bool WIDE, bool SMEM>
-__device__ __noinline__ void learn_warp_rows(const LearnArgs &a, const LearnCtx<SMEM> &ctx, double *s_e, int wbeg, int wend)
+// the sampler of one chain for a warp row: the shared-memory one, or nb_warp_sample_wide for a
+// cardinality above 255 (2-byte graphs)
+template <bool WIDE, bool SMEM, class T>
+__device__ __forceinline__ int nb_warp_sample_any(const LearnArgs<T> &a, const NbRow &r, int64_t wr, const uint2 *inc, int n_inc,
+                                                  uint32_t self, uint32_t meta, const T *vals, const LearnCtx<SMEM> &ctx,
+                                                  double *se, NbUniforms &rng)
+{
+    if (sizeof(T) > 1 && NB_META_CARD(meta) == 0)
+        return nb_warp_sample_wide<WIDE>(r, (int)(a.wrow_ptr[wr + 1] - a.wrow_ptr[wr]), inc, n_inc, self, meta,
+                                         a.card(meta, self), NbValsCG<T>(vals), CtxWts<SMEM>{ctx}, rng);
+    return nb_warp_sample_l<WIDE, SMEM>(r, inc, n_inc, self, meta, vals, ctx, se, rng);
+}
+
+template <bool WIDE, bool SMEM, class T>
+__device__ __noinline__ void learn_warp_rows(const LearnArgs<T> &a, const LearnCtx<SMEM> &ctx, double *s_e, int wbeg, int wend)
 {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     for (int64_t wr = (int64_t)wbeg + blockIdx.x * (int64_t)NB_LWARPS + warp; wr < wend;
@@ -410,13 +427,13 @@ __device__ __noinline__ void learn_warp_rows(const LearnArgs &a, const LearnCtx<
         int ev;
         if (evid != 1) {
             NbUniforms rng(id, a.epoch, NB_TAG_EVID, a.seed);
-            ev = nb_warp_sample_l<WIDE, SMEM>(r, inc, n_inc, self, meta, a.val_evid, ctx, s_e, rng);
+            ev = nb_warp_sample_any<WIDE, SMEM>(a, r, wr, inc, n_inc, self, meta, a.val_evid, ctx, s_e, rng);
         } else {
             ev = (int)a.vinit[nid];
         }
         NbUniforms rng(id, a.epoch, NB_TAG_FREE, a.seed);
-        int prop = nb_warp_sample_l<WIDE, SMEM>(r, inc, n_inc, self, meta, a.val_free, ctx, s_e, rng);
-        if (lane == 0) { a.val_evid[nid] = (nb_val_t)ev; a.val_free[nid] = (nb_val_t)prop; }
+        int prop = nb_warp_sample_any<WIDE, SMEM>(a, r, wr, inc, n_inc, self, meta, a.val_free, ctx, s_e, rng);
+        if (lane == 0) { a.val_evid[nid] = (T)ev; a.val_free[nid] = (T)prop; }
         if (!a.learn_non_evidence && evid != 1) continue;
         nb_row_gradient<WIDE, SMEM>(r, 0, self, meta, ev, prop, a, nb_cnt_inc(a, id), ctx, lane, 32, inc, n_inc);
     }
@@ -429,15 +446,15 @@ __device__ __noinline__ void learn_warp_rows(const LearnArgs &a, const LearnCtx<
 // ---------------------------------------------------------------------------
 
 // (two id ranges per call: the cell's PAIR rows and its FAST rows -- one copy of the code)
-template <bool SMEM>
-__device__ __noinline__ void learn_tt_slices(const LearnArgs &a, const LearnCtx<SMEM> &ctx, int beg0, int end0, int beg1, int end1,
+template <bool SMEM, class T>
+__device__ __noinline__ void learn_tt_slices(const LearnArgs<T> &a, const LearnCtx<SMEM> &ctx, int beg0, int end0, int beg1, int end1,
                                              uint32_t kfree, uint32_t kevid, uint32_t ktrunc, int rot)
 {
     const unsigned FULL = 0xFFFFFFFFu;
     const int lane = threadIdx.x & 31;
     const int64_t warp_global = blockIdx.x * (int64_t)NB_LWARPS + (threadIdx.x >> 5);
     const int64_t n_warps = (int64_t)gridDim.x * NB_LWARPS;
-    const nb_val_t *vF = a.val_free, *vE = a.val_evid;
+    const T *vF = a.val_free, *vE = a.val_evid;
     const int64_t s0b = beg0 >> 5, s0e = end0 > beg0 ? (((int64_t)end0 + 31) >> 5) : s0b;
     const int64_t s1b = beg1 >> 5, s1e = end1 > beg1 ? (((int64_t)end1 + 31) >> 5) : s1b;
     const int64_t ns0 = s0e - s0b, ns = ns0 + (s1e - s1b);
@@ -495,7 +512,7 @@ __device__ __noinline__ void learn_tt_slices(const LearnArgs &a, const LearnCtx<
         }
         const double uf = nb_philox2x32_u53(rid, (uint32_t)a.epoch, kfree);
         const int prop = uf <= (double)(1.0f / (1.0f + __expf((float)dF))) ? 0 : 1;
-        if (valid) { a.val_evid[nid] = (nb_val_t)ev; a.val_free[nid] = (nb_val_t)prop; }
+        if (valid) { a.val_evid[nid] = (T)ev; a.val_free[nid] = (T)prop; }
         const bool active = valid && (a.learn_non_evidence || evid == 1);        // :70-71
         uint32_t cinc = 1;
         if (a.regularization == 1)                                                // :90
@@ -552,14 +569,14 @@ __device__ __forceinline__ int nb_grad_of(uint32_t p, int prop, int ev)
     return fF - fE;
 }
 
-template <bool SMEM>
-__device__ __noinline__ void learn_tt_rows(const LearnArgs &a, const LearnCtx<SMEM> &ctx, int beg0, int end0, int beg1, int end1,
+template <bool SMEM, class T>
+__device__ __noinline__ void learn_tt_rows(const LearnArgs<T> &a, const LearnCtx<SMEM> &ctx, int beg0, int end0, int beg1, int end1,
                                            uint32_t kfree, uint32_t kevid, uint32_t ktrunc, int rot)
 {
     const int lane = threadIdx.x & 31;
     const int64_t warp_global = blockIdx.x * (int64_t)NB_LWARPS + (threadIdx.x >> 5);
     const int64_t n_warps = (int64_t)gridDim.x * NB_LWARPS;
-    const nb_val_t *vF = a.val_free, *vE = a.val_evid;
+    const T *vF = a.val_free, *vE = a.val_evid;
     const int64_t n0 = max(end0 - beg0, 0), ntot = n0 + max(end1 - beg1, 0);
 
     int64_t it_first = warp_global + rot;
@@ -630,7 +647,7 @@ __device__ __noinline__ void learn_tt_rows(const LearnArgs &a, const LearnCtx<SM
         const double uf = nb_philox2x32_u53(rid, (uint32_t)a.epoch, kfree);
         const int prop = uf <= (double)(1.0f / (1.0f + __expf((float)dF))) ? 0 : 1;
         __syncwarp();
-        if (lane == 0) { a.val_evid[nid] = (nb_val_t)ev; a.val_free[nid] = (nb_val_t)prop; }
+        if (lane == 0) { a.val_evid[nid] = (T)ev; a.val_free[nid] = (T)prop; }
         if (!a.learn_non_evidence && evid != 1) continue;                        // :70-71
         uint32_t cinc = 1;
         if (a.regularization == 1)
@@ -676,8 +693,9 @@ __device__ __forceinline__ void nb_grid_sync(unsigned *bar)
     __syncthreads();
 }
 
+// (1-byte graphs only: 2-byte graphs learn in throughput mode)
 template <bool WIDE, bool SMEM>
-__global__ void __launch_bounds__(NB_LEARN_THREADS) k_learn_cells(LearnArgs a, CellPlan plan, int cell_beg, int cell_end,
+__global__ void __launch_bounds__(NB_LEARN_THREADS) k_learn_cells(LearnArgs<nb_val_t> a, CellPlan plan, int cell_beg, int cell_end,
                                                                   int only_color)
 {
     extern __shared__ unsigned char s_raw[];
@@ -824,8 +842,8 @@ __global__ void __launch_bounds__(NB_LEARN_THREADS) k_learn_cells(LearnArgs a, C
 // device functions, 64-register budgets, full grids -- plus one apply kernel; a handful of launches
 // per cell is nothing against cells of hundreds of microseconds.
 // ---------------------------------------------------------------------------
-template <bool SMEM>
-__device__ __forceinline__ LearnCtx<SMEM> nb_lean_ctx(const LearnArgs &a, unsigned char *s_raw, int slot)
+template <bool SMEM, class T>
+__device__ __forceinline__ LearnCtx<SMEM> nb_lean_ctx(const LearnArgs<T> &a, unsigned char *s_raw, int slot)
 {
     const int W = a.W;
     double *s_w = (double *)s_raw;
@@ -844,8 +862,8 @@ __device__ __forceinline__ LearnCtx<SMEM> nb_lean_ctx(const LearnArgs &a, unsign
     return ctx;
 }
 
-template <bool SMEM>
-__device__ __forceinline__ void nb_lean_flush(const LearnArgs &a, const LearnCtx<SMEM> &ctx, int slot)
+template <bool SMEM, class T>
+__device__ __forceinline__ void nb_lean_flush(const LearnArgs<T> &a, const LearnCtx<SMEM> &ctx, int slot)
 {
     if (!SMEM) return;
     __syncthreads();
@@ -859,47 +877,48 @@ __device__ __forceinline__ void nb_lean_flush(const LearnArgs &a, const LearnCtx
     }
 }
 
-template <bool SMEM>
-__global__ void __launch_bounds__(NB_LEARN_THREADS, 3) k_cell_tt(LearnArgs a, int pb, int pe, int fb, int fe, int by_row, int slot,
+template <bool SMEM, class T>
+__global__ void __launch_bounds__(NB_LEARN_THREADS, 3) k_cell_tt(LearnArgs<T> a, int pb, int pe, int fb, int fe, int by_row, int slot,
                                                                  uint32_t kf, uint32_t ke, uint32_t kt)
 {
     extern __shared__ unsigned char s_raw[];
-    const LearnCtx<SMEM> ctx = nb_lean_ctx<SMEM>(a, s_raw, slot);
+    const LearnCtx<SMEM> ctx = nb_lean_ctx<SMEM, T>(a, s_raw, slot);
     if (by_row) learn_tt_rows<SMEM>(a, ctx, pb, pe, fb, fe, kf, ke, kt, 0);
     else learn_tt_slices<SMEM>(a, ctx, pb, pe, fb, fe, kf, ke, kt, 0);
-    nb_lean_flush<SMEM>(a, ctx, slot);
+    nb_lean_flush<SMEM, T>(a, ctx, slot);
 }
 
-template <bool WIDE, bool SMEM>
-__global__ void __launch_bounds__(NB_LEARN_THREADS, 4) k_cell_thread(LearnArgs a, int tb, int te, int slot)
+template <bool WIDE, bool SMEM, class T>
+__global__ void __launch_bounds__(NB_LEARN_THREADS, 4) k_cell_thread(LearnArgs<T> a, int tb, int te, int slot)
 {
     extern __shared__ unsigned char s_raw[];
-    const LearnCtx<SMEM> ctx = nb_lean_ctx<SMEM>(a, s_raw, slot);
+    const LearnCtx<SMEM> ctx = nb_lean_ctx<SMEM, T>(a, s_raw, slot);
     learn_thread_rows<WIDE, SMEM>(a, ctx, 0, 0, tb, te);
-    nb_lean_flush<SMEM>(a, ctx, slot);
+    nb_lean_flush<SMEM, T>(a, ctx, slot);
 }
 
-template <bool SMEM>
-__global__ void __launch_bounds__(NB_LEARN_THREADS, 4) k_cell_cat(LearnArgs a, int cb, int ce, int slot, uint32_t kf, uint32_t ke)
+template <bool SMEM, class T>
+__global__ void __launch_bounds__(NB_LEARN_THREADS, 4) k_cell_cat(LearnArgs<T> a, int cb, int ce, int slot, uint32_t kf, uint32_t ke)
 {
     extern __shared__ unsigned char s_raw[];
-    const LearnCtx<SMEM> ctx = nb_lean_ctx<SMEM>(a, s_raw, slot);
+    const LearnCtx<SMEM> ctx = nb_lean_ctx<SMEM, T>(a, s_raw, slot);
     learn_cat_rows<SMEM>(a, ctx, cb, ce, kf, ke);
-    nb_lean_flush<SMEM>(a, ctx, slot);
+    nb_lean_flush<SMEM, T>(a, ctx, slot);
 }
 
-template <bool WIDE, bool SMEM>
-__global__ void __launch_bounds__(NB_LEARN_THREADS, 2) k_cell_warp(LearnArgs a, int wb, int we, int slot)
+template <bool WIDE, bool SMEM, class T>
+__global__ void __launch_bounds__(NB_LEARN_THREADS, 2) k_cell_warp(LearnArgs<T> a, int wb, int we, int slot)
 {
     extern __shared__ unsigned char s_raw[];
     __shared__ double s_e[NB_LWARPS][NB_MAX_CARD + 1];
-    const LearnCtx<SMEM> ctx = nb_lean_ctx<SMEM>(a, s_raw, slot);
+    const LearnCtx<SMEM> ctx = nb_lean_ctx<SMEM, T>(a, s_raw, slot);
     learn_warp_rows<WIDE, SMEM>(a, ctx, s_e[threadIdx.x >> 5], wb, we);
-    nb_lean_flush<SMEM>(a, ctx, slot);
+    nb_lean_flush<SMEM, T>(a, ctx, slot);
 }
 
 // apply the cell's sums to the global weights and clear the table for its next use
-__global__ void k_cell_apply(LearnArgs a, int slot)
+template <class T>
+__global__ void k_cell_apply(LearnArgs<T> a, int slot)
 {
     nb_fix_t *g_gf = a.g_grad + (size_t)slot * a.W;
     uint32_t *g_cn = a.g_cnt + (size_t)slot * a.W;
@@ -921,8 +940,8 @@ struct RowRanges {
     int wbeg, wend;        // warp rows
 };
 
-template <bool WIDE>
-__global__ void k_visit_histogram(LearnArgs a, RowRanges rr, uint32_t *hist)
+template <bool WIDE, class T>
+__global__ void k_visit_histogram(LearnArgs<T> a, RowRanges rr, uint32_t *hist)
 {
     int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     int64_t nid = -1;
@@ -961,13 +980,14 @@ __global__ void k_max_u32(const uint32_t *x, int n, uint32_t *out)
 // ---------------------------------------------------------------------------
 // host driver
 // ---------------------------------------------------------------------------
-static LearnArgs learn_args(nb_graph *g)
+template <class T>
+static LearnArgs<T> learn_args(nb_graph *g)
 {
-    LearnArgs a;
-    memset(&a, 0, sizeof(a));
+    LearnArgs<T> a{};
     a.vmeta = g->d_vmeta; a.slice_ptr = g->d_slice_ptr; a.twords = g->d_twords;
     a.wrow_ptr = g->d_wrow_ptr; a.wwords = g->d_wwords; a.inc_ptr = g->d_inc_ptr; a.inc = g->d_inc;
-    a.rng_id = g->d_rng_id; a.vinit = g->d_vinit; a.val_free = g->d_val[0]; a.val_evid = g->d_val[1];
+    a.rng_id = g->d_rng_id; a.vinit = (const T *)g->d_vinit; a.val_free = nb_vals<T>(g, 0); a.val_evid = nb_vals<T>(g, 1);
+    if constexpr (sizeof(T) > 1) a.vcard = g->d_vcard;
     a.weight = g->d_weight; a.wfixed = g->d_wfixed; a.n_trows = g->n_trows; a.W = (int)g->W;
     a.g_grad = g->d_grad; a.g_cnt = g->d_nvis; a.bar = g->d_learn_bar;
     a.tt_ptr = g->d_tt_ptr; a.tt = g->d_tt; a.tt_base = g->d_tt_base; a.tt_wid = g->d_tt_wid;
@@ -986,7 +1006,8 @@ static int ensure_learn_buffers(nb_graph *g)
 }
 
 // max over weights of the gradient visits one sweep of colour c can make
-static int color_visit_bounds(nb_graph *g, LearnArgs a, std::vector<int64_t> &out)
+template <class T>
+static int color_visit_bounds(nb_graph *g, LearnArgs<T> a, std::vector<int64_t> &out)
 {
     out.assign((size_t)g->n_colors, 0);
     uint32_t *d_max, *d_hist;
@@ -1005,8 +1026,8 @@ static int color_visit_bounds(nb_graph *g, LearnArgs a, std::vector<int64_t> &ou
         cudaMemsetAsync(d_hist, 0, (size_t)g->W * 4, g->stream);
         cudaMemsetAsync(d_max, 0, 4, g->stream);
         unsigned grid = (unsigned)((n + 255) / 256);
-        if (g->wide) k_visit_histogram<true><<<grid, 256, 0, g->stream>>>(a, rr, d_hist);
-        else k_visit_histogram<false><<<grid, 256, 0, g->stream>>>(a, rr, d_hist);
+        if (g->wide) k_visit_histogram<true, T><<<grid, 256, 0, g->stream>>>(a, rr, d_hist);
+        else k_visit_histogram<false, T><<<grid, 256, 0, g->stream>>>(a, rr, d_hist);
         k_max_u32<<<64, 256, 0, g->stream>>>(d_hist, (int)g->W, d_max);
         uint32_t m = 0;
         cudaMemcpyAsync(&m, d_max, 4, cudaMemcpyDeviceToHost, g->stream);
@@ -1019,10 +1040,11 @@ static int color_visit_bounds(nb_graph *g, LearnArgs a, std::vector<int64_t> &ou
 }
 
 // per-graph cache of the visit bounds (depends on learn_non_evidence) and the device-side plan data
-static int learn_prepare(nb_graph *g, LearnArgs &a, std::vector<int64_t> &vmax, int learn_non_evidence)
+template <class T>
+static int learn_prepare(nb_graph *g, LearnArgs<T> &a, std::vector<int64_t> &vmax, int learn_non_evidence)
 {
     NB_TRY(ensure_learn_buffers(g));
-    a = learn_args(g);
+    a = learn_args<T>(g);
     a.learn_non_evidence = learn_non_evidence;
     if (g->learn_vmax_flag != learn_non_evidence || (int)g->learn_vmax.size() != g->n_colors) {
         NB_TRY(color_visit_bounds(g, a, g->learn_vmax));
@@ -1084,15 +1106,20 @@ static CellPlan make_plan(const nb_graph *g, int n_blocks)
 
 int nb_learn_block_count(nb_graph *g, double step, int learn_non_evidence, int64_t batch_visits, int *n_blocks)
 {
-    LearnArgs a;
     std::vector<int64_t> vmax;
-    NB_TRY(learn_prepare(g, a, vmax, learn_non_evidence));
+    if (g->value_bytes == 1) {
+        LearnArgs<nb_val_t> a;
+        NB_TRY(learn_prepare(g, a, vmax, learn_non_evidence));
+    } else {
+        LearnArgs<nb_val16_t> a;
+        NB_TRY(learn_prepare(g, a, vmax, learn_non_evidence));
+    }
     *n_blocks = block_count(g, vmax, default_batch_visits(step, batch_visits));
     return NB_OK;
 }
 
 template <bool WIDE, bool SMEM>
-static int launch_cells_t(nb_graph *g, LearnArgs a, CellPlan plan, int cell_beg, int cell_end, int only_color)
+static int launch_cells_t(nb_graph *g, LearnArgs<nb_val_t> a, CellPlan plan, int cell_beg, int cell_end, int only_color)
 {
     const size_t smem = SMEM ? (size_t)g->W * 24 : 0;
     auto kern = k_learn_cells<WIDE, SMEM>;
@@ -1154,7 +1181,7 @@ static int launch_cells_t(nb_graph *g, LearnArgs a, CellPlan plan, int cell_beg,
     return NB_OK;
 }
 
-static int launch_cells(nb_graph *g, const LearnArgs &a, const CellPlan &plan, int cell_beg, int cell_end, int only_color)
+static int launch_cells(nb_graph *g, const LearnArgs<nb_val_t> &a, const CellPlan &plan, int cell_beg, int cell_end, int only_color)
 {
     const bool smem = g->W <= NB_LEARN_SMEM_W;
     if (g->wide) return smem ? launch_cells_t<true, true>(g, a, plan, cell_beg, cell_end, only_color)
@@ -1164,8 +1191,8 @@ static int launch_cells(nb_graph *g, const LearnArgs &a, const CellPlan &plan, i
 }
 
 // one cell as ordinary launches (throughput mode)
-template <bool WIDE, bool SMEM>
-static int launch_cell_lean_t(nb_graph *g, const LearnArgs &a, const CellPlan &plan, int block, int color)
+template <bool WIDE, bool SMEM, class T>
+static int launch_cell_lean_t(nb_graph *g, const LearnArgs<T> &a, const CellPlan &plan, int block, int color)
 {
     CellPlan hp = plan;
     hp.win_start = g->win_start.data();            // host copy of the window table
@@ -1183,40 +1210,41 @@ static int launch_cell_lean_t(nb_graph *g, const LearnArgs &a, const CellPlan &p
     const uint32_t kf = nb_fold_key(a.seed, a.epoch, NB_TAG_FREE), ke = nb_fold_key(a.seed, a.epoch, NB_TAG_EVID),
                    kt = nb_fold_key(a.seed, a.epoch, NB_TAG_TRUNC);
     if (smem > 32 * 1024) {
-        NB_CUDA(cudaFuncSetAttribute(k_cell_tt<SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        NB_CUDA(cudaFuncSetAttribute(k_cell_thread<WIDE, SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        NB_CUDA(cudaFuncSetAttribute(k_cell_cat<SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        NB_CUDA(cudaFuncSetAttribute(k_cell_warp<WIDE, SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        NB_CUDA(cudaFuncSetAttribute(k_cell_tt<SMEM, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        NB_CUDA(cudaFuncSetAttribute(k_cell_thread<WIDE, SMEM, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        NB_CUDA(cudaFuncSetAttribute(k_cell_cat<SMEM, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        NB_CUDA(cudaFuncSetAttribute(k_cell_warp<WIDE, SMEM, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
     if (pe > pb || fe > fb) {
         const int64_t rows = (int64_t)(pe - pb) + (fe - fb);
         const int by_row = (g->learn_long_rows[(size_t)color] || rows <= 2 * cap * NB_LWARPS) ? 1 : 0;
         const int64_t need = by_row ? (rows + NB_LWARPS - 1) / NB_LWARPS : (rows / 32 + 2 + NB_LWARPS - 1) / NB_LWARPS;
-        k_cell_tt<SMEM><<<(unsigned)std::max<int64_t>(1, std::min(need, cap)), NB_LEARN_THREADS, smem, g->stream>>>(
+        k_cell_tt<SMEM, T><<<(unsigned)std::max<int64_t>(1, std::min(need, cap)), NB_LEARN_THREADS, smem, g->stream>>>(
             a, pb, pe, fb, fe, by_row, 0, kf, ke, kt);
         g->launches++;
     }
     if (ce > cb) {
         const int64_t need = ((int64_t)(ce - cb) + NB_LEARN_THREADS - 1) / NB_LEARN_THREADS;
-        k_cell_cat<SMEM><<<(unsigned)std::max<int64_t>(1, std::min(need, cap)), NB_LEARN_THREADS, smem, g->stream>>>(a, cb, ce, 0, kf, ke);
+        k_cell_cat<SMEM, T><<<(unsigned)std::max<int64_t>(1, std::min(need, cap)), NB_LEARN_THREADS, smem, g->stream>>>(a, cb, ce, 0, kf, ke);
         g->launches++;
     }
     if (te > tb) {
         const int64_t need = ((int64_t)(te - tb) + NB_LEARN_THREADS - 1) / NB_LEARN_THREADS;
-        k_cell_thread<WIDE, SMEM><<<(unsigned)std::max<int64_t>(1, std::min(need, cap)), NB_LEARN_THREADS, smem, g->stream>>>(a, tb, te, 0);
+        k_cell_thread<WIDE, SMEM, T><<<(unsigned)std::max<int64_t>(1, std::min(need, cap)), NB_LEARN_THREADS, smem, g->stream>>>(a, tb, te, 0);
         g->launches++;
     }
     if (we > wb) {
         const int64_t need = ((int64_t)(we - wb) + NB_LWARPS - 1) / NB_LWARPS;
-        k_cell_warp<WIDE, SMEM><<<(unsigned)std::max<int64_t>(1, std::min(need, cap)), NB_LEARN_THREADS, smem, g->stream>>>(a, wb, we, 0);
+        k_cell_warp<WIDE, SMEM, T><<<(unsigned)std::max<int64_t>(1, std::min(need, cap)), NB_LEARN_THREADS, smem, g->stream>>>(a, wb, we, 0);
         g->launches++;
     }
-    k_cell_apply<<<(unsigned)std::max<int64_t>(1, std::min<int64_t>((g->W + 255) / 256, cap)), 256, 0, g->stream>>>(a, 0);
+    k_cell_apply<T><<<(unsigned)std::max<int64_t>(1, std::min<int64_t>((g->W + 255) / 256, cap)), 256, 0, g->stream>>>(a, 0);
     g->launches++;
     return NB_OK;
 }
 
-static int launch_cell_lean(nb_graph *g, const LearnArgs &a, const CellPlan &plan, int block, int color)
+template <class T>
+static int launch_cell_lean(nb_graph *g, const LearnArgs<T> &a, const CellPlan &plan, int block, int color)
 {
     const bool smem = g->W <= NB_LEARN_SMEM_W;
     if (g->wide) return smem ? launch_cell_lean_t<true, true>(g, a, plan, block, color) : launch_cell_lean_t<true, false>(g, a, plan, block, color);
@@ -1226,33 +1254,43 @@ static int launch_cell_lean(nb_graph *g, const LearnArgs &a, const CellPlan &pla
 // Latency mode (persistent kernel) or throughput mode (lean launches per cell)?  The persistent
 // grid has 2 x 256 threads per SM; beyond ~16 rows per thread and cell the cells are long enough
 // (hundreds of microseconds) for launch overhead not to matter and for occupancy to decide.
-static bool lean_mode(const nb_graph *g, int64_t cells)
+// 2-byte graphs always learn in throughput mode: the persistent kernel is instantiated for 1-byte
+// values only (it is the 128-register kernel whose instruction footprint DESIGN.md section 4 keeps small).
+static int lean_mode(const nb_graph *g, int64_t cells, bool *lean)
 {
     const char *e = getenv("NUMBSKULL_B200_LEARN_MODE");   // 1 persistent, 2 lean (tests compare the two)
     const int force = e ? atoi(e) : 0;
-    if (force == 1) return false;
-    if (force == 2) return true;
+    if (g->value_bytes != 1) {
+        if (force == 1)
+            NB_FAIL(NB_ERR_UNSUPPORTED, "NUMBSKULL_B200_LEARN_MODE=1 (latency mode) is not available on graphs with "
+                                        "cardinalities above 255: they learn in throughput mode only");
+        *lean = true;
+        return NB_OK;
+    }
+    if (force == 1 || force == 2) { *lean = force == 2; return NB_OK; }
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, g->device);
-    return g->V / std::max<int64_t>(cells, 1) > (int64_t)sms * 2 * NB_LEARN_THREADS * 2;
+    *lean = g->V / std::max<int64_t>(cells, 1) > (int64_t)sms * 2 * NB_LEARN_THREADS * 2;
+    return NB_OK;
 }
 
 // one (block, colour) cell: the partitioned runner exchanges halo values between the cells itself
-int nb_learn_color(nb_graph *g, int color, int block, int n_blocks, double step, int regularization, double reg_param,
-                   double truncation, int learn_non_evidence, uint64_t seed, uint64_t epoch)
+template <class T>
+static int learn_color_t(nb_graph *g, int color, int block, int n_blocks, double step, int regularization, double reg_param,
+                         double truncation, int learn_non_evidence, uint64_t seed, uint64_t epoch)
 {
-    if (color < 0 || color >= g->n_colors) return NB_OK;   // a colour this rank does not own
-    if (n_blocks < 1 || block < 0 || block >= n_blocks) NB_FAIL(NB_ERR_INVALID, "block %d of %d", block, n_blocks);
-    LearnArgs a;
+    LearnArgs<T> a;
     std::vector<int64_t> vmax;
     NB_TRY(learn_prepare(g, a, vmax, learn_non_evidence));
     a.seed = seed; a.reg_param = reg_param; a.truncation = truncation; a.regularization = regularization;
     a.step = step; a.epoch = epoch;
-    if (lean_mode(g, (int64_t)n_blocks * g->n_colors)) {
+    bool lean = true;
+    NB_TRY(lean_mode(g, (int64_t)n_blocks * g->n_colors, &lean));
+    if (lean) {
         NB_CUDA(cudaMemsetAsync(a.g_grad, 0, (size_t)g->W * sizeof(nb_fix_t), g->stream));
         NB_CUDA(cudaMemsetAsync(a.g_cnt, 0, (size_t)g->W * sizeof(uint32_t), g->stream));
         NB_TRY(launch_cell_lean(g, a, make_plan(g, n_blocks), block, color));
-    } else {
+    } else if constexpr (sizeof(T) == 1) {
         NB_TRY(launch_cells(g, a, make_plan(g, n_blocks), block, block + 1, color));
     }
     g->weights_version++;
@@ -1260,11 +1298,23 @@ int nb_learn_color(nb_graph *g, int color, int block, int n_blocks, double step,
     return NB_OK;
 }
 
-int nb_run_learn(nb_graph *g, int64_t n_epochs, double *stepsize, double decay, int regularization, double reg_param,
-                 double truncation, int learn_non_evidence, uint64_t seed, int64_t batch_visits)
+int nb_learn_color(nb_graph *g, int color, int block, int n_blocks, double step, int regularization, double reg_param,
+                   double truncation, int learn_non_evidence, uint64_t seed, uint64_t epoch)
 {
-    if (n_epochs <= 0) return NB_OK;
-    LearnArgs a;
+    if (color < 0 || color >= g->n_colors) return NB_OK;   // a colour this rank does not own
+    if (n_blocks < 1 || block < 0 || block >= n_blocks) NB_FAIL(NB_ERR_INVALID, "block %d of %d", block, n_blocks);
+    if (g->value_bytes == 1)
+        return learn_color_t<nb_val_t>(g, color, block, n_blocks, step, regularization, reg_param, truncation,
+                                       learn_non_evidence, seed, epoch);
+    return learn_color_t<nb_val16_t>(g, color, block, n_blocks, step, regularization, reg_param, truncation,
+                                     learn_non_evidence, seed, epoch);
+}
+
+template <class T>
+static int run_learn_t(nb_graph *g, int64_t n_epochs, double *stepsize, double decay, int regularization, double reg_param,
+                       double truncation, int learn_non_evidence, uint64_t seed, int64_t batch_visits)
+{
+    LearnArgs<T> a;
     std::vector<int64_t> vmax;
     NB_TRY(learn_prepare(g, a, vmax, learn_non_evidence));
     a.seed = seed; a.reg_param = reg_param; a.truncation = truncation; a.regularization = regularization;
@@ -1274,14 +1324,16 @@ int nb_run_learn(nb_graph *g, int64_t n_epochs, double *stepsize, double decay, 
         a.epoch = g->epoch_counter++;
         const int nb = block_count(g, vmax, default_batch_visits(step, batch_visits));
         const int64_t cells = (int64_t)nb * g->n_colors;
-        if (lean_mode(g, cells)) {
+        bool lean = true;
+        NB_TRY(lean_mode(g, cells, &lean));
+        if (lean) {
             // throughput mode: a few lean launches per cell (table 0 starts clear, k_cell_apply clears it again)
             NB_CUDA(cudaMemsetAsync(a.g_grad, 0, (size_t)g->W * sizeof(nb_fix_t), g->stream));
             NB_CUDA(cudaMemsetAsync(a.g_cnt, 0, (size_t)g->W * sizeof(uint32_t), g->stream));
             const CellPlan plan = make_plan(g, nb);
             for (int b = 0; b < nb; b++)
                 for (int c = 0; c < g->n_colors; c++) NB_TRY(launch_cell_lean(g, a, plan, b, c));
-        } else {
+        } else if constexpr (sizeof(T) == 1) {
             // latency mode: one persistent launch per epoch (cell indices are 32-bit: split absurdly long epochs)
             for (int64_t c0 = 0; c0 < cells; c0 += (1 << 30)) {
                 const int64_t c1 = std::min<int64_t>(cells, c0 + (1 << 30));
@@ -1294,4 +1346,15 @@ int nb_run_learn(nb_graph *g, int64_t n_epochs, double *stepsize, double decay, 
     }
     *stepsize = step;
     return NB_OK;
+}
+
+int nb_run_learn(nb_graph *g, int64_t n_epochs, double *stepsize, double decay, int regularization, double reg_param,
+                 double truncation, int learn_non_evidence, uint64_t seed, int64_t batch_visits)
+{
+    if (n_epochs <= 0) return NB_OK;
+    if (g->value_bytes == 1)
+        return run_learn_t<nb_val_t>(g, n_epochs, stepsize, decay, regularization, reg_param, truncation, learn_non_evidence,
+                                     seed, batch_visits);
+    return run_learn_t<nb_val16_t>(g, n_epochs, stepsize, decay, regularization, reg_param, truncation, learn_non_evidence,
+                                   seed, batch_visits);
 }

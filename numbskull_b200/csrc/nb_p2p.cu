@@ -35,6 +35,8 @@ extern "C" int nb_p2p_export(nb_graph *g, int world, int rank, uint8_t *handles 
 {
     NB_CUDA(cudaSetDevice(g->device));
     if (!g->finalized) NB_FAIL(NB_ERR_INVALID, "graph not finalized");
+    // the halo moves one byte per value: graphs with cardinalities above 255 are single-GPU only
+    if (g->value_bytes != 1) NB_FAIL(NB_ERR_UNSUPPORTED, "cardinalities above 255 are single-GPU only");
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
     if (!g->p2p) g->p2p = new NbP2P();
     NbP2P *p = p2p_of(g);
@@ -207,7 +209,7 @@ extern "C" int nb_p2p_exchange(nb_graph *g, int color, int chain_mask)
     const bool has = color >= 0 && color + 1 < (int)p->color_ptr.size();
     a.beg = has ? p->color_ptr[(size_t)color] : 0;
     a.end = has ? p->color_ptr[(size_t)color + 1] : 0;
-    a.val0 = g->d_val[0]; a.val1 = g->d_val[1];
+    a.val0 = nb_vals<nb_val_t>(g, 0); a.val1 = nb_vals<nb_val_t>(g, 1);
     a.peer_val0 = p->d_peer_val[0]; a.peer_val1 = p->d_peer_val[1];
     a.peer_flags = p->d_peer_flags; a.flags = p->d_flags; a.neigh = p->d_neigh; a.n_neigh = p->n_neigh;
     a.rank = p->rank; a.chain_mask = chain_mask & 3; a.wait = (chain_mask & 16) ? 0 : 1;

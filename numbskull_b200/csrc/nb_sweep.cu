@@ -8,7 +8,9 @@
 // shuffles (shared memory for categorical rows).
 #include "nb_eval.cuh"
 
-struct SweepArgs {
+// T = element type of the value arrays (nb_val_t or nb_val16_t, see nb_graph::value_bytes)
+template <class T>
+struct SweepArgs : NbCardOf<T> {   // (cardinalities: a.card(meta, nid))
     const uint32_t *vmeta;
     const int64_t *slice_ptr;
     const uint32_t *twords;
@@ -20,7 +22,7 @@ struct SweepArgs {
     const uint32_t *cstart;
     int32_t *count;
     int32_t *count_b;
-    nb_val_t *val;
+    T *val;
     uint32_t *valbits;       // bit-packed mirror of val (nullptr: not in use), see nb_graph::d_valbits
     const double *weight;
     int64_t n_trows;
@@ -36,7 +38,8 @@ struct SweepArgs {
 
 // Prologue of every sweep kernel: ghost values may only be read once each neighbour rank has
 // signalled the latest halo phase (its peer stores are fenced before the signal).
-__device__ __forceinline__ void nb_wait_halo(const SweepArgs &a)
+template <class T>
+__device__ __forceinline__ void nb_wait_halo(const SweepArgs<T> &a)
 {
     if (a.w_n == 0) return;
     if ((int)threadIdx.x < a.w_n) {
@@ -52,12 +55,14 @@ __device__ __forceinline__ void nb_wait_halo(const SweepArgs &a)
     __syncthreads();
 }
 
-static SweepArgs sweep_args(nb_graph *g, int chain, int burnin, int sample_evidence, uint64_t seed, uint64_t epoch)
+template <class T>
+static SweepArgs<T> sweep_args(nb_graph *g, int chain, int burnin, int sample_evidence, uint64_t seed, uint64_t epoch)
 {
-    SweepArgs a;
+    SweepArgs<T> a;
     a.vmeta = g->d_vmeta; a.slice_ptr = g->d_slice_ptr; a.twords = g->d_twords;
     a.wrow_ptr = g->d_wrow_ptr; a.wwords = g->d_wwords; a.inc_ptr = g->d_inc_ptr; a.inc = g->d_inc;
-    a.rng_id = g->d_rng_id; a.cstart = g->d_cstart; a.count = g->d_count; a.count_b = g->d_count_b; a.val = g->d_val[chain];
+    a.rng_id = g->d_rng_id; a.cstart = g->d_cstart; a.count = g->d_count; a.count_b = g->d_count_b; a.val = nb_vals<T>(g, chain);
+    if constexpr (sizeof(T) > 1) a.vcard = g->d_vcard;
     a.valbits = (g->use_bits && chain == 0) ? g->d_valbits : nullptr;
     a.weight = g->d_weight; a.n_trows = g->n_trows; a.seed = seed; a.epoch = epoch;
     a.burnin = burnin; a.sample_evidence = sample_evidence;
@@ -65,7 +70,15 @@ static SweepArgs sweep_args(nb_graph *g, int chain, int burnin, int sample_evide
     return a;
 }
 
-__device__ __forceinline__ void nb_tally(const SweepArgs &a, int64_t nid, int card, int k)
+// cardinality of new id nid
+template <class T>
+__device__ __forceinline__ int nb_card(const SweepArgs<T> &a, uint32_t meta, int64_t nid)
+{
+    return a.card(meta, (uint32_t)nid);
+}
+
+template <class T>
+__device__ __forceinline__ void nb_tally(const SweepArgs<T> &a, int64_t nid, int card, int k)
 {
     if (a.burnin) return;
     uint32_t cs = a.cstart[nid];
@@ -73,8 +86,8 @@ __device__ __forceinline__ void nb_tally(const SweepArgs &a, int64_t nid, int ca
     else a.count[cs + k] += 1;             // :32-33
 }
 
-template <bool WIDE>
-__global__ void __launch_bounds__(256) k_gibbs_thread(SweepArgs a, int beg, int end)
+template <bool WIDE, class T>
+__global__ void __launch_bounds__(256) k_gibbs_thread(SweepArgs<T> a, int beg, int end)
 {
     nb_wait_halo(a);
     int64_t nid = (int64_t)beg + blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -85,9 +98,9 @@ __global__ void __launch_bounds__(256) k_gibbs_thread(SweepArgs a, int beg, int 
     if (!(evid == 0 || a.sample_evidence)) return;          // :24
     NbRow r = nb_thread_row(a.twords, a.slice_ptr, nid);
     NbUniforms rng(a.rng_id[nid], a.epoch, NB_TAG_FREE, a.seed);
-    int k = nb_sample_row<WIDE>(r, NB_META_ROWLEN(meta), (uint32_t)nid, meta, a.val, a.weight, rng);
-    a.val[nid] = (nb_val_t)k;
-    nb_tally(a, nid, NB_META_CARD(meta), k);
+    int k = nb_sample_row<WIDE>(r, NB_META_ROWLEN(meta), (uint32_t)nid, meta, a.val, a, a.weight, rng);
+    a.val[nid] = (T)k;
+    nb_tally(a, nid, nb_card(a, meta, nid), k);
 }
 
 // FAST rows: truth-table stream, one 16-byte quad per incidence (weight value inlined), uniform
@@ -106,8 +119,8 @@ __device__ __forceinline__ void nb_publish_bits(uint32_t *valbits, int64_t nid, 
     if ((threadIdx.x & 31) == 0 && m) valbits[nid >> 5] = (valbits[nid >> 5] & ~m) | b;
 }
 
-template <int UNROLL, int MINB, bool BITS>
-__global__ void __launch_bounds__(256, MINB) k_gibbs_tt(SweepArgs a, const int64_t *__restrict__ tt_ptr,
+template <int UNROLL, int MINB, bool BITS, class T>
+__global__ void __launch_bounds__(256, MINB) k_gibbs_tt(SweepArgs<T> a, const int64_t *__restrict__ tt_ptr,
                                                         const uint4 *__restrict__ tt, int beg, int end, uint32_t key)
 {
     nb_wait_halo(a);
@@ -121,7 +134,7 @@ __global__ void __launch_bounds__(256, MINB) k_gibbs_tt(SweepArgs a, const int64
     const int64_t q0 = nb_lds(tt_ptr + (nid >> 5)), q1 = nb_lds(tt_ptr + (nid >> 5) + 1);
     const int n = (int)((q1 - q0) >> 5);                      // incidences of the longest row of this slice
     const double d = BITS ? nb_tt_delta_v<UNROLL>(tt + q0 + (nid & 31), n, (uint32_t)nid, NbValsBits{a.valbits})
-                          : nb_tt_delta_v<UNROLL>(tt + q0 + (nid & 31), n, (uint32_t)nid, NbValsBytes{a.val});   // e1 - e0
+                          : nb_tt_delta_v<UNROLL>(tt + q0 + (nid & 31), n, (uint32_t)nid, NbValsBytes<T>{a.val});   // e1 - e0
     const int evid = NB_META_EVID(meta);
     // inference.py:21-24
     const bool sampled = in && NB_META_VALID(meta) && evid != 4 && (evid == 0 || a.sample_evidence);
@@ -131,15 +144,15 @@ __global__ void __launch_bounds__(256, MINB) k_gibbs_tt(SweepArgs a, const int64
     const float p0 = 1.0f / (1.0f + __expf((float)d));
     const int k = u <= (double)p0 ? 0 : 1;
     if (sampled) {
-        a.val[nid] = (nb_val_t)k;
+        a.val[nid] = (T)k;
         if (!a.burnin && k) __stcs(a.count_b + nid, nb_lds(a.count_b + nid) + 1);   // inference.py:30-31
     }
     if (BITS) nb_publish_bits(a.valbits, nid0, sampled, k);
 }
 
 // PAIR rows: 8-byte records, two per quad -- or, in uniform slices, bare member ids, four per quad.
-template <bool BITS>
-__global__ void __launch_bounds__(256) k_gibbs_tt2(SweepArgs a, const int64_t *__restrict__ tt2_ptr,
+template <bool BITS, class T>
+__global__ void __launch_bounds__(256) k_gibbs_tt2(SweepArgs<T> a, const int64_t *__restrict__ tt2_ptr,
                                                    const uint32_t *__restrict__ tt2_common,
                                                    const uint4 *__restrict__ tt2, int beg, int end, uint32_t key)
 {
@@ -154,7 +167,7 @@ __global__ void __launch_bounds__(256) k_gibbs_tt2(SweepArgs a, const int64_t *_
     const uint32_t common = nb_lds(tt2_common + (nid >> 5));
     const int n = (int)((q1 - q0) >> 5);                      // quads of the longest row of this slice
     const double d = BITS ? nb_tt2_delta_v(tt2 + q0 + (nid & 31), n, common, (uint32_t)nid, NbValsBits{a.valbits}, a.weight)
-                          : nb_tt2_delta_v(tt2 + q0 + (nid & 31), n, common, (uint32_t)nid, NbValsBytes{a.val}, a.weight);   // e1 - e0
+                          : nb_tt2_delta_v(tt2 + q0 + (nid & 31), n, common, (uint32_t)nid, NbValsBytes<T>{a.val}, a.weight);   // e1 - e0
     const int evid = NB_META_EVID(meta);
     const bool sampled = in && NB_META_VALID(meta) && evid != 4 && (evid == 0 || a.sample_evidence);   // inference.py:21-24
     if (!BITS && !sampled) return;
@@ -162,7 +175,7 @@ __global__ void __launch_bounds__(256) k_gibbs_tt2(SweepArgs a, const int64_t *_
     const float p0 = 1.0f / (1.0f + __expf((float)d));
     const int k = u <= (double)p0 ? 0 : 1;
     if (sampled) {
-        a.val[nid] = (nb_val_t)k;
+        a.val[nid] = (T)k;
         if (!a.burnin && k) __stcs(a.count_b + nid, nb_lds(a.count_b + nid) + 1);   // inference.py:30-31
     }
     if (BITS) nb_publish_bits(a.valbits, nid0, sampled, k);
@@ -181,7 +194,7 @@ __global__ void k_pack_bits(const nb_val_t *__restrict__ val, uint32_t *__restri
 int nb_pack_value_bits(nb_graph *g)
 {
     const int64_t n = g->n_trows + g->n_wrows;
-    k_pack_bits<<<(unsigned)std::min<int64_t>((n + 255) / 256, 148 * 16), 256, 0, g->stream>>>(g->d_val[0], g->d_valbits, n);
+    k_pack_bits<<<(unsigned)std::min<int64_t>((n + 255) / 256, 148 * 16), 256, 0, g->stream>>>(nb_vals<nb_val_t>(g, 0), g->d_valbits, n);
     NB_CUDA(cudaGetLastError());
     return NB_OK;
 }
@@ -195,7 +208,8 @@ struct NbCatSmemAcc {
     __device__ __forceinline__ void add(int k, float w) { e[k][tid] += w; }
 };
 
-__global__ void __launch_bounds__(256) k_gibbs_cat(SweepArgs a, const int64_t *__restrict__ cat_ptr,
+template <class T>
+__global__ void __launch_bounds__(256) k_gibbs_cat(SweepArgs<T> a, const int64_t *__restrict__ cat_ptr,
                                                    const uint4 *__restrict__ cat, int64_t first_id, int beg, int end)
 {
     __shared__ float s_e[NB_CAT_MAX_CARD][256];
@@ -205,7 +219,7 @@ __global__ void __launch_bounds__(256) k_gibbs_cat(SweepArgs a, const int64_t *_
     const uint32_t meta = nb_lds(a.vmeta + nid);
     const uint32_t rid = nb_lds(a.rng_id + nid);
     const uint32_t cs = nb_lds(a.cstart + nid);
-    const int card = NB_META_CARD(meta);
+    const int card = NB_META_CARD(meta);       // CAT rows: card <= NB_CAT_MAX_CARD
     const int64_t s = (nid - first_id) >> 5;
     const int64_t q0 = nb_lds(cat_ptr + s), q1 = nb_lds(cat_ptr + s + 1);
     const int n = (int)((q1 - q0) >> 5);
@@ -229,7 +243,7 @@ __global__ void __launch_bounds__(256) k_gibbs_cat(SweepArgs a, const int64_t *_
         acc_z += s_e[k][tid];
         if (acc_z >= t) { pick = k; break; }
     }
-    a.val[nid] = (nb_val_t)pick;
+    a.val[nid] = (T)pick;
     if (!a.burnin) {
         if (card == 2) a.count[cs] += pick;                  // inference.py:30-31
         else a.count[cs + pick] += 1;                        // :32-33
@@ -244,11 +258,12 @@ __global__ void __launch_bounds__(256) k_gibbs_cat(SweepArgs a, const int64_t *_
 // Energies of every value over incidences [i0, i1) of the warp row `wr`, lanes striding over
 // them.  dataType 0, card <= 4: returned in e[] on all lanes.  Otherwise the per-value
 // energies land in the warp's shared array se[0..card).
-template <bool WIDE>
+// (card <= NB_MAX_CARD: wider rows take nb_warp_sample_wide)
+template <bool WIDE, class T>
 __device__ inline void nb_warp_row_energies(const uint32_t *__restrict__ wwords, const int64_t *__restrict__ wrow_ptr,
                                             const uint2 *__restrict__ inc, int64_t i0, int64_t i1,
                                             int64_t wr, uint32_t self, uint32_t meta,
-                                            const nb_val_t *__restrict__ vals, const double *__restrict__ weight,
+                                            const T *__restrict__ vals, const double *__restrict__ weight,
                                             double e[4], double *se)
 {
     const int lane = threadIdx.x & 31;
@@ -302,8 +317,8 @@ struct WarpTasks {
 };
 
 // Phase 1: one warp per task (a slice of one long row) -> partial energies.
-template <bool WIDE>
-__global__ void __launch_bounds__(32 * NB_WARPS_PER_BLOCK) k_gibbs_warp_partial(SweepArgs a, WarpTasks t, int kbeg, int kend)
+template <bool WIDE, class T>
+__global__ void __launch_bounds__(32 * NB_WARPS_PER_BLOCK) k_gibbs_warp_partial(SweepArgs<T> a, WarpTasks t, int kbeg, int kend)
 {
     __shared__ double s_e[NB_WARPS_PER_BLOCK][NB_MAX_CARD + 1];
     nb_wait_halo(a);
@@ -316,6 +331,7 @@ __global__ void __launch_bounds__(32 * NB_WARPS_PER_BLOCK) k_gibbs_warp_partial(
     const int evid = NB_META_EVID(meta), card = NB_META_CARD(meta);
     if (!NB_META_VALID(meta) || evid == 4) return;
     if (!(evid == 0 || a.sample_evidence)) return;
+    if (sizeof(T) > 1 && card == 0) return;     // cardinality above 255: sampled whole by k_gibbs_warp_finish
     const int64_t i0 = a.inc_ptr[wr] + t.task_beg[task];
     const int64_t i1 = min(i0 + (int64_t)NB_WARP_TASK, a.inc_ptr[wr + 1]);
     double e[4] = {0.0, 0.0, 0.0, 0.0};
@@ -329,8 +345,8 @@ __global__ void __launch_bounds__(32 * NB_WARPS_PER_BLOCK) k_gibbs_warp_partial(
 }
 
 // Phase 2: one warp per row sums its tasks' partials, samples, stores, tallies.
-template <bool WIDE>
-__global__ void __launch_bounds__(32 * NB_WARPS_PER_BLOCK) k_gibbs_warp_finish(SweepArgs a, WarpTasks t, int wbeg, int wend)
+template <bool WIDE, class T>
+__global__ void __launch_bounds__(32 * NB_WARPS_PER_BLOCK) k_gibbs_warp_finish(SweepArgs<T> a, WarpTasks t, int wbeg, int wend)
 {
     __shared__ double s_e[NB_WARPS_PER_BLOCK][NB_MAX_CARD + 1];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -341,6 +357,18 @@ __global__ void __launch_bounds__(32 * NB_WARPS_PER_BLOCK) k_gibbs_warp_finish(S
     const int evid = NB_META_EVID(meta), card = NB_META_CARD(meta);
     if (!NB_META_VALID(meta) || evid == 4) return;
     if (!(evid == 0 || a.sample_evidence)) return;
+    if (sizeof(T) > 1 && card == 0) {           // cardinality above 255 (2-byte graphs)
+        NbUniforms rng(a.rng_id[nid], a.epoch, NB_TAG_FREE, a.seed);
+        const NbRow r = nb_warp_row(a.wwords, a.wrow_ptr, wr);
+        const int k = nb_warp_sample_wide<WIDE>(r, (int)(a.wrow_ptr[wr + 1] - a.wrow_ptr[wr]), a.inc + a.inc_ptr[wr],
+                                                (int)(a.inc_ptr[wr + 1] - a.inc_ptr[wr]), (uint32_t)nid, meta,
+                                                nb_card(a, meta, nid), NbValsGlobal<T>(a.val), NbWtsGlobal{a.weight}, rng);
+        if (lane == 0) {
+            a.val[nid] = (T)k;
+            nb_tally(a, nid, nb_card(a, meta, nid), k);
+        }
+        return;
+    }
     // fixed summation tree (lane l takes tasks l, l + 32, ..., then the warp butterfly): the result
     // depends on the row's task list only, not on the launch or the partition
     const int64_t t0 = t.task_ptr[wr], t1 = t.task_ptr[wr + 1];
@@ -363,7 +391,7 @@ __global__ void __launch_bounds__(32 * NB_WARPS_PER_BLOCK) k_gibbs_warp_finish(S
     }
     if (lane == 0) {
         if (a.valbits && (int)a.val[nid] != k) atomicXor(a.valbits + (nid >> 5), 1u << (nid & 31));   // (all-Boolean graph)
-        a.val[nid] = (nb_val_t)k;
+        a.val[nid] = (T)k;
         nb_tally(a, nid, card, k);
     }
 }
@@ -384,13 +412,11 @@ static int fan_streams(nb_graph *g)
     return NB_OK;
 }
 
-int nb_launch_gibbs_color(nb_graph *g, int color, int burnin, int sample_evidence, uint64_t seed, uint64_t epoch)
+template <class T>
+static int launch_gibbs_color_t(nb_graph *g, int color, int burnin, int sample_evidence, uint64_t seed, uint64_t epoch)
 {
-    if (color < 0) NB_FAIL(NB_ERR_INVALID, "negative colour %d", color);
-    if (color >= g->n_colors) return NB_OK;   // partitioned graphs: a colour this rank does not own
     const NbColorRange &c = g->colors[(size_t)color];
-    if (!burnin && epoch != g->last_tally_epoch) { g->tally_bound++; g->last_tally_epoch = epoch; }
-    SweepArgs a = sweep_args(g, 0, burnin, sample_evidence, seed, epoch);
+    SweepArgs<T> a = sweep_args<T>(g, 0, burnin, sample_evidence, seed, epoch);
     if (c.f_end > c.f_beg || c.c_end > c.c_beg) NB_TRY(nb_refresh_inlined_weights(g));
     // streams of the five row classes (PAIR, FAST, CAT, GEN, WARP)
     const int64_t rows[5] = {c.p_end - c.p_beg, c.f_end - c.f_beg, c.c_end - c.c_beg, c.t_end - c.t_beg, c.w_end - c.w_beg};
@@ -414,26 +440,34 @@ int nb_launch_gibbs_color(nb_graph *g, int color, int burnin, int sample_evidenc
     if (c.p_end > c.p_beg) {
         unsigned grid = (unsigned)((c.p_end - c.p_beg + 255) / 256);
         uint32_t key = nb_fold_key(seed, epoch, NB_TAG_FREE);
-        if (a.valbits) k_gibbs_tt2<true><<<grid, 256, 0, st[0]>>>(a, g->d_tt2_ptr, g->d_tt2_common, g->d_tt2, c.p_beg, c.p_end, key);
-        else k_gibbs_tt2<false><<<grid, 256, 0, st[0]>>>(a, g->d_tt2_ptr, g->d_tt2_common, g->d_tt2, c.p_beg, c.p_end, key);
+        bool bits = false;
+        if constexpr (sizeof(T) == 1) {     // (the bit mirror exists on all-Boolean graphs only)
+            bits = a.valbits != nullptr;
+            if (bits) k_gibbs_tt2<true, T><<<grid, 256, 0, st[0]>>>(a, g->d_tt2_ptr, g->d_tt2_common, g->d_tt2, c.p_beg, c.p_end, key);
+        }
+        if (!bits) k_gibbs_tt2<false, T><<<grid, 256, 0, st[0]>>>(a, g->d_tt2_ptr, g->d_tt2_common, g->d_tt2, c.p_beg, c.p_end, key);
         g->launches++;
     }
     if (c.f_end > c.f_beg) {
         unsigned grid = (unsigned)((c.f_end - c.f_beg + 255) / 256);
         uint32_t key = nb_fold_key(seed, epoch, NB_TAG_FREE);
-        if (a.valbits) k_gibbs_tt<NB_TT_UNROLL_SWEEP, NB_TT_MINB, true><<<grid, 256, 0, st[1]>>>(a, g->d_tt_ptr, g->d_tt, c.f_beg, c.f_end, key);
-        else k_gibbs_tt<NB_TT_UNROLL_SWEEP, NB_TT_MINB, false><<<grid, 256, 0, st[1]>>>(a, g->d_tt_ptr, g->d_tt, c.f_beg, c.f_end, key);
+        bool bits = false;
+        if constexpr (sizeof(T) == 1) {
+            bits = a.valbits != nullptr;
+            if (bits) k_gibbs_tt<NB_TT_UNROLL_SWEEP, NB_TT_MINB, true, T><<<grid, 256, 0, st[1]>>>(a, g->d_tt_ptr, g->d_tt, c.f_beg, c.f_end, key);
+        }
+        if (!bits) k_gibbs_tt<NB_TT_UNROLL_SWEEP, NB_TT_MINB, false, T><<<grid, 256, 0, st[1]>>>(a, g->d_tt_ptr, g->d_tt, c.f_beg, c.f_end, key);
         g->launches++;
     }
     if (c.c_end > c.c_beg) {
         unsigned grid = (unsigned)((c.c_end - c.c_beg + 255) / 256);
-        k_gibbs_cat<<<grid, 256, 0, st[2]>>>(a, g->d_cat_ptr, g->d_cat, g->n_frows, c.c_beg, c.c_end);
+        k_gibbs_cat<T><<<grid, 256, 0, st[2]>>>(a, g->d_cat_ptr, g->d_cat, g->n_frows, c.c_beg, c.c_end);
         g->launches++;
     }
     if (c.t_end > c.t_beg) {
         unsigned grid = (unsigned)((c.t_end - c.t_beg + 255) / 256);
-        if (g->wide) k_gibbs_thread<true><<<grid, 256, 0, st[3]>>>(a, c.t_beg, c.t_end);
-        else k_gibbs_thread<false><<<grid, 256, 0, st[3]>>>(a, c.t_beg, c.t_end);
+        if (g->wide) k_gibbs_thread<true, T><<<grid, 256, 0, st[3]>>>(a, c.t_beg, c.t_end);
+        else k_gibbs_thread<false, T><<<grid, 256, 0, st[3]>>>(a, c.t_beg, c.t_end);
         g->launches++;
     }
     if (c.w_end > c.w_beg) {
@@ -441,11 +475,11 @@ int nb_launch_gibbs_color(nb_graph *g, int color, int burnin, int sample_evidenc
         unsigned grid1 = (unsigned)((c.k_end - c.k_beg + NB_WARPS_PER_BLOCK - 1) / NB_WARPS_PER_BLOCK);
         unsigned grid2 = (unsigned)((c.w_end - c.w_beg + NB_WARPS_PER_BLOCK - 1) / NB_WARPS_PER_BLOCK);
         if (g->wide) {
-            k_gibbs_warp_partial<true><<<grid1, 32 * NB_WARPS_PER_BLOCK, 0, st[4]>>>(a, t, c.k_beg, c.k_end);
-            k_gibbs_warp_finish<true><<<grid2, 32 * NB_WARPS_PER_BLOCK, 0, st[4]>>>(a, t, c.w_beg, c.w_end);
+            k_gibbs_warp_partial<true, T><<<grid1, 32 * NB_WARPS_PER_BLOCK, 0, st[4]>>>(a, t, c.k_beg, c.k_end);
+            k_gibbs_warp_finish<true, T><<<grid2, 32 * NB_WARPS_PER_BLOCK, 0, st[4]>>>(a, t, c.w_beg, c.w_end);
         } else {
-            k_gibbs_warp_partial<false><<<grid1, 32 * NB_WARPS_PER_BLOCK, 0, st[4]>>>(a, t, c.k_beg, c.k_end);
-            k_gibbs_warp_finish<false><<<grid2, 32 * NB_WARPS_PER_BLOCK, 0, st[4]>>>(a, t, c.w_beg, c.w_end);
+            k_gibbs_warp_partial<false, T><<<grid1, 32 * NB_WARPS_PER_BLOCK, 0, st[4]>>>(a, t, c.k_beg, c.k_end);
+            k_gibbs_warp_finish<false, T><<<grid2, 32 * NB_WARPS_PER_BLOCK, 0, st[4]>>>(a, t, c.w_beg, c.w_end);
         }
         g->launches += 2;
     }
@@ -458,19 +492,28 @@ int nb_launch_gibbs_color(nb_graph *g, int color, int burnin, int sample_evidenc
     return NB_OK;
 }
 
+int nb_launch_gibbs_color(nb_graph *g, int color, int burnin, int sample_evidence, uint64_t seed, uint64_t epoch)
+{
+    if (color < 0) NB_FAIL(NB_ERR_INVALID, "negative colour %d", color);
+    if (color >= g->n_colors) return NB_OK;   // partitioned graphs: a colour this rank does not own
+    if (!burnin && epoch != g->last_tally_epoch) { g->tally_bound++; g->last_tally_epoch = epoch; }
+    return g->value_bytes == 1 ? launch_gibbs_color_t<nb_val_t>(g, color, burnin, sample_evidence, seed, epoch)
+                               : launch_gibbs_color_t<nb_val16_t>(g, color, burnin, sample_evidence, seed, epoch);
+}
+
 // ---------------------------------------------------------------------------
 // potential() parity hook (inference.py:55-71): one thread per requested
 // variable walks its row once per value, summing in bucket order.
 // ---------------------------------------------------------------------------
-template <bool WIDE>
-__global__ void k_potentials(SweepArgs a, const int32_t *old2new, const int64_t *var_ids, int64_t n,
+template <bool WIDE, class T>
+__global__ void k_potentials(SweepArgs<T> a, const int32_t *old2new, const int64_t *var_ids, int64_t n,
                              const int64_t *out_offsets, double *out)
 {
     int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int64_t nid = old2new[var_ids[i]];
     const uint32_t meta = a.vmeta[nid];
-    const int card = NB_META_CARD(meta);
+    const int card = nb_card(a, meta, nid);
     NbRow r = nid < a.n_trows ? nb_thread_row(a.twords, a.slice_ptr, nid) : nb_warp_row(a.wwords, a.wrow_ptr, nid - a.n_trows);
     const int len = nid < a.n_trows ? NB_META_ROWLEN(meta)
                                     : (int)(a.wrow_ptr[nid - a.n_trows + 1] - a.wrow_ptr[nid - a.n_trows]);
@@ -508,10 +551,16 @@ int nb_run_potentials(nb_graph *g, int chain, const int64_t *var_ids, int64_t n,
     cudaMemcpyAsync(d_ids, var_ids, (size_t)n * 8, cudaMemcpyHostToDevice, g->stream);
     cudaMemcpyAsync(d_off, out_offsets, (size_t)n * 8, cudaMemcpyHostToDevice, g->stream);
     cudaMemsetAsync(d_out, 0, (size_t)n_out * 8, g->stream);
-    SweepArgs a = sweep_args(g, chain, 1, 1, 0, 0);
     unsigned grid = (unsigned)((n + 127) / 128);
-    if (g->wide) k_potentials<true><<<grid, 128, 0, g->stream>>>(a, g->d_old2new, d_ids, n, d_off, d_out);
-    else k_potentials<false><<<grid, 128, 0, g->stream>>>(a, g->d_old2new, d_ids, n, d_off, d_out);
+    if (g->value_bytes == 1) {
+        SweepArgs<nb_val_t> a = sweep_args<nb_val_t>(g, chain, 1, 1, 0, 0);
+        if (g->wide) k_potentials<true><<<grid, 128, 0, g->stream>>>(a, g->d_old2new, d_ids, n, d_off, d_out);
+        else k_potentials<false><<<grid, 128, 0, g->stream>>>(a, g->d_old2new, d_ids, n, d_off, d_out);
+    } else {
+        SweepArgs<nb_val16_t> a = sweep_args<nb_val16_t>(g, chain, 1, 1, 0, 0);
+        if (g->wide) k_potentials<true><<<grid, 128, 0, g->stream>>>(a, g->d_old2new, d_ids, n, d_off, d_out);
+        else k_potentials<false><<<grid, 128, 0, g->stream>>>(a, g->d_old2new, d_ids, n, d_off, d_out);
+    }
     cudaMemcpyAsync(out, d_out, (size_t)n_out * 8, cudaMemcpyDeviceToHost, g->stream);
     cudaError_t e = cudaStreamSynchronize(g->stream);
     cudaFree(d_ids); cudaFree(d_off); cudaFree(d_out);
@@ -539,7 +588,8 @@ struct RecordStreams {
     int64_t n_prows, n_frows, n_crows;
 };
 
-__global__ void k_potentials_records(SweepArgs a, RecordStreams R, const int32_t *old2new, const int64_t *var_ids, int64_t n,
+template <class T>
+__global__ void k_potentials_records(SweepArgs<T> a, RecordStreams R, const int32_t *old2new, const int64_t *var_ids, int64_t n,
                                      const int64_t *out_offsets, double *out, int32_t *row_class)
 {
     int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -565,7 +615,7 @@ __global__ void k_potentials_records(SweepArgs a, RecordStreams R, const int32_t
         for (int k = 0; k < NB_CAT_MAX_CARD; k++) e[k] = 0.0f;
         NbCatLocalAcc acc{e};
         nb_cat_energies(R.cat + q0 + (nid & 31), (int)((R.cat_ptr[sc + 1] - q0) >> 5), (uint32_t)nid, a.val, acc);
-        const int card = NB_META_CARD(meta);
+        const int card = NB_META_CARD(meta);   // CAT rows: card <= NB_CAT_MAX_CARD
         for (int k = 0; k < card; k++) o[k] = (double)e[k];
         row_class[i] = NB_CLASS_CAT;
     } else {
@@ -591,11 +641,17 @@ int nb_run_potentials_records(nb_graph *g, int chain, const int64_t *var_ids, in
     cudaMemcpyAsync(d_ids, var_ids, (size_t)n * 8, cudaMemcpyHostToDevice, g->stream);
     cudaMemcpyAsync(d_off, out_offsets, (size_t)n * 8, cudaMemcpyHostToDevice, g->stream);
     cudaMemsetAsync(d_out, 0, (size_t)n_out * 8, g->stream);
-    SweepArgs a = sweep_args(g, chain, 1, 1, 0, 0);
-    a.w_n = 0;
     RecordStreams R{g->d_tt2_ptr, g->d_tt2_common, g->d_tt2, g->d_tt_ptr, g->d_tt, g->d_cat_ptr, g->d_cat,
                     g->n_prows, g->n_frows, g->n_crows};
-    k_potentials_records<<<(unsigned)((n + 127) / 128), 128, 0, g->stream>>>(a, R, g->d_old2new, d_ids, n, d_off, d_out, d_cls);
+    if (g->value_bytes == 1) {
+        SweepArgs<nb_val_t> a = sweep_args<nb_val_t>(g, chain, 1, 1, 0, 0);
+        a.w_n = 0;
+        k_potentials_records<<<(unsigned)((n + 127) / 128), 128, 0, g->stream>>>(a, R, g->d_old2new, d_ids, n, d_off, d_out, d_cls);
+    } else {
+        SweepArgs<nb_val16_t> a = sweep_args<nb_val16_t>(g, chain, 1, 1, 0, 0);
+        a.w_n = 0;
+        k_potentials_records<<<(unsigned)((n + 127) / 128), 128, 0, g->stream>>>(a, R, g->d_old2new, d_ids, n, d_off, d_out, d_cls);
+    }
     cudaMemcpyAsync(out, d_out, (size_t)n_out * 8, cudaMemcpyDeviceToHost, g->stream);
     cudaMemcpyAsync(row_class, d_cls, (size_t)n * 4, cudaMemcpyDeviceToHost, g->stream);
     cudaError_t e = cudaStreamSynchronize(g->stream);

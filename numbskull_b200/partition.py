@@ -324,10 +324,18 @@ class Exchange(object):
 
 
 # --------------------------------------------------------------------------- runner
+def _check_single_byte(variable):
+    """The halo moves one byte per value: graphs with a cardinality above 255 (2-byte device
+    values) run on one GPU only."""
+    if len(variable) and int(variable["cardinality"].max()) > 255:
+        raise ValueError("cardinalities above 255 are single-GPU only")
+
+
 class PartitionedGibbs(object):
     """One rank of a partitioned factor graph on its GPU."""
 
     def __init__(self, local, n_global, rank, world, device, seed, color_seed=0x5EED, group=None):
+        _check_single_byte(local["variable"])
         import torch
         import torch.distributed as dist
         from . import _lib
@@ -667,6 +675,7 @@ def partition_graph(weight, variable, factor, fmap, rank, world, device, seed, g
     the placement ``owner[v]`` -- e.g. :func:`owners_from_salt_keys` (the reference's partition
     keys) or :func:`locality_owners`.  Samples do not depend on the placement: colours and Philox
     streams are functions of the global ids."""
+    _check_single_byte(variable)
     if owner is None:
         # contiguous blocks: the same cut as extract_local (the tests compare them), made by host threads
         bounds = block_bounds(len(variable), world)

@@ -280,6 +280,66 @@ def categorical(nvar, card=16, factors_per_var=3, rng=None, n_weights=1 << 20,
     return _pack(weight, variable, factor, fmap)
 
 
+def wide_categorical(n_mentions, card=1000, cands=32, feats=4, couplings=4, rng=None, n_weights=1 << 12,
+                     evidence_frac=0.2):
+    """Entity-linking shape with cardinalities above 255 (2-byte device values): ``n_mentions``
+    dataType 1 variables of cardinality ``card`` (a mention over its candidate entities), each with
+    ``cands`` candidate values drawn from ``card``.  Every candidate c of a mention m has one
+    EQUAL_CAT_CONST(15) prior (m == c) and ``feats`` AND_CAT(12) features (m == c and f == 1) on
+    Boolean evidence variables f; ``couplings`` AND_CAT factors per mention tie it to another
+    mention on a shared candidate (both == c).  Weights are tied into ``n_weights`` learnable
+    ids; ``evidence_frac`` of the mentions are labelled with one of their candidates.  The values
+    a mention takes outside its candidates sit in empty buckets.  Variables: mentions first, then
+    ``n_mentions`` feature variables."""
+    rng = rng or np.random.default_rng(0)
+    M, F = int(n_mentions), int(n_mentions)
+    weight = np.zeros(n_weights, Weight)
+    weight["initialValue"] = rng.normal(0.0, 0.5, n_weights)
+    variable = np.concatenate((_variables(M, data_type=1, cardinality=card), _variables(F, is_evidence=1)))
+    variable["initialValue"][M:] = rng.integers(0, 2, F)
+    cands = min(cands, card)
+    # distinct candidates: evenly spaced values from a random start
+    cand = np.sort((rng.integers(0, card, M)[:, None] + np.arange(cands) * (card // cands)) % card, axis=1)
+    lab = rng.random(M) < evidence_frac
+    variable["isEvidence"][:M] = lab
+    variable["initialValue"][:M] = cand[np.arange(M), rng.integers(0, cands, M)]
+    m_of = np.repeat(np.arange(M, dtype=np.int64), cands)
+    c_of = cand.reshape(-1)
+    slot = np.tile(np.arange(cands, dtype=np.int64), M)
+    # priors: m == c
+    n_pri = M * cands
+    w_pri = (slot * 7 + c_of) % n_weights
+    # features: m == c and f == 1
+    n_feat = n_pri * feats
+    fm_m = np.repeat(m_of, feats)
+    fm_c = np.repeat(c_of, feats)
+    fvar = M + rng.integers(0, F, n_feat)
+    w_feat = (np.repeat(c_of, feats) * 131 + np.tile(np.arange(feats), n_pri) * 17 + 1) % n_weights
+    # couplings: m == c and m' == c on a candidate c of m
+    n_cpl = M * couplings
+    a_m = np.repeat(np.arange(M, dtype=np.int64), couplings)
+    a_c = cand[a_m, rng.integers(0, cands, n_cpl)]
+    b_m = (a_m + rng.integers(1, max(M, 2), n_cpl)) % max(M, 1)
+    w_cpl = np.full(n_cpl, n_weights - 1, np.int64)
+    func = np.concatenate((np.full(n_pri, FUNC["EQUAL_CAT_CONST"]), np.full(n_feat + n_cpl, FUNC["AND_CAT"])))
+    arity = np.concatenate((np.ones(n_pri, np.int64), np.full(n_feat + n_cpl, 2, np.int64)))
+    factor = _factors(func, np.concatenate((w_pri, w_feat, w_cpl)), arity)
+    fmap = np.zeros(n_pri + 2 * (n_feat + n_cpl), FactorToVar)
+    fmap["vid"][:n_pri] = m_of
+    fmap["dense_equal_to"][:n_pri] = c_of
+    o = n_pri
+    fmap["vid"][o:o + 2 * n_feat:2] = fm_m
+    fmap["dense_equal_to"][o:o + 2 * n_feat:2] = fm_c
+    fmap["vid"][o + 1:o + 2 * n_feat:2] = fvar
+    fmap["dense_equal_to"][o + 1:o + 2 * n_feat:2] = 1
+    o += 2 * n_feat
+    fmap["vid"][o::2] = a_m
+    fmap["vid"][o + 1::2] = b_m
+    fmap["dense_equal_to"][o::2] = a_c
+    fmap["dense_equal_to"][o + 1::2] = a_c
+    return _pack(weight, variable, factor, fmap)
+
+
 BOOLEAN_FUNCS = (0, 1, 2, 3, 4, 7, 8, 9)
 
 
