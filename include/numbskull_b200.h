@@ -275,6 +275,9 @@ int nb_scatter_values_dev(nb_graph *g, int chain, const int32_t *dev_local_ids, 
 int nb_learn_blocks(nb_graph *g, double stepsize, int learn_non_evidence, int64_t batch_visits, int *n_blocks);
 int nb_learn_color_phase(nb_graph *g, int color, int block, int n_blocks, double stepsize, int regularization,
                          double reg_param, double truncation, int learn_non_evidence, uint64_t seed, int64_t epoch);
+/* Parity hook: the ORIGINAL ids of the variables cell (block, colour) holds (`ids` has room for
+ * n_variable entries; *n receives the count) -- which variables nb_learn_color_phase samples. */
+int nb_learn_cell_ids(nb_graph *g, int color, int block, int n_blocks, int64_t *ids, int64_t *n);
 /* Distributed Jones-Plassmann (graphs created with deferred_coloring): one round over the
  * owned, still uncoloured variables; ghosts are consulted through the colours last scattered
  * in.  *remaining != 0 iff an owned variable is still uncoloured after the round. */

@@ -103,6 +103,7 @@ SIGNATURES = {
     "nb_scatter_values_dev": (C.c_int, [_P, C.c_int, _P, _I64, _P]),
     "nb_learn_color_phase": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _DBL, C.c_int, _DBL, _DBL, C.c_int, _U64, _I64]),
     "nb_learn_blocks": (C.c_int, [_P, _DBL, C.c_int, _I64, C.POINTER(C.c_int)]),
+    "nb_learn_cell_ids": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, C.POINTER(_I64)]),
     "nb_color_round": (C.c_int, [_P, C.POINTER(_I64)]),
     "nb_color_restart": (C.c_int, [_P, C.c_int]),
     "nb_split_colors": (C.c_int, [_P, _P, _I64]),

@@ -753,6 +753,13 @@ extern "C" int nb_learn_blocks(nb_graph *g, double stepsize, int learn_non_evide
     return nb_learn_block_count(g, stepsize, learn_non_evidence, batch_visits, n_blocks);
 }
 
+extern "C" int nb_learn_cell_ids(nb_graph *g, int color, int block, int n_blocks, int64_t *ids, int64_t *n)
+{
+    NB_CUDA(cudaSetDevice(g->device));
+    NB_TRY(check_runnable(g));
+    return nb_learn_cell_id_list(g, color, block, n_blocks, ids, n);
+}
+
 extern "C" int nb_color_round(nb_graph *g, int64_t *remaining)
 {
     NB_CUDA(cudaSetDevice(g->device));

@@ -385,6 +385,7 @@ int nb_build_relabel_colors(nb_graph *g, const int32_t *map, int n);
 int nb_learn_color(nb_graph *g, int color, int block, int n_blocks, double step, int regularization, double reg_param,
                    double truncation, int learn_non_evidence, uint64_t seed, uint64_t epoch);
 int nb_learn_block_count(nb_graph *g, double step, int learn_non_evidence, int64_t batch_visits, int *n_blocks);
+int nb_learn_cell_id_list(nb_graph *g, int color, int block, int n_blocks, int64_t *ids, int64_t *n);
 
 // sweeps (nb_sweep.cu / nb_learn.cu)
 int nb_launch_gibbs_color(nb_graph *g, int color, int burnin, int sample_evidence, uint64_t seed,

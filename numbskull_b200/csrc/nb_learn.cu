@@ -1310,6 +1310,28 @@ int nb_learn_color(nb_graph *g, int color, int block, int n_blocks, double step,
                                      learn_non_evidence, seed, epoch);
 }
 
+// Parity hook: the ORIGINAL ids of the variables that cell (block, colour) of an epoch cut into
+// n_blocks blocks holds, class by class in new-id order (the plan nb_learn_color walks).
+int nb_learn_cell_id_list(nb_graph *g, int color, int block, int n_blocks, int64_t *ids, int64_t *n)
+{
+    if (n_blocks < 1 || block < 0 || block >= n_blocks) NB_FAIL(NB_ERR_INVALID, "block %d of %d", block, n_blocks);
+    *n = 0;
+    if (color < 0 || color >= g->n_colors) return NB_OK;
+    CellPlan hp = make_plan(g, n_blocks);
+    hp.win_start = g->win_start.data();            // host copy of the window table
+    std::vector<int32_t> n2o;
+    for (int cls = 0; cls < NB_N_CLASSES; cls++) {
+        int beg = 0, end = 0;
+        nb_plan_range(hp, cls, color, block, beg, end);
+        if (end <= beg) continue;
+        n2o.resize((size_t)(end - beg));
+        NB_CUDA(cudaMemcpy(n2o.data(), g->d_new2old + beg, n2o.size() * 4, cudaMemcpyDeviceToHost));
+        for (int32_t v : n2o)
+            if (v >= 0) ids[(*n)++] = v;
+    }
+    return NB_OK;
+}
+
 template <class T>
 static int run_learn_t(nb_graph *g, int64_t n_epochs, double *stepsize, double decay, int regularization, double reg_param,
                        double truncation, int learn_non_evidence, uint64_t seed, int64_t batch_visits)

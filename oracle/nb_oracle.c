@@ -628,3 +628,299 @@ int nbo_exact_marginals(const nbo_graph *g, int clamp_evidence, double *out, dou
 
 int nbo_sizeof_rng(void) { return (int)sizeof(nbo_rng); }
 int nbo_sizeof_graph(void) { return (int)sizeof(nbo_graph); }
+
+/* ------------------------------------------------------------------ */
+/* Counter-based streams of the CUDA library, restated from the        */
+/* specification (Salmon et al., SC'11; Random123 constants) so that   */
+/* tests can replay every draw of a sweep on the host.  The device     */
+/* headers are deliberately NOT included: this is a second,            */
+/* independent implementation.                                         */
+/* ------------------------------------------------------------------ */
+void nbo_philox4x32(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4])
+{
+    uint32_t x0 = ctr[0], x1 = ctr[1], x2 = ctr[2], x3 = ctr[3], k0 = key[0], k1 = key[1];
+    for (int r = 0; r < 10; r++) {
+        uint64_t a = (uint64_t)0xD2511F53u * x0, b = (uint64_t)0xCD9E8D57u * x2;
+        uint32_t y0 = (uint32_t)(b >> 32) ^ x1 ^ k0, y1 = (uint32_t)b;
+        uint32_t y2 = (uint32_t)(a >> 32) ^ x3 ^ k1, y3 = (uint32_t)a;
+        x0 = y0; x1 = y1; x2 = y2; x3 = y3;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+    out[0] = x0; out[1] = x1; out[2] = x2; out[3] = x3;
+}
+
+void nbo_philox2x32(const uint32_t ctr[2], uint32_t key, uint32_t out[2])
+{
+    uint32_t x0 = ctr[0], x1 = ctr[1];
+    for (int r = 0; r < 10; r++) {
+        uint64_t a = (uint64_t)0xD256D193u * x0;
+        uint32_t y0 = (uint32_t)(a >> 32) ^ x1 ^ key;
+        x1 = (uint32_t)a;
+        x0 = y0;
+        key += 0x9E3779B9u;
+    }
+    out[0] = x0; out[1] = x1;
+}
+
+/* 53-bit uniform in [0, 1): the top 53 bits of hi:lo */
+double nbo_u53(uint32_t hi, uint32_t lo)
+{
+    return (double)((((uint64_t)hi << 32) | lo) >> 11) / 9007199254740992.0;
+}
+
+/* 32-bit key of the single-draw (Philox2x32) streams: seed, the epoch bits above 32 and the tag
+ * mixed by the MurmurHash3 finaliser half, folded to 32 bits. */
+uint32_t nbo_fold_key(uint64_t seed, uint64_t epoch, uint32_t tag)
+{
+    uint64_t x = seed ^ ((epoch >> 32) * 0x9E3779B97F4A7C15ull) ^ ((uint64_t)tag << 56);
+    x ^= x >> 33;
+    x *= 0xFF51AFD7ED558CCDull;
+    x ^= x >> 33;
+    return (uint32_t)x ^ (uint32_t)(x >> 32);
+}
+
+/* The single uniform of a record row: counter (id, low epoch word), folded key. */
+double nbo_philox2x32_u53(uint32_t id, uint64_t epoch, uint64_t seed, uint32_t tag)
+{
+    uint32_t c[2] = {id, (uint32_t)epoch}, o[2];
+    nbo_philox2x32(c, nbo_fold_key(seed, epoch, tag), o);
+    return nbo_u53(o[0], o[1]);
+}
+
+/* The multi-draw stream of one (variable, epoch, tag): counter (id, low epoch word,
+ * epoch bits 32..47 | tag << 24, block), key = seed; the four words of a block are read in
+ * order, then block++. */
+typedef struct { uint32_t c[3]; uint32_t key[2]; uint32_t block; uint32_t r[4]; int used; } nbo_stream;
+
+void nbo_stream_init(nbo_stream *s, uint32_t id, uint64_t epoch, uint32_t tag, uint64_t seed)
+{
+    s->c[0] = id;
+    s->c[1] = (uint32_t)epoch;
+    s->c[2] = (uint32_t)((epoch >> 32) & 0xFFFFu) | (tag << 24);
+    s->key[0] = (uint32_t)seed;
+    s->key[1] = (uint32_t)(seed >> 32);
+    s->block = 0;
+    s->used = 4;
+}
+
+uint32_t nbo_stream_word(nbo_stream *s)
+{
+    if (s->used == 4) {
+        uint32_t ctr[4] = {s->c[0], s->c[1], s->c[2], s->block++};
+        nbo_philox4x32(ctr, s->key, s->r);
+        s->used = 0;
+    }
+    return s->r[s->used++];
+}
+
+/* two words, the first one high: the 53-bit draw of small-cardinality rows */
+double nbo_stream_next(nbo_stream *s)
+{
+    uint32_t hi = nbo_stream_word(s);
+    return nbo_u53(hi, nbo_stream_word(s));
+}
+
+/* one word, centred: the per-value decisions of the reservoir */
+double nbo_stream_next32(nbo_stream *s)
+{
+    return ((double)nbo_stream_word(s) + 0.5) / 4294967296.0;
+}
+
+int nbo_sizeof_stream(void) { return (int)sizeof(nbo_stream); }
+
+/* ------------------------------------------------------------------ */
+/* float64 decision rules.  Each returns the pick and, through         */
+/* *margin, how far the uniform was from changing it (in units of the  */
+/* uniform): a float32 implementation of the same rule may only pick   */
+/* differently when the margin is of the order of its rounding.        */
+/* ------------------------------------------------------------------ */
+static double dmin(double a, double b) { return a < b ? a : b; }
+
+/* Boolean rule: P(0) = 1 / (1 + exp(e1 - e0)), pick 0 iff u <= P(0) */
+int64_t nbo_draw_bool(double e0, double e1, double u, double *margin)
+{
+    double p0 = 1.0 / (1.0 + exp(e1 - e0));
+    *margin = fabs(u - p0);
+    return u <= p0 ? 0 : 1;
+}
+
+/* inverse CDF (draw_sample, inference.py:36-52, maximum subtracted): the first k whose cumulative
+ * mass reaches u * total; card - 1 if none does.  Margin: distance of u to the nearest boundary. */
+int64_t nbo_draw_cdf(const double *e, int64_t card, double u, double *margin)
+{
+    double m = e[0], tot = 0.0, acc = 0.0;
+    for (int64_t k = 1; k < card; k++) if (e[k] > m) m = e[k];
+    for (int64_t k = 0; k < card; k++) tot += exp(e[k] - m);
+    int64_t pick = -1;
+    *margin = INFINITY;
+    for (int64_t k = 0; k < card; k++) {
+        acc += exp(e[k] - m);
+        if (k < card - 1) *margin = dmin(*margin, fabs(acc / tot - u));
+        if (pick < 0 && acc >= u * tot) pick = k;
+    }
+    return pick < 0 ? card - 1 : pick;
+}
+
+/* Weighted reservoir with a running maximum: group j (energy e, `mult` values) replaces the pick
+ * when u * s < t, t = mult * exp(e - m) its mass and s the mass seen so far including it.  The first
+ * group always takes the pick (its uniform is still consumed). */
+typedef struct { double m, s; int empty; } nbo_reservoir;
+
+static int reservoir_add(nbo_reservoir *r, double e, double mult, double u, double *margin)
+{
+    if (r->empty) { r->m = e; r->s = mult; r->empty = 0; return 1; }
+    double t;
+    if (e > r->m) { r->s = r->s * exp(r->m - e) + mult; r->m = e; t = mult; }
+    else { t = mult * exp(e - r->m); r->s += t; }
+    *margin = dmin(*margin, fabs(u - t / r->s));
+    return u * r->s < t;
+}
+
+/* Streaming categorical draw.  nonempty == NULL: every value is its own group, in ascending order
+ * (dataType 0 rows, warp rows).  Otherwise the values with nonempty[k] in ascending order, then ONE
+ * group of the n_empty remaining values (energy 0), inside which a second uniform picks the
+ * floor(u * n_empty)-th empty value. */
+int64_t nbo_draw_reservoir(const double *e, int64_t card, const uint8_t *nonempty, nbo_stream *s, double *margin)
+{
+    nbo_reservoir r = {0.0, 0.0, 1};
+    int64_t pick = 0, n_empty = 0;
+    *margin = INFINITY;
+    for (int64_t k = 0; k < card; k++) {
+        if (nonempty && !nonempty[k]) { n_empty++; continue; }
+        if (reservoir_add(&r, e[k], 1.0, nbo_stream_next32(s), margin)) pick = k;
+    }
+    if (n_empty > 0 && reservoir_add(&r, 0.0, (double)n_empty, nbo_stream_next32(s), margin)) {
+        double x = nbo_stream_next32(s) * (double)n_empty;
+        int64_t j = (int64_t)x;
+        if (j > n_empty - 1) j = n_empty - 1;
+        *margin = dmin(*margin, dmin(x - floor(x), ceil(x) - x) / (double)n_empty);
+        for (int64_t k = 0; k < card; k++)
+            if (!nonempty[k] && j-- == 0) { pick = k; break; }
+    }
+    return pick;
+}
+
+/* ------------------------------------------------------------------ */
+/* Batched entries for the sweep replay.                               */
+/* ------------------------------------------------------------------ */
+/* potential(v, k) for every value of each listed variable, under chain 0 (var_value) or 1
+ * (var_value_evid); variable ids[i] writes cardinality entries from out[off], off running. */
+int nbo_energies(const nbo_graph *g, int chain, const int64_t *ids, int64_t n, double *out)
+{
+    int err = 0;
+    const int64_t *vals = chain ? g->var_value_evid : g->var_value;
+    int64_t off = 0;
+    for (int64_t i = 0; i < n; i++) {
+        int64_t card = g->variable[ids[i]].cardinality;
+        for (int64_t k = 0; k < card; k++) out[off++] = nbo_potential(g, ids[i], k, vals, &err);
+    }
+    return err;
+}
+
+/* Row classes of the CUDA library, and the rule each one samples with:
+ *   PAIR / FAST (0, 1): Boolean rule, one Philox2x32 uniform;
+ *   CAT (2):            inverse CDF, one Philox2x32 uniform;
+ *   GEN (3):            multi-draw stream: dataType 0 with cardinality <= 4 takes one 53-bit draw
+ *                       (Boolean rule for cardinality 2, inverse CDF otherwise); other dataType 0
+ *                       rows a reservoir over every value; dataType 1 rows a reservoir over the
+ *                       values with a non-empty bucket, then the group of the empty ones;
+ *   WARP (4):           multi-draw stream: one 53-bit draw as GEN for small dataType 0 rows,
+ *                       otherwise a reservoir over every value;
+ *   WIDE (5):           warp rows above cardinality 255: the GEN rule. */
+enum { NBO_PAIR = 0, NBO_FAST = 1, NBO_CAT = 2, NBO_GEN = 3, NBO_WARP = 4, NBO_WIDE = 5 };
+
+static int64_t draw_one(const nbo_graph *g, int64_t v, const double *e, int cls, uint32_t id, uint64_t seed,
+                        uint64_t epoch, uint32_t tag, uint8_t *nonempty, double *margin)
+{
+    const nbo_variable *var = &g->variable[v];
+    int64_t card = var->cardinality;
+    if (cls == NBO_PAIR || cls == NBO_FAST)
+        return nbo_draw_bool(e[0], e[1], nbo_philox2x32_u53(id, epoch, seed, tag), margin);
+    if (cls == NBO_CAT) return nbo_draw_cdf(e, card, nbo_philox2x32_u53(id, epoch, seed, tag), margin);
+    nbo_stream s;
+    nbo_stream_init(&s, id, epoch, tag, seed);
+    if (var->dataType == 0 && card <= 4) {
+        double u = nbo_stream_next(&s);
+        if (card == 2) return nbo_draw_bool(e[0], e[1], u, margin);
+        return nbo_draw_cdf(e, card, u, margin);
+    }
+    if (var->dataType == 0 || cls == NBO_WARP) return nbo_draw_reservoir(e, card, NULL, &s, margin);
+    for (int64_t k = 0; k < card; k++) nonempty[k] = g->vmap[var->vtf_offset + k].factor_index_length > 0;
+    return nbo_draw_reservoir(e, card, nonempty, &s, margin);
+}
+
+/* Replays the draw of each listed variable from its float64 energies under `chain`.  cls[i] is
+ * the row class of ids[i], rng_id[i] its stream id (low 32 bits of the global id). */
+int nbo_replay_draws(const nbo_graph *g, int chain, const int64_t *ids, int64_t n, const int32_t *cls,
+                     const uint32_t *rng_id, uint64_t seed, uint64_t epoch, uint32_t tag, int64_t *pick,
+                     double *margin)
+{
+    int err = 0;
+    const int64_t *vals = chain ? g->var_value_evid : g->var_value;
+    int64_t maxcard = 1;
+    for (int64_t i = 0; i < n; i++)
+        if (g->variable[ids[i]].cardinality > maxcard) maxcard = g->variable[ids[i]].cardinality;
+    double *e = (double *)malloc(sizeof(double) * (size_t)maxcard);
+    uint8_t *ne = (uint8_t *)malloc((size_t)maxcard);
+    for (int64_t i = 0; i < n; i++) {
+        int64_t v = ids[i], card = g->variable[v].cardinality;
+        for (int64_t k = 0; k < card; k++) e[k] = nbo_potential(g, v, k, vals, &err);
+        pick[i] = draw_one(g, v, e, cls[i], rng_id[i], seed, epoch, tag, ne, &margin[i]);
+    }
+    free(e);
+    free(ne);
+    return err;
+}
+
+/* The first uniform of each listed stream: family 0 = Philox2x32 (record rows), 1 = the multi-draw
+ * stream's 53-bit draw.  Used for the truncation draws of L1 learning. */
+void nbo_first_uniforms(const uint32_t *rng_id, int64_t n, const int32_t *family, uint64_t seed, uint64_t epoch,
+                        uint32_t tag, double *out)
+{
+    for (int64_t i = 0; i < n; i++) {
+        if (family[i] == 0) { out[i] = nbo_philox2x32_u53(rng_id[i], epoch, seed, tag); continue; }
+        nbo_stream s;
+        nbo_stream_init(&s, rng_id[i], epoch, tag, seed);
+        out[i] = nbo_stream_next(&s);
+    }
+}
+
+/* learning.py:73-108 for a batch of variables whose evidence-chain value is ev[i] and free-chain
+ * value prop[i]: every learnable factor of the buckets of ev and prop (once per factor) adds
+ * (f(prop | var_value) - f(ev | var_value_evid)) * featureValue, rounded to 2^-20 units as the
+ * library reduces it, to G_fix[weightId], and cnt_inc[i] to cnt[weightId]. */
+int nbo_cell_gradients(const nbo_graph *g, const int64_t *ids, int64_t n, const int64_t *ev, const int64_t *prop,
+                       const uint32_t *cnt_inc, int64_t *G_fix, int64_t *cnt)
+{
+    int err = 0;
+    int64_t maxb = 1;
+    for (int64_t i = 0; i < g->n_vmap; i++)
+        if (g->vmap[i].factor_index_length > maxb) maxb = g->vmap[i].factor_index_length;
+    int64_t *fids = (int64_t *)malloc(sizeof(int64_t) * (size_t)(2 * maxb));
+    for (int64_t i = 0; i < n; i++) {
+        int64_t v = ids[i], s0, e0, s1, e1, m;
+        bucket_range(g, v, ev[i], &s0, &e0);
+        memcpy(fids, g->factor_index + s0, (size_t)(e0 - s0) * sizeof(int64_t));
+        m = e0 - s0;
+        if (ev[i] != prop[i]) {
+            bucket_range(g, v, prop[i], &s1, &e1);
+            memcpy(fids + m, g->factor_index + s1, (size_t)(e1 - s1) * sizeof(int64_t));
+            m += e1 - s1;
+            qsort(fids, (size_t)m, sizeof(int64_t), cmp_i64);
+        }
+        int64_t last = -1;
+        for (int64_t j = 0; j < m; j++) {
+            int64_t fid = fids[j];
+            if (fid == last) continue;
+            last = fid;
+            int64_t wid = g->factor[fid].weightId;
+            if (g->weight[wid].isFixed) continue;
+            double p1 = nbo_eval_factor(g, fid, v, prop[i], g->var_value, &err);
+            double p0 = nbo_eval_factor(g, fid, v, ev[i], g->var_value_evid, &err);
+            G_fix[wid] += llrint((p1 - p0) * g->factor[fid].featureValue * 1048576.0);
+            cnt[wid] += cnt_inc[i];
+        }
+    }
+    free(fids);
+    return err;
+}
