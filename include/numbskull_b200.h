@@ -331,6 +331,33 @@ int nb_p2p_close(nb_graph *g);
 int nb_set_stream(nb_graph *g, void *cuda_stream);
 int nb_begin_epoch(nb_graph *g, int64_t *epoch); /* returns and advances the sweep counter */
 
+/* ------------------- in-place record edits of a built graph ------------------- */
+/* The reference reads variable.isEvidence, variable.initialValue and weight.isFixed on every sweep
+ * (inference.py:21-24, learning.py:60-61,98-99), so its callers flip them between calls.  None of
+ * them changes the layout of the device graph: these calls patch the words that carry them and
+ * leave the graph exactly as a rebuild from the edited records would (nb_graph_digest). */
+/* Edit variables in place (ORIGINAL ids).  A NULL array leaves that field alone.  isEvidence is
+ * packed as the build packs it; the stored initialValue is the given one where it lies in
+ * [0, cardinality), else 0.  value != NULL also stores value[i] into BOTH chains, as construction
+ * does.  A duplicated id takes its last entry.  All or nothing: every entry is validated before
+ * anything is written; NB_ERR_INVALID for an id out of range, isEvidence 4 or a variable that has
+ * it (ghosts belong to the partitioner), an evidence variable (isEvidence 1) whose initialValue lies
+ * outside [0, cardinality) -- without a new initialValue the stored one counts, and an
+ * out-of-domain initialValue was stored as 0 -- and a value outside [0, cardinality).  O(n): no
+ * per-variable array crosses PCIe. */
+int nb_update_variables(nb_graph *g, const int64_t *var_ids, int64_t n, const int8_t *is_evidence,
+                        const int64_t *initial_value, const int64_t *value);
+/* Set weight.isFixed (0 / non-zero) of the listed weights: d_wfixed and the fixed bit of every
+ * record that carries one of them.  The last entry of a duplicated id wins; nothing is launched when
+ * no flag changes. */
+int nb_update_weights_fixed(nb_graph *g, const int64_t *weight_ids, int64_t n, const uint8_t *is_fixed);
+/* Parity hook: one 64-bit digest per device array a build derives from the records, in this order
+ * (an array a graph does not have hashes as 0): vmeta, vinit, vcard, v_evid, v_init, wfixed,
+ * thread-row words, warp-row words, tt, tt_wid, tt2, tt2_common, cat, cat_wid, new2old.  Each is
+ * the sum mod 2^64 of a hash of (position, element).  `digest` has room for n >= NB_DIGEST_ARRAYS. */
+#define NB_DIGEST_ARRAYS 15
+int nb_graph_digest(const nb_graph *g, uint64_t *digest, int n);
+
 #ifdef __cplusplus
 }
 #endif

@@ -124,7 +124,14 @@ SIGNATURES = {
     "nb_p2p_close": (C.c_int, [_P]),
     "nb_set_stream": (C.c_int, [_P, _P]),
     "nb_begin_epoch": (C.c_int, [_P, C.POINTER(_I64)]),
+    "nb_update_variables": (C.c_int, [_P, _P, _I64, _P, _P, _P]),
+    "nb_update_weights_fixed": (C.c_int, [_P, _P, _I64, _P]),
+    "nb_graph_digest": (C.c_int, [_P, _P, C.c_int]),
 }
+
+# nb_graph_digest order (include/numbskull_b200.h)
+DIGEST_ARRAYS = ("vmeta", "vinit", "vcard", "v_evid", "v_init", "wfixed", "twords", "wwords", "tt", "tt_wid",
+                 "tt2", "tt2_common", "cat", "cat_wid", "new2old")
 
 
 def build(force=False, verbose=False):

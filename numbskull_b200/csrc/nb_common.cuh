@@ -347,7 +347,8 @@ struct nb_graph {
     std::vector<int32_t> win_start;    // [NB_N_CLASSES * (n_colors + 1)][n_win + 1] first new id of each window per group
     std::vector<uint8_t> learn_long_rows;  // host copy of d_long_rows
     std::vector<int64_t> learn_vmax;   // per colour: max gradient visits of one weight
-    int learn_vmax_flag = -1;
+    int learn_vmax_flag = -1;         // learn_non_evidence the bounds were computed for; -1 = none
+    std::vector<uint8_t> h_wfixed;     // host copy of d_wfixed, fetched by the first nb_update_weights_fixed
     std::vector<NbColorRange> colors;
     std::vector<void *> allocs;
 };

@@ -85,6 +85,11 @@ __device__ __forceinline__ NbRow nb_thread_row(const uint32_t *twords, const int
 {
     return NbRow{twords + ((slice_ptr[nid >> 5] + (nid & 31)) << 2), 1};
 }
+// address of word i of thread-path row nid (the SELL-32 layout NbRow::w reads), for in-place patches
+__device__ __forceinline__ uint32_t *nb_thread_row_word(uint32_t *twords, const int64_t *slice_ptr, int64_t nid, int i)
+{
+    return twords + ((slice_ptr[nid >> 5] + (nid & 31)) << 2) + (((size_t)(i >> 2)) << 7) + (i & 3);
+}
 __device__ __forceinline__ NbRow nb_warp_row(const uint32_t *wwords, const int64_t *wrow_ptr, int64_t wr)
 {
     return NbRow{wwords + wrow_ptr[wr], 0};

@@ -23,8 +23,13 @@ the public arrays (``var_value``, ``var_value_evid``, ``weight_value``,
 * ``weight_value`` is small: it is compared with the last uploaded copy on
   entry and downloaded after every ``learn``;
 * the record arrays (``variable`` / ``weight`` / ``factor`` / ``fmap``) are read
-  once, when the device graph is built; call :meth:`invalidate` after editing
-  them (e.g. flipping ``isEvidence``).
+  once, when the device graph is built.  ``variable.isEvidence``,
+  ``variable.initialValue`` and ``weight.isFixed`` -- the fields the reference
+  reads on every sweep -- are edited in place with :meth:`update_variables` /
+  :meth:`update_weights`, which write the records and patch the device graph
+  without a rebuild.  Any other record edit (cardinality, dataType,
+  featureValue, weightId, factors, fmap), or an edit of those fields made
+  directly in the arrays, needs :meth:`invalidate`.
 """
 from __future__ import print_function
 
@@ -363,6 +368,105 @@ class FactorGraph(object):
         self._dev_row = {k: None for k in self._dev_row}
         self._count_dev_valid = True       # a rebuilt graph starts with zero tallies, like count
         self._pristine = False
+
+    # ------------------------------------------------------------------
+    # in-place record edits
+    # ------------------------------------------------------------------
+    @staticmethod
+    def _last_wins(ids, n_records, what, *columns):
+        """Ids in range, one entry per id (the last occurrence, as numpy's a[ids] = x) in increasing
+        id order, and the matching entries of each column (None stays None)."""
+        ids = np.asarray(ids, np.int64).reshape(-1)
+        cols = [None if c is None else np.broadcast_to(np.asarray(c), ids.shape) for c in columns]
+        bad = (ids < 0) | (ids >= n_records)
+        if bad.any():
+            raise ValueError("%s id %d out of range [0, %d)" % (what, int(ids[np.argmax(bad)]), n_records))
+        uniq, first_of_reversed = np.unique(ids[::-1], return_index=True)
+        pick = len(ids) - 1 - first_of_reversed
+        return uniq, [None if c is None else c[pick] for c in cols]
+
+    def update_variables(self, var_ids, isEvidence=None, initialValue=None, value=None, var_copy=0):
+        """Edit ``isEvidence`` / ``initialValue`` of the listed variables in place, without a
+        rebuild; ``value`` also sets both chains (``var_value[var_copy]`` and
+        ``var_value_evid[var_copy]``) of those variables.  A duplicated id takes its last entry.
+        ``self.variable`` is edited too, so a later :meth:`invalidate` rebuilds the same graph.
+        Everything is validated before anything is written (ValueError)."""
+        V = self.variable.shape[0]
+        ids, (ev, ini, val) = self._last_wins(var_ids, V, "variable", isEvidence, initialValue, value)
+        if len(ids) == 0 or (ev is None and ini is None and val is None):
+            return
+        ev = None if ev is None else ev.astype(np.int8)
+        ini = None if ini is None else ini.astype(np.int64)
+        val = None if val is None else val.astype(np.int64)
+        # the checks of the build (and of nb_update_variables), against the records
+        rec = self.variable[ids]
+        card = rec["cardinality"].astype(np.int64)
+        if ev is not None and (ev == 4).any():
+            raise ValueError("isEvidence 4 marks a ghost, which only the partitioner creates (variable %d)"
+                             % int(ids[np.argmax(ev == 4)]))
+        ghost = rec["isEvidence"] == 4
+        if ghost.any():
+            raise ValueError("variable %d is a ghost (isEvidence 4): the partitioner owns it" % int(ids[np.argmax(ghost)]))
+        e = rec["isEvidence"].astype(np.int64) if ev is None else ev.astype(np.int64)
+        x = rec["initialValue"].astype(np.int64) if ini is None else ini
+        bad = (e == 1) & ((x < 0) | (x >= card))
+        if bad.any():
+            raise ValueError("invalid factor graph: evidence variable with initialValue outside [0, cardinality) "
+                             "(index %d)" % int(ids[np.argmax(bad)]))
+        if val is not None:
+            bad = (val < 0) | (val >= card)
+            if bad.any():
+                raise ValueError("value of variable %d lies outside [0, cardinality)" % int(ids[np.argmax(bad)]))
+
+        names = ("var_value", "var_value_evid")
+        if self._g is not None:
+            L = _lib.lib()
+            # the device chains take the value only if they hold row var_copy (else the host row is edited
+            # and uploaded by the next call)
+            dev_val = val is not None and all(self._dev_row[n] == var_copy for n in names)
+            _lib.check(L.nb_update_variables(self._g, _lib.ptr(ids), len(ids), _lib.ptr(ev), _lib.ptr(ini),
+                                             _lib.ptr(val) if dev_val else None))
+            if val is not None:
+                for n in names:
+                    if dev_val:
+                        # exposed mirrors are uploaded on entry to the next call: they must agree; a stale
+                        # mirror is refreshed from the device when it is read
+                        if n not in self._stale:
+                            getattr(self, "_" + n)[var_copy][ids] = val
+                    else:
+                        if n in self._stale and self._dev_row[n] == var_copy:
+                            self._fetch(n)
+                        getattr(self, "_" + n)[var_copy][ids] = val
+                        if self._dev_row[n] == var_copy:
+                            self._dev_row[n] = None
+        elif val is not None or ini is not None:
+            # no device graph yet: the chains it will start from are the host rows, not initialValue
+            for n in names:
+                if val is not None:
+                    getattr(self, "_" + n)[var_copy][ids] = val
+            self._pristine = False
+        if ev is not None:
+            self.variable["isEvidence"][ids] = ev
+        if ini is not None:
+            self.variable["initialValue"][ids] = ini
+
+    def update_weights(self, weight_ids, isFixed):
+        """Edit ``weight.isFixed`` of the listed weights in place, without a rebuild (a duplicated id
+        takes its last entry); ``self.weight`` is edited too."""
+        ids, (fx,) = self._last_wins(weight_ids, self.weight.shape[0], "weight", isFixed)
+        if len(ids) == 0:
+            return
+        fx = (np.asarray(fx) != 0).astype(np.uint8)
+        if self._g is not None:
+            _lib.check(_lib.lib().nb_update_weights_fixed(self._g, _lib.ptr(ids), len(ids), _lib.ptr(fx)))
+        self.weight["isFixed"][ids] = fx
+
+    def device_digest(self):
+        """{array name: 64-bit digest} of the device arrays a build derives from the records
+        (nb_graph_digest): equal digests = the same device graph."""
+        out = np.zeros(len(_lib.DIGEST_ARRAYS), np.uint64)
+        _lib.check(_lib.lib().nb_graph_digest(self._device_graph(), _lib.ptr(out), len(out)))
+        return {n: int(d) for n, d in zip(_lib.DIGEST_ARRAYS, out)}
 
     def __del__(self):
         try:
