@@ -149,17 +149,14 @@ static int host_chunks(nb_graph *g, int64_t n, F fn)   // fn(chunk index, begin,
 }
 
 // Widening loops.  The int64 / float64 result arrays are written once and not read back here, so
-// on x86 they go out as 32-byte non-temporal stores (no read-for-ownership of 3 x 134 MB on the C2
-// graph); NUMBSKULL_B200_NT_STORES=0 selects the plain loops.
+// on x86 hosts with AVX2 they go out as 32-byte non-temporal stores (no read-for-ownership of
+// 3 x 134 MB on the C2 graph); other hosts use the plain loops.
 #if defined(__x86_64__)
 #include <immintrin.h>
 #define NB_HAVE_AVX2_PATH 1
 static bool nb_use_nt()
 {
-    static const bool on = [] {
-        const char *e = getenv("NUMBSKULL_B200_NT_STORES");
-        return (!e || atoi(e) != 0) && __builtin_cpu_supports("avx2");
-    }();
+    static const bool on = __builtin_cpu_supports("avx2");
     return on;
 }
 __attribute__((target("avx2"))) static void widen_u8_nt(const uint8_t *s, int64_t *d, int64_t a, int64_t b)
@@ -865,6 +862,5 @@ extern "C" int nb_set_stream(nb_graph *g, void *cuda_stream)
     if (g->own_stream && g->stream) cudaStreamDestroy(g->stream);
     g->stream = (cudaStream_t)cuda_stream;
     g->own_stream = false;
-    if (g->finalized) nb_set_l2_policy(g, g->stream);
     return NB_OK;
 }

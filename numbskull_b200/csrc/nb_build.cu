@@ -571,7 +571,7 @@ __global__ void k_tt2_row_word(RawGraph G, const int32_t *old2new, int64_t n_pro
 
 // slice width in quads and the slice's common word (NB_PAIR_NONE = two 8-byte records per quad)
 __global__ void k_tt2_slice_width(int64_t n_slices, const int32_t *new2old, const uint32_t *ninc, const uint32_t *row_word,
-                                  int uniform_ok, int64_t *quads, uint32_t *common_out)
+                                  int64_t *quads, uint32_t *common_out)
 {
     int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (s >= n_slices) return;
@@ -585,7 +585,7 @@ __global__ void k_tt2_slice_width(int64_t n_slices, const int32_t *new2old, cons
         if (common == NB_PAIR_ANY) common = rw;
         else if (common != rw) common = NB_PAIR_NONE;
     }
-    if (common == NB_PAIR_ANY || !uniform_ok) common = NB_PAIR_NONE;
+    if (common == NB_PAIR_ANY) common = NB_PAIR_NONE;
     common_out[s] = common;
     quads[s] = (common != NB_PAIR_NONE ? (int64_t)((w + 3) / 4) : (int64_t)((w + 1) / 2)) * 32;
 }
@@ -1169,7 +1169,7 @@ int nb_build_finalize(nb_graph *g)
     NB_TRY(nb_alloc(g, &d_rowlen_new, (size_t)Vn));
     NB_TRY(nb_dev_alloc(g, &g->d_vinit, (size_t)Vn * g->value_bytes, true));
     NB_TRY(nb_alloc(g, &g->d_rng_id, (size_t)Vn));
-    // both chains in one allocation: one L2 access-policy window covers them (nb_set_l2_policy)
+    // both chains in one allocation, val_stride elements apart (d_val[1] is not an allocation of its own)
     g->val_stride = ((size_t)Vn + 255) & ~(size_t)255;
     NB_TRY(nb_dev_alloc(g, &g->d_val[0], 2 * g->val_stride * g->value_bytes, true));
     g->d_val[1] = (char *)g->d_val[0] + g->val_stride * g->value_bytes;
@@ -1323,8 +1323,6 @@ int nb_build_finalize(nb_graph *g)
         const int64_t nps = g->n_prows / 32;
         int64_t *d_q;
         uint32_t *d_row_word;
-        const char *env = getenv("NUMBSKULL_B200_UNIFORM_SLICES");
-        const int uniform_ok = (env && atoi(env) == 0) ? 0 : 1;
         NB_TRY(nb_alloc(g, &d_q, (size_t)nps + 1));
         NB_TRY(nb_alloc(g, &g->d_tt2_ptr, (size_t)nps + 1));
         NB_TRY(nb_alloc(g, &g->d_tt2_common, (size_t)nps + 1, false));
@@ -1336,8 +1334,7 @@ int nb_build_finalize(nb_graph *g)
             else
                 k_tt2_row_word<false><<<grid_for(V), 256, 0, g->stream>>>(G, g->d_old2new, g->n_prows, g->d_slice_ptr, g->d_twords,
                                                                           g->d_wfixed, d_row_word);
-            k_tt2_slice_width<<<grid_for(nps), 256, 0, g->stream>>>(nps, g->d_new2old, d_ninc, d_row_word, uniform_ok, d_q,
-                                                                    g->d_tt2_common);
+            k_tt2_slice_width<<<grid_for(nps), 256, 0, g->stream>>>(nps, g->d_new2old, d_ninc, d_row_word, d_q, g->d_tt2_common);
         }
         NB_TRY(exclusive_scan(g, d_q, g->d_tt2_ptr, nps + 1));
         NB_CUDA(cudaMemcpyAsync(&g->n_tt2_quads, g->d_tt2_ptr + nps, 8, cudaMemcpyDeviceToHost, g->stream));
@@ -1378,36 +1375,7 @@ int nb_build_finalize(nb_graph *g)
     if (g->bits_eligible) NB_TRY(nb_alloc(g, &g->d_valbits, (size_t)((g->n_trows + g->n_wrows + 31) / 32 + 1)));
     nb_release_color_scratch(g);
     g->finalized = true;
-    nb_set_l2_policy(g, g->stream);
     return NB_OK;
-}
-
-// The gathered value arrays are the only data with re-use.  Loading everything else evict-first
-// (nb_lds) is what keeps them in L2; additionally pinning them in the PERSISTING part of L2 through
-// an access-policy window was measured and is off by default: on B200 it made the sweeps slower
-// (KBC 50 M: 2.51 -> 2.86 ms, KBC 200 M: 8.97 -> 9.58 ms, Ising: 0.162 -> 0.184 ms;
-// profiles/r2c_*), presumably because the carve-out shrinks the cache left for the streams' own
-// short-lived lines.  NUMBSKULL_B200_L2_PERSIST=1 enables it.
-void nb_set_l2_policy(nb_graph *g, cudaStream_t stream)
-{
-    const char *env = getenv("NUMBSKULL_B200_L2_PERSIST");
-    if (!env || atoi(env) == 0 || !g->d_val[0] || !stream) return;
-    int max_persist = 0, max_window = 0;
-    if (cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, g->device) != cudaSuccess ||
-        cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, g->device) != cudaSuccess ||
-        max_persist <= 0 || max_window <= 0) { cudaGetLastError(); return; }
-    cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)max_persist);
-    cudaStreamAttrValue attr;
-    memset(&attr, 0, sizeof(attr));
-    const size_t bytes = std::min<size_t>(2 * g->val_stride * g->value_bytes, (size_t)max_window);
-    attr.accessPolicyWindow.base_ptr = g->d_val[0];
-    attr.accessPolicyWindow.num_bytes = bytes;
-    attr.accessPolicyWindow.hitRatio = (float)std::min(1.0, 0.9 * (double)max_persist / (double)std::max<size_t>(bytes, 1));
-    attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-    cudaStreamSetAttribute(stream, cudaStreamAttributeAccessPolicyWindow, &attr);
-    cudaGetLastError();
-    g->l2_persist_bytes = (int64_t)std::min<size_t>(bytes, (size_t)max_persist);
 }
 
 extern "C" int nb_graph_check_coloring(nb_graph *g, int64_t *conflicts)

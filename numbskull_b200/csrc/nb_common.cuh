@@ -320,7 +320,6 @@ struct nb_graph {
     void *d_val[2] = {nullptr, nullptr};  // [Vn] chain 0 = free, 1 = evidence (one allocation, val_stride elements apart)
     size_t val_stride = 0;
     int value_bytes = 1;             // element width of d_val / d_vinit: 1 (nb_val_t) or 2 (nb_val16_t)
-    int64_t l2_persist_bytes = 0;    // bytes of the value arrays pinned in the persisting part of L2
     int32_t *d_count = nullptr;      // [count_entries] new-order layout
     double *d_weight = nullptr;      // [W]
     uint8_t *d_wfixed = nullptr;     // [W]
@@ -379,7 +378,6 @@ int nb_build_color_restart(nb_graph *g, int mode);
 int nb_natural_round_cap(void);
 void nb_release_color_scratch(nb_graph *g);
 int nb_build_finalize(nb_graph *g);
-void nb_set_l2_policy(nb_graph *g, cudaStream_t stream);
 int nb_refresh_inlined_weights(nb_graph *g);   // d_tt quads carry fp32 weight values: re-inline after a weight change
 int nb_build_color_min_ids(nb_graph *g, int n_colors, int64_t *min_ids);
 int nb_build_relabel_colors(nb_graph *g, const int32_t *map, int n);

@@ -2,7 +2,6 @@
 // binary parsers and the (bit-exact) variable-to-factor index builder.
 #include <algorithm>
 #include <atomic>
-#include <chrono>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -115,14 +114,6 @@ static bool var_map_partitioned(const nb_variable_rec *variable, int64_t n_varia
                                 int64_t *factor_index, int64_t n_factor_index, int *bad_out, char *msg, size_t msg_len)
 {
     if (n_fmap < (1 << 20) || n_factor >= (1ll << 32) || n_variable < 64 || n_factor_index < n_fmap) return false;
-    const bool timing = getenv("NUMBSKULL_B200_HOST_TIMING") != nullptr;
-    auto t_last = std::chrono::steady_clock::now();
-    auto lap = [&](const char *what) {
-        if (!timing) return;
-        auto now = std::chrono::steady_clock::now();
-        fprintf(stderr, "  partitioned %-8s %.3f s\n", what, std::chrono::duration<double>(now - t_last).count());
-        t_last = now;
-    };
     const char *nt_env = getenv("NUMBSKULL_B200_HOST_THREADS");
     const int nt = nt_env ? std::max(1, std::min(64, atoi(nt_env)))
                           : (int)std::min<int64_t>(32, std::max(1u, std::thread::hardware_concurrency()));
@@ -163,7 +154,6 @@ static bool var_map_partitioned(const nb_variable_rec *variable, int64_t n_varia
     });
     if (!canonical.load()) return false;
     if (bad.load()) { *bad_out = 1; return true; }
-    lap("hist");
     // ranges of whole bins with ~n_fmap / nt entries each
     std::vector<int64_t> total((size_t)nbins, 0);
     for (int t = 0; t < nt; t++)
@@ -228,21 +218,18 @@ static bool var_map_partitioned(const nb_variable_rec *variable, int64_t n_varia
         if (bad.load()) { *bad_out = 1; return true; }
         return false;   // (nothing was written to vmap / factor_index yet)
     }
-    lap("stage");
     // bucket lengths, per range
     run_threads(nt, [&](int r) {
         const int64_t base = bucket_base[(size_t)r];
         for (int64_t i = range_beg[(size_t)r]; i < range_beg[(size_t)r + 1]; i++)
             vmap[base + staged[i].bucket_rel].factor_index_length += 1;
     });
-    lap("count");
     int64_t last_len = 0, last_off = 0;
     for (int64_t i = 0; i < n_vmap; i++) {
         vmap[i].factor_index_offset = last_off + last_len;
         last_len = vmap[i].factor_index_length;
         last_off = vmap[i].factor_index_offset;
     }
-    lap("scan");
     // fill (ascending factor ids per bucket) and drop duplicates in place, like dataloading.py:67-81
     run_threads(nt, [&](int r) {
         const int64_t base = bucket_base[(size_t)r], nb = bucket_base[(size_t)r + 1] - base;
@@ -263,7 +250,6 @@ static bool var_map_partitioned(const nb_variable_rec *variable, int64_t n_varia
             vmap[b].factor_index_length = n;
         }
     });
-    lap("fill");
     free(staged);
     return true;
 }
@@ -275,14 +261,6 @@ extern "C" int nb_compute_var_map(nb_variable_rec *variable, int64_t n_variable,
                                   const uint8_t *domain_mask, const int64_t *factors_to_skip,
                                   int64_t n_skip)
 {
-    const bool timing = getenv("NUMBSKULL_B200_HOST_TIMING") != nullptr;
-    auto t_last = std::chrono::steady_clock::now();
-    auto lap = [&](const char *what) {
-        if (!timing) return;
-        auto now = std::chrono::steady_clock::now();
-        fprintf(stderr, "compute_var_map %-10s %.3f s\n", what, std::chrono::duration<double>(now - t_last).count());
-        t_last = now;
-    };
     std::atomic<int> bad(0);
     char msg[200] = "";
     auto fail = [&](const char *what, int64_t idx) {
@@ -301,7 +279,6 @@ extern "C" int nb_compute_var_map(nb_variable_rec *variable, int64_t n_variable,
         if (domain_mask && domain_mask[i]) continue;
         for (int64_t k = 0; k < v.cardinality; k++) vmap[v.vtf_offset + k].value = k;
     }
-    lap("domains");
     // skip list -> flag per factor
     std::vector<uint8_t> skip;
     if (n_skip > 0) {
@@ -325,7 +302,6 @@ extern "C" int nb_compute_var_map(nb_variable_rec *variable, int64_t n_variable,
         if (var_map_partitioned(variable, n_variable, factor, n_factor, fmap, n_fmap, vmap, n_vmap, factor_index,
                                 n_factor_index, &bad_graph, msg, sizeof(msg))) {
             if (bad_graph) NB_FAIL(NB_ERR_INVALID, "invalid factor graph: %s", msg);
-            lap("partitioned");
             return NB_OK;
         }
     }
@@ -342,7 +318,6 @@ extern "C" int nb_compute_var_map(nb_variable_rec *variable, int64_t n_variable,
         }
     });
     if (bad.load()) NB_FAIL(NB_ERR_INVALID, "invalid factor graph: %s", msg);
-    lap("count");
     if (n_skip > 0)
         for (int64_t s = 0; s < n_skip; s++) {
             const nb_factor_rec &f = factor[factors_to_skip[s]];
@@ -361,7 +336,6 @@ extern "C" int nb_compute_var_map(nb_variable_rec *variable, int64_t n_variable,
                 "factor_index holds %lld entries but the buckets need %lld (the reference overruns "
                 "here when factors_to_skip is non-empty)",
                 (long long)n_factor_index, (long long)(last_off + last_len));
-    lap("scan");
     // :48-65 scatter (bucket cursors advanced atomically; order inside a bucket is fixed by the sort below)
     std::vector<int64_t> cursor((size_t)n_vmap);
     for (int64_t i = 0; i < n_vmap; i++) cursor[(size_t)i] = vmap[i].factor_index_offset;
@@ -373,7 +347,6 @@ extern "C" int nb_compute_var_map(nb_variable_rec *variable, int64_t n_variable,
                 factor_index[atomic_fetch_add_i64(&cursor[(size_t)bucket_of(variable, fmap[j])], 1)] = i;
         }
     });
-    lap("scatter");
     // :67-81 sort + unique each bucket; offsets are not compacted
     host_threads(n_vmap, [&](int64_t a, int64_t b) {
         for (int64_t i = a; i < b; i++) {
@@ -389,7 +362,6 @@ extern "C" int nb_compute_var_map(nb_variable_rec *variable, int64_t n_variable,
             vmap[i].factor_index_length = n;
         }
     });
-    lap("sort");
     return NB_OK;
 }
 

@@ -69,21 +69,8 @@ struct LearnArgs : NbCardOf<T> {   // (cardinalities: a.card(meta, nid))
     // reduction by weight id: three rotating global tables [3][W] (cell c uses c % 3)
     nb_fix_t *g_grad;
     uint32_t *g_cnt;
-    // NUMBSKULL_B200_LEARN_TRACE=1: per-phase nanoseconds summed over CTAs and cells
-    // [0] range lookup + zeroing  [1] truth-table rows  [2] thread rows  [3] warp rows  [4] flush
-    // [5] grid barrier  [6] apply  [7] cells processed  [8] sum over cells of the slowest CTA's work time
     unsigned *bar;            // grid barrier state {arrivals, generation}
-    unsigned long long *trace;
-    unsigned long long *trace_cell;   // [n cells] scratch: max work time of the cell over the CTAs
-    unsigned long long *trace_cta;    // [grid][3] per-CTA sums: truth-table rows, thread rows, whole work phase
 };
-
-__device__ __forceinline__ unsigned long long nb_now()
-{
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
 
 // Where the cells' rows are: block b of n_blocks covers the units [T b / nb, T (b + 1) / nb) of
 // T = n_win * k_sub units; unit u is sub-range (u % k_sub) of k_sub of id window u / k_sub.  Inside a
@@ -720,8 +707,6 @@ __global__ void __launch_bounds__(NB_LEARN_THREADS) k_learn_cells(LearnArgs<nb_v
         // caller drives the colours itself (partitioned graphs) and `cell` is the block
         const int block = only_color >= 0 ? cell : cell / plan.n_colors;
         const int color = only_color >= 0 ? only_color : cell % plan.n_colors;
-        const bool tr = a.trace != nullptr && threadIdx.x == 0;
-        unsigned long long t0 = tr ? nb_now() : 0ull, t1;
         // The cell's id ranges (64-bit divisions and dependent loads) come from shared memory: five
         // threads of the LAST warp looked them up while the previous cell was being processed.
         __syncthreads();
@@ -765,10 +750,6 @@ __global__ void __launch_bounds__(NB_LEARN_THREADS) k_learn_cells(LearnArgs<nb_v
                 z_cn[w] = 0u;
             }
         }
-        const unsigned long long t_begin = t0;
-#define NB_TRACE(i) if (a.trace != nullptr) { __syncthreads(); if (tr) { t1 = nb_now(); atomicAdd(a.trace + (i), t1 - t0); \
-            if ((i) == 1 || (i) == 2) a.trace_cta[3 * blockIdx.x + (i) - 1] += t1 - t0; t0 = t1; } }
-        NB_TRACE(0)
         if (pe > pb || fe > fb) {
             // One warp per row when the rows are long -- or when the cell holds fewer truth-table rows
             // than the grid has warps, whatever their length: a thread walking a 100-incidence row on
@@ -782,12 +763,9 @@ __global__ void __launch_bounds__(NB_LEARN_THREADS) k_learn_cells(LearnArgs<nb_v
             if (by_row) learn_tt_rows<SMEM>(a, ctx, pb, pe, fb, fe, kf, ke, kt, rot);
             else learn_tt_slices<SMEM>(a, ctx, pb, pe, fb, fe, kf, ke, kt, rot);
         }
-        NB_TRACE(1)
         if (ce > cb) learn_cat_rows<SMEM>(a, ctx, cb, ce, kf, ke);
         if (te > tb) learn_thread_rows<WIDE, SMEM>(a, ctx, 0, 0, tb, te);
-        NB_TRACE(2)
         if (we > wb) learn_warp_rows<WIDE, SMEM>(a, ctx, s_e[threadIdx.x >> 5], wb, we);
-        NB_TRACE(3)
 
         if (SMEM) {
             // flush this CTA's tables: one integer atomic per touched weight
@@ -800,10 +778,7 @@ __global__ void __launch_bounds__(NB_LEARN_THREADS) k_learn_cells(LearnArgs<nb_v
                 s_gf[w] = 0; s_gi[w] = 0; s_cnt[w] = 0u;
             }
         }
-        NB_TRACE(4)
-        if (tr) { atomicMax(a.trace_cell + (cell - cell_beg), t0 - t_begin); a.trace_cta[3 * blockIdx.x + 2] += t0 - t_begin; }
         nb_grid_sync(a.bar);     // (fences the CTAs' writes: values, tables)
-        NB_TRACE(5)
         if (SMEM) {
             // every CTA applies the same sums to its own copy of the weights; CTA 0 publishes them
             for (int w = threadIdx.x; w < W; w += blockDim.x) {
@@ -827,9 +802,6 @@ __global__ void __launch_bounds__(NB_LEARN_THREADS) k_learn_cells(LearnArgs<nb_v
             }
             nb_grid_sync(a.bar);
         }
-        NB_TRACE(6)
-        if (tr && blockIdx.x == 0) { atomicAdd(a.trace + 7, 1ull); atomicAdd(a.trace + 8, a.trace_cell[cell - cell_beg]); }
-#undef NB_TRACE
         k++;
     }
 }
@@ -1130,54 +1102,11 @@ static int launch_cells_t(nb_graph *g, LearnArgs<nb_val_t> a, CellPlan plan, int
     if (per_sm < 1) NB_FAIL(NB_ERR_CUDA, "the learning kernel does not fit on an SM");
     // all CTAs must be co-resident (grid barrier); two per SM hide each other's latencies
     const int grid = sms * std::min(per_sm, 2);
-    static const bool trace_on = [] { const char *e = getenv("NUMBSKULL_B200_LEARN_TRACE"); return e && atoi(e) != 0; }();
-    unsigned long long *d_trace = nullptr;
-    if (trace_on) {
-        const size_t n = 64 + 3 * 4096 + (size_t)(cell_end - cell_beg);
-        NB_CUDA(cudaMalloc(&d_trace, n * 8));
-        NB_CUDA(cudaMemsetAsync(d_trace, 0, n * 8, g->stream));
-        a.trace = d_trace;
-        a.trace_cta = d_trace + 64;
-        a.trace_cell = d_trace + 64 + 3 * 4096;
-    }
     NB_CUDA(cudaMemsetAsync(a.g_grad, 0, (size_t)g->W * sizeof(nb_fix_t), g->stream));   // rotating table 0
     NB_CUDA(cudaMemsetAsync(a.g_cnt, 0, (size_t)g->W * sizeof(uint32_t), g->stream));
     void *args[] = {&a, &plan, &cell_beg, &cell_end, &only_color};
     NB_CUDA(cudaLaunchCooperativeKernel((void *)kern, dim3((unsigned)grid), dim3(NB_LEARN_THREADS), args, smem, g->stream));
     g->launches++;
-    if (d_trace) {
-        std::vector<unsigned long long> hv(64 + 3 * 4096 + (size_t)std::min(cell_end - cell_beg, 4096));
-        if (false) {}
-        unsigned long long *h = hv.data();
-        NB_CUDA(cudaMemcpyAsync(h, d_trace, hv.size() * 8, cudaMemcpyDeviceToHost, g->stream));
-        NB_CUDA(cudaStreamSynchronize(g->stream));
-        cudaFree(d_trace);
-        {
-            std::vector<std::pair<unsigned long long, int>> tot;
-            for (int b = 0; b < grid && b < 4096; b++) tot.push_back({h[64 + 3 * b + 2], b});
-            std::sort(tot.begin(), tot.end());
-            fprintf(stderr, "[learn trace] per-CTA work (ms): min %.3f (cta %d) median %.3f max %.3f (cta %d); slowest CTAs:",
-                    1e-6 * tot.front().first, tot.front().second, 1e-6 * tot[tot.size() / 2].first, 1e-6 * tot.back().first,
-                    tot.back().second);
-            for (size_t i = tot.size() > 6 ? tot.size() - 6 : 0; i < tot.size(); i++)
-                fprintf(stderr, " %d: tt %.3f thr %.3f all %.3f;", tot[i].second, 1e-6 * h[64 + 3 * tot[i].second],
-                        1e-6 * h[64 + 3 * tot[i].second + 1], 1e-6 * tot[i].first);
-            fprintf(stderr, "\n");
-            {
-                const int nc = std::min(cell_end - cell_beg, 4096), ncol = std::max(plan.n_colors, 1);
-                std::vector<double> sum((size_t)ncol, 0.0), cnt((size_t)ncol, 0.0);
-                for (int c = 0; c < nc; c++) { sum[(size_t)(c % ncol)] += 1e-3 * h[64 + 3 * 4096 + c]; cnt[(size_t)(c % ncol)] += 1; }
-                fprintf(stderr, "[learn trace] slowest CTA's work per cell by colour (us):");
-                for (int c = 0; c < ncol && c < 12; c++) fprintf(stderr, " %.1f", sum[(size_t)c] / std::max(cnt[(size_t)c], 1.0));
-                fprintf(stderr, "\n");
-            }
-        }
-        const double cells = (double)std::max<unsigned long long>(h[7], 1), per = 1e-3 / (cells * grid);
-        fprintf(stderr, "[learn trace] %d CTAs, %.0f cells; us per cell and CTA: lookup %.2f, tt rows %.2f, thread rows %.2f, "
-                        "warp rows %.2f, flush %.2f, barrier wait %.2f, apply %.2f; slowest CTA's work per cell %.2f us\n",
-                grid, cells, h[0] * per, h[1] * per, h[2] * per, h[3] * per, h[4] * per, h[5] * per, h[6] * per,
-                1e-3 * (double)h[8] / cells);
-    }
     return NB_OK;
 }
 

@@ -255,7 +255,6 @@ static int sweeps_split(nb_graph *g, NbP2P *p, int64_t n_epochs, int burnin, int
         int lo = 0, hi = 0;
         NB_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
         NB_CUDA(cudaStreamCreateWithPriority(&p->side, cudaStreamNonBlocking, hi));
-        nb_set_l2_policy(g, p->side);
         NB_CUDA(cudaEventCreateWithFlags(&p->ev_main, cudaEventDisableTiming));
         NB_CUDA(cudaEventCreateWithFlags(&p->ev_side, cudaEventDisableTiming));
     }
