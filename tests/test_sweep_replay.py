@@ -14,6 +14,9 @@ included), so these tests can say "this variable, in this sweep, must take this 
   * learning, one (block, colour) cell at a time (``nb_learn_color_phase``, both execution
     modes): both chains, the truncation draws, the fixed-point gradient sums, the visit counts and
     the closed-form weight update.
+  * large learning cells: whole colours sized from the SM count, so that the branches only large
+    cells take (SELL slices, several rows per warp or thread, long rows) are replayed too;
+    ``learn_branches`` asserts which branch each cell takes.
 
 Tolerance, the same everywhere: the GPU may pick differently from the float64 replay only where
 the replay's decision margin (distance of the uniform to the nearest point that changes the pick)
@@ -23,6 +26,7 @@ counted, printed, and must stay below 1e-4 of the draws.
 The Philox known answers and the comparison with the library's own host-callable Philox
 functions (compiled from its header by nvcc into a temporary directory) run without a GPU.
 """
+import math
 import os
 import shutil
 import subprocess
@@ -291,7 +295,48 @@ def _spec(name):
     if name == "big_table":
         return _graph(13, dt0_cards=(2, 3), cat_frac=0.2, n_weights=5000, nfac=9000, hubs=4,
                       funcs0=(0, 1, 2, 3, 4, 7, 9)), {"warp_row_words": 40}, ("GEN",)
+    # Large cells, sized from the SM count S to about twice the threshold of the branch they are for
+    # (learn_branches; the grids' two colours hold n^2 / 2 rows each)
+    S = _sms()
+    if name in ("pair_slices", "pair_slices_windows"):      # > 128 S rows: slices in both modes, one tied weight
+        return _grid(math.isqrt(512 * S - 1) + 1), ({"sigma_shift": 12} if name.endswith("windows") else {}), ("PAIR",)
+    if name == "pair_slices_untied":                         # W > 2048 (global tables): > 512 S rows
+        return _grid(math.isqrt(2048 * S - 1) + 1, n_weights=5000, fixed_frac=0.1), {}, ("PAIR",)
+    if name == "pair_blocks":                                # 3 blocks of cells of > 128 S rows
+        return _grid(math.isqrt(1536 * S - 1) + 1), {}, ("PAIR",)
+    if name == "fast_slices":                                # largest colour ~ 1/3 of the rows: > 32 S FAST rows
+        return (synth.kbc(200 * S, np.random.default_rng(3), n_weights=1000, window=64, hub_frac=0.0, fixed_frac=0.2),
+                {}, ("FAST",))
+    if name == "lf_many":                                    # one colour of ~ 4100 S LF rows (GEN), one of 41 S labels
+        return synth.lf_model(41 * S, 100, np.random.default_rng(14)), {}, ("PAIR", "GEN")
+    if name == "lf_long":                                    # label rows of 301 incidences, kept off the warp path
+        return synth.lf_model(64, 300, np.random.default_rng(15)), {"warp_row_words": 4096}, ("PAIR", "GEN")
+    if name == "cat_many":                                   # largest colour ~ 55 % of the rows: > 512 S CAT rows
+        return (synth.categorical(1900 * S, 16, 1, np.random.default_rng(16), n_weights=512, window=64), {},
+                ("CAT",))
     raise KeyError(name)
+
+
+def _sms():
+    import torch
+    return torch.cuda.get_device_properties(0).multi_processor_count
+
+
+def _grid(n, n_weights=1, fixed_frac=0.0):
+    """n x n Ising grid (EQUAL to the up and left neighbours), 20 % evidence, random initial values;
+    n_weights > 1 spreads the factors over a table of that many weights, fixed_frac of them fixed."""
+    from numbskull_b200 import synth
+    from numbskull_b200.numbskulltypes import Weight
+    g = list(synth.ising_grid(n, n, coupling=0.37, fixed=False))
+    rng = np.random.default_rng(n)
+    g[1]["isEvidence"] = rng.random(len(g[1])) < 0.2
+    g[1]["initialValue"] = rng.integers(0, 2, len(g[1]))
+    if n_weights > 1:
+        g[0] = np.zeros(n_weights, Weight)
+        g[0]["isFixed"] = rng.random(n_weights) < fixed_frac
+        g[0]["initialValue"] = rng.normal(0.0, 0.5, n_weights)
+        g[2]["weightId"] = rng.integers(0, n_weights, len(g[2]))
+    return tuple(g)
 
 
 class Replay(object):
@@ -575,11 +620,13 @@ LEARN = [  # graph, regularization, learn_non_evidence
     ("gen_boolean", 2, True), ("gen_card", 1, True), ("gen_cat_empty", 2, False), ("gen_cat_empty", 1, True),
     ("cat", 1, True), ("cat", 2, False), ("warp", 2, True), ("warp", 1, True), ("warp", 0, False),
     ("big_table", 2, True), ("big_table", 1, False),
+    ("wide_headers", 2, True), ("wide_headers", 1, False), ("global_vid", 1, True), ("global_vid", 2, False),
+    ("saturating", 2, True), ("saturating", 0, True), ("pair_uniform", 1, True), ("pair_uniform", 2, False),
 ]
 
 
-def _learn(r, reg, lne, n_blocks_list, rng):
-    step, reg_param, trunc = 0.05, 0.5, 3.0
+def _learn(r, reg, lne, n_blocks_list, rng, reg_param=0.5):
+    step, trunc = 0.05, 3.0
     touched = 0
     for i, epoch in enumerate((3, (1 << 32) + 5, (1 << 40) + 1)):
         r.random_state(rng)
@@ -633,3 +680,162 @@ def test_learning_cells_at_the_default_block_count(monkeypatch):
             r.learn_cell(c, b, nb.value, step, 2, 0.5, 3.0, True, 9)
     assert seen == set(np.nonzero(r.evid != 4)[0].tolist())
     r.finish()
+
+
+# =========================================================================== GPU: large learning cells
+def learn_branches(r, color, cell, mode, sms):
+    """The code paths of nb_learn.cu that cell `cell` (ids of colour `color`) takes in latency mode
+    (1: k_learn_cells, a grid of 2 CTAs of 256 threads per SM) or throughput mode (2: the lean
+    launches of launch_cell_lean_t, at most `cap` CTAs each), by the library's own rules:
+      * truth-table rows (PAIR + FAST) go one warp per row (learn_tt_rows) when the colour is
+        flagged long-row (learn_prepare: incidences >= 16 x rows) or the cell has at most 2 rows
+        per warp of the grid, else SELL slices (learn_tt_slices);
+      * a warp takes several rows when there are more rows than warps; a row of more than
+        NB_ROW_STASH x 32 = 256 incidences re-reads its tail;
+      * GEN (learn_thread_rows) and CAT (learn_cat_rows) threads take several rows when the cell
+        has more of them than the grid has threads.
+    Slices whose learnable incidences all share one weight id reduce it warp-wide (the tied branch);
+    with several ids the lanes can add one by one."""
+    fm, fac, w = r.fg.fmap, r.fg.factor, r.fg.weight
+    ninc = np.bincount(fm["vid"], minlength=r.V)
+    live = np.nonzero((r.colors == color) & (r.evid != 4))[0]
+    tt_cls = (oracle.oracle.PAIR, oracle.oracle.FAST)
+    long_rows = np.isin(r.cls[live], tt_cls).any() and ninc[live].sum() >= 16 * len(live)
+    cls = r.cls[cell]
+    tt_ids = cell[np.isin(cls, tt_cls)]
+    tt, cat, gen = len(tt_ids), int((cls == oracle.oracle.CAT).sum()), int((cls == oracle.oracle.GEN).sum())
+    if mode == 1:
+        rows_warps, threads = 16 * sms, 512 * sms
+        slices = not long_rows and tt > 2 * rows_warps
+    else:
+        cap = sms * (8 if len(w) <= 2048 else 32)
+        slices = not long_rows and tt > 2 * cap * 8
+        rows_warps = min((tt + 7) // 8, cap) * 8
+        threads = cap * 256          # a thread takes several rows once the grid is capped
+    out = set()
+    if tt and slices:
+        out.add("tt_slices")
+        fidx = np.repeat(np.arange(len(fac)), fac["arity"])
+        inc = np.isin(fm["vid"], tt_ids)
+        wids = np.unique(fac["weightId"][fidx[inc]])
+        wids = wids[~w["isFixed"][wids].astype(bool)]
+        out.add("tt_slices_tied" if len(wids) == 1 else "tt_slices_per_lane")
+    elif tt:
+        out.add("tt_rows")
+        if tt > rows_warps:
+            out.add("tt_rows_several_per_warp")
+        if ninc[tt_ids].max() > 256:
+            out.add("tt_rows_tail")
+    if gen > threads:
+        out.add("gen_several_per_thread")
+    if cat > threads:
+        out.add("cat_several_per_thread")
+    return out
+
+
+LARGE = [  # graph, mode, regularization, learn_non_evidence, branches that must be taken
+    ("pair_slices", 1, 2, True, {"tt_slices_tied"}), ("pair_slices", 2, 1, False, {"tt_slices_tied"}),
+    ("pair_slices_untied", 1, 0, True, {"tt_slices_per_lane"}),
+    ("pair_slices_untied", 2, 2, False, {"tt_slices_per_lane"}),
+    ("fast_slices", 1, 1, True, {"tt_slices_per_lane"}), ("fast_slices", 1, 2, False, {"tt_slices_per_lane"}),
+    ("lf_many", 1, 1, False, {"gen_several_per_thread", "tt_rows_several_per_warp"}),
+    ("lf_many", 2, 2, True, {"gen_several_per_thread"}),
+    ("lf_long", 1, 2, True, {"tt_rows_tail"}), ("lf_long", 2, 1, True, {"tt_rows_tail"}),
+    ("cat_many", 1, 1, True, {"cat_several_per_thread"}), ("cat_many", 1, 0, False, {"cat_several_per_thread"}),
+]
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name,mode,reg,lne,want", LARGE, ids=["%s-m%d-r%d-%s" % c[:4] for c in LARGE])
+def test_large_learning_cells_replay_exactly(name, mode, reg, lne, want, monkeypatch):
+    """Whole colours as cells (one block), large enough for the branches that only large cells
+    take; every cell is replayed, and the branches it takes are checked, so that a smaller fixture or
+    a moved threshold cannot quietly turn this back into a small-cell test."""
+    monkeypatch.setenv("NUMBSKULL_B200_LEARN_MODE", str(mode))
+    r = Replay(name)
+    sms = _sms()
+    taken = set()
+    for c in range(r.info["n_colors"]):
+        taken |= learn_branches(r, c, r.cell_ids(c, 0, 1), mode, sms)
+    assert want <= taken, (name, mode, taken)
+    # a whole colour visits a weight 10^3 - 10^5 times: at the small cells' reg_param every L1 update
+    # would clamp the weights to 0 and every L2 shrink s^n underflow, whatever the visit counts
+    assert _learn(r, reg, lne, (1,), np.random.default_rng(len(name) * 31 + reg), reg_param=1e-5) > 0
+    r.finish()
+
+
+@pytest.mark.gpu
+def test_large_learning_cells_in_cut_id_windows(monkeypatch):
+    """Id windows of 4096 variables (the size graphs of 2^22 variables or more get) and more blocks
+    than windows, so that the plan cuts every window further (CellPlan::k_sub > 1): the cells of each
+    epoch partition the live variables, and every one of them is replayed."""
+    monkeypatch.setenv("NUMBSKULL_B200_LEARN_MODE", "1")
+    r = Replay("pair_slices_windows")
+    n_win = (r.V >> 12) + 1
+    n_blocks = 2 * n_win + 1
+    rng = np.random.default_rng(12)
+    live = set(np.nonzero(r.evid != 4)[0].tolist())
+    for epoch in (3, (1 << 32) + 5, (1 << 40) + 1):
+        r.random_state(rng)
+        seen = []
+        for b in range(n_blocks):
+            for c in range(r.info["n_colors"]):
+                seen.extend(r.cell_ids(c, b, n_blocks).tolist())
+                r.learn_cell(c, b, n_blocks, 0.05, 2, 0.5, 3.0, True, epoch)
+        assert len(seen) == len(live) and set(seen) == live
+    r.finish()
+
+
+def _visit_bound(fg, colors, lne):
+    """Sum over colours of the most visits one weight gets in a colour (color_visit_bounds)."""
+    fm, fac, w, var = fg.fmap, fg.factor, fg.weight, fg.variable
+    fidx = np.repeat(np.arange(len(fac)), fac["arity"])
+    vid, wid = fm["vid"], fac["weightId"][fidx]
+    ev = var["isEvidence"][vid]
+    keep = (ev != 4) & (colors[vid] >= 0) & ~w["isFixed"][wid].astype(bool) & (bool(lne) | (ev == 1))
+    hist = np.zeros((int(colors.max()) + 1, len(w)), np.int64)
+    np.add.at(hist, (colors[vid[keep]], wid[keep]), 1)
+    return int(hist.max(axis=1).sum())
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name", ["pair_blocks", "lf_many"])
+def test_large_learning_modes_agree_bit_for_bit(name, monkeypatch):
+    """Whole epochs (FactorGraph.learn, decaying step) of 3 blocks of large cells: the persistent
+    launch (mode 1: rotating tables, next-cell range lookup, per-CTA weight copies) and the lean
+    launches (mode 2) give identical weights and chains.  Both modes take the same truth-table
+    branch in every cell -- slices on the tied grid, rows on the long-row label colour -- since
+    the two branches sum the float64 energies in different orders."""
+    import ctypes as C
+    import numbskull_b200 as nb
+    lne, step = True, 0.01
+    r = Replay(name)
+    bv = -(-_visit_bound(r.fg, r.colors, lne) // 3)
+    n_blocks = C.c_int(0)
+    r._chk(r.L.nb_learn_blocks(r.g, step, int(lne), bv, C.byref(n_blocks)))
+    assert n_blocks.value == 3
+    sms = _sms()
+    for mode in (1, 2):
+        for b in range(3):
+            for c in range(r.info["n_colors"]):
+                br = learn_branches(r, c, r.cell_ids(c, b, 3), mode, sms)
+                if name == "pair_blocks":
+                    assert "tt_slices_tied" in br, (mode, b, c, br)
+                else:
+                    assert "tt_slices" not in br, (mode, b, c, br)
+    r.fg.clear()
+    g, attrs, _ = _spec(name)
+    runs = []
+    for mode in ("1", "2"):
+        monkeypatch.setenv("NUMBSKULL_B200_LEARN_MODE", mode)
+        ns = nb.NumbSkull(quiet=True)
+        ns.loadFactorGraph(*g)
+        fg = ns.factorGraphs[0]
+        fg.seed, fg.batch_visits = SEED, bv
+        for k, v in attrs.items():
+            setattr(fg, k, v)
+        fg.learn(0, 4, step, 0.9, 2, 0.01, 1, learn_non_evidence=lne)
+        runs.append((fg.weight_value.copy(), fg.var_value.copy(), fg.var_value_evid.copy()))
+        fg.clear()
+    for a, b in zip(runs[0], runs[1]):
+        assert np.array_equal(a, b)
