@@ -1042,7 +1042,8 @@ static int order_colors_by_min_id(nb_graph *g, int n_colors)
 
 int nb_build_device_graph(nb_graph *g, const nb_graph_desc *d)
 {
-    if (d->warp_row_words > 0) g->warp_row_words = d->warp_row_words;
+    // thread rows take their length from the 17-bit vmeta field: anything longer must be a warp row
+    if (d->warp_row_words > 0) g->warp_row_words = (int)std::min<uint32_t>((uint32_t)d->warp_row_words, NB_META_MAX_ROWLEN);
     g->deferred = d->deferred_coloring != 0;
     NB_TRY(extract_and_upload(g, d));
     if (d->sigma_shift > 0) g->sigma_shift = d->sigma_shift;

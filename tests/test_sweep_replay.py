@@ -194,25 +194,40 @@ def test_host_restatement_matches_the_library_philox(philox_shim):
 
 
 # =========================================================================== GPU: graphs
-def _graph(seed, nvar=3000, nfac=6000, cat_frac=0.0, cat_cards=(6, 12), dt0_cards=(2,), funcs0=(0, 1, 2, 3, 4, 7, 9),
-           funcs1=(12, 14, 15), max_arity=4, hubs=0, hub_degree=150, evidence_frac=0.3, ghost_frac=0.0,
-           fixed_frac=0.2, n_weights=None, w_scale=1.0, feature_values=False, wide_arity=0, ratio=False):
+def _graph(seed, nvar=3000, nfac=6000, cat_frac=0.0, cat_cards=(6, 12), cat_card_set=None, dt0_cards=(2,),
+           funcs0=(0, 1, 2, 3, 4, 7, 9), funcs1=(12, 14, 15), max_arity=4, hubs=0, hub_degree=150, hub_rows=(),
+           evidence_frac=0.3, ghost_frac=0.0, fixed_frac=0.2, n_weights=None, w_scale=1.0, feature_values=False,
+           wide_arity=0, ratio=False):
     """Random graph for the replay.  dataType-0 variables (cardinalities from dt0_cards) share
-    factors of funcs0 (plus RATIO if `ratio`); dataType-1 variables (cardinalities in cat_cards)
-    factors of funcs1 with dense_equal_to below each member's cardinality.  `hubs` variables get
-    `hub_degree` extra pairwise factors each (long rows: warp path with several tasks)."""
+    factors of funcs0 (plus RATIO if `ratio`); dataType-1 variables (cardinalities in the range
+    cat_cards, or from cat_card_set) factors of funcs1 with dense_equal_to below each member's
+    cardinality.  `hubs` variables get `hub_degree` extra pairwise factors each (long rows: warp
+    path with several tasks).  Each (dataType, cardinality, incidences) of `hub_rows` makes one more
+    hub, a free variable of that type and cardinality with exactly that many incidences; a
+    categorical one of these leaves a fifth of its values without incidences (empty buckets)."""
     from numbskull_b200.numbskulltypes import Weight, Variable, Factor, FactorToVar
     rng = np.random.default_rng(seed)
     variable = np.zeros(nvar, Variable)
     cat = rng.random(nvar) < cat_frac
     card = rng.choice(np.array(dt0_cards), nvar)
-    card[cat] = rng.integers(cat_cards[0], cat_cards[1] + 1, int(cat.sum()))
+    if cat_card_set is None:
+        card[cat] = rng.integers(cat_cards[0], cat_cards[1] + 1, int(cat.sum()))
+    else:
+        card[cat] = rng.choice(np.array(cat_card_set), int(cat.sum()))
+    hub_dtype = np.array([h[0] for h in hub_rows], bool)
+    rows = np.zeros(len(hub_rows), np.int64)                 # the hub_rows variables
+    for want in (False, True):
+        if (hub_dtype == want).any():
+            rows[hub_dtype == want] = rng.choice(np.nonzero(cat == want)[0], int((hub_dtype == want).sum()),
+                                                 replace=False)
+    card[rows] = [h[1] for h in hub_rows]
     variable["dataType"] = cat
     variable["cardinality"] = card
     ev = rng.random(nvar) < evidence_frac
     variable["isEvidence"] = ev
     variable["isEvidence"][rng.random(nvar) < ghost_frac] = 4
     variable["initialValue"] = rng.integers(0, 1 << 30, nvar) % card
+    variable["isEvidence"][rows] = 0
     ids0, ids1 = np.nonzero(~cat)[0], np.nonzero(cat)[0]
     f0 = tuple(funcs0) + ((8,) if ratio else ())
     facs, members = [], []
@@ -224,16 +239,21 @@ def _graph(seed, nvar=3000, nfac=6000, cat_frac=0.0, cat_cards=(6, 12), dt0_card
         a = 1 if func == 15 else a
         facs.append(func)
         members.append(rng.choice(pool, min(a, len(pool)), replace=False))
-    hub_ids = rng.choice(ids0 if len(ids0) else ids1, hubs, replace=False) if hubs else []
-    for h in hub_ids:
-        pool = ids0 if variable["dataType"][h] == 0 else ids1
-        for _ in range(hub_degree):
-            o = int(rng.choice(pool))
-            facs.append(int(rng.choice((3, 7, 9)) if variable["dataType"][h] == 0 else 12))
-            members.append(np.array([h, o] if o != h else [h]))
     if wide_arity:                                   # one long factor: 2-word incidence headers
         facs.append(7)
         members.append(rng.choice(ids0, wide_arity, replace=False))
+    arity = [np.array([len(m) for m in members])]
+    # hub factors, pairwise (hub, other): funcs (3, 7, 9) on dataType 0, AND_CAT on dataType 1
+    ninc = np.bincount(np.concatenate(members), minlength=nvar)
+    hub_ids = rng.choice(np.setdiff1d(ids0 if len(ids0) else ids1, rows), hubs, replace=False) if hubs else []
+    every_hub = np.concatenate((hub_ids, rows)).astype(np.int64)
+    for h, m in list(zip(hub_ids, [hub_degree] * hubs)) + [(h, r[2] - ninc[h]) for h, r in zip(rows, hub_rows)]:
+        assert m >= 0, "hub row already has more incidences than asked for"
+        pool = ids1 if cat[h] else ids0
+        other = rng.choice(pool[~np.isin(pool, every_hub)], m)
+        facs.extend(np.full(m, 12) if cat[h] else rng.choice((3, 7, 9), m))
+        members.append(np.stack([np.full(m, h), other], axis=1).ravel())
+        arity.append(np.full(m, 2))
     nf = len(facs)
     n_weights = n_weights or max(1, nf // 3)
     weight = np.zeros(n_weights, Weight)
@@ -243,12 +263,15 @@ def _graph(seed, nvar=3000, nfac=6000, cat_frac=0.0, cat_cards=(6, 12), dt0_card
     factor["factorFunction"] = facs
     factor["weightId"] = rng.integers(0, n_weights, nf)
     factor["featureValue"] = rng.choice([1.0, 0.5, 2.0], nf) if feature_values else 1.0
-    factor["arity"] = [len(m) for m in members]
+    factor["arity"] = np.concatenate(arity)
     factor["ftv_offset"] = np.concatenate(([0], np.cumsum(factor["arity"])[:-1]))
     vids = np.concatenate(members).astype(np.int64)
     fmap = np.zeros(len(vids), FactorToVar)
     fmap["vid"] = vids
     fmap["dense_equal_to"] = rng.integers(0, 1 << 30, len(vids)) % card[vids]
+    for h in rows[cat[rows]]:                        # empty buckets: a fifth of the values get no incidence
+        at = np.nonzero(vids == h)[0]
+        fmap["dense_equal_to"][at] = rng.choice(rng.permutation(card[h])[:card[h] - card[h] // 5], len(at))
     return weight, variable, factor, fmap, np.zeros(nvar, np.bool_), len(vids)
 
 
@@ -295,6 +318,24 @@ def _spec(name):
     if name == "big_table":
         return _graph(13, dt0_cards=(2, 3), cat_frac=0.2, n_weights=5000, nfac=9000, hubs=4,
                       funcs0=(0, 1, 2, 3, 4, 7, 9)), {"warp_row_words": 40}, ("GEN",)
+    if name == "hub_tasks":          # HUB_TASKS: rows of 32, 33 and more than 64 warp tasks
+        return _graph(17, dt0_cards=(2, 2, 3), cat_frac=0.3, hub_rows=[(d, c, n) for (d, c), n in HUB_TASKS]), {}, \
+            ("WARP", "GEN", "CAT")
+    if name == "hub_tasks_wide":     # a categorical hub above 255 values (2-byte graph): nb_warp_sample_wide
+        return _graph(18, dt0_cards=(2, 3), cat_frac=0.3, hub_rows=[(1, 700, 2100)]), {}, ("WIDE", "GEN")
+    if name == "hub_mirror":         # all-Boolean; hubs of ~ 0.3 x 2 x 4000 = 2400 IMPLY and as many OR incidences
+        return synth.kbc(8000, np.random.default_rng(19), n_weights=1024, window=64, hub_frac=0.3), {}, \
+            ("FAST", "WARP")
+    if name == "card_band":          # 1-byte graph, cardinalities 33 - 255, each as GEN and as WARP rows
+        return (_graph(20, nvar=4000, nfac=9000, dt0_cards=CARD_BAND[0], cat_frac=0.5, cat_card_set=CARD_BAND[1],
+                       max_arity=3), {"warp_row_words": 14}, ("GEN", "WARP"))
+    if name == "cat32":              # CAT rows at NB_CAT_MAX_CARD, and cardinality-33 rows next to them
+        g = synth.categorical(4000, 32, 3, np.random.default_rng(21), n_weights=512, window=64)
+        g[1]["cardinality"][np.random.default_rng(22).choice(len(g[1]), 40, replace=False)] = 33
+        return g, {}, ("CAT",)
+    if name == "thread_row_long":    # one Boolean hub of > NB_META_MAX_ROWLEN words, as long as thread rows may be
+        return (_graph(23, dt0_cards=(2,), feature_values=True, hub_rows=[(0, 2, 46000)]), {"warp_row_words": 1 << 20},
+                ("GEN",))
     # Large cells, sized from the SM count S to about twice the threshold of the branch they are for
     # (learn_branches; the grids' two colours hold n^2 / 2 rows each)
     S = _sms()
@@ -314,7 +355,65 @@ def _spec(name):
     if name == "cat_many":                                   # largest colour ~ 55 % of the rows: > 512 S CAT rows
         return (synth.categorical(1900 * S, 16, 1, np.random.default_rng(16), n_weights=512, window=64), {},
                 ("CAT",))
+    # rows of 3 or 4 incidences (9 or 12 words) on the warp path: a colour of ~ n^2 / 2 warp rows
+    if name == "warp_crowd":                                 # > 2 x 64 S rows (8 warps x cap = 8 S CTAs)
+        return _grid(math.isqrt(320 * S - 1) + 1), {"warp_row_words": 8}, ("WARP", "PAIR")
+    if name == "warp_crowd_untied":                          # W > 2048 (cap = 32 S CTAs): > 2 x 256 S rows
+        return (_grid(math.isqrt(1280 * S - 1) + 1, n_weights=5000, fixed_frac=0.1), {"warp_row_words": 8},
+                ("WARP", "PAIR"))
     raise KeyError(name)
+
+
+# hub rows of "hub_tasks": ((dataType, cardinality), incidences).  A warp task takes NB_WARP_TASK = 64
+# incidences and k_gibbs_warp_finish's lanes stride over a row's tasks: 32 tasks fill the lanes once, 33
+# wrap once, more than 64 wrap twice.  Cardinality 2 takes the e[4] path, 6 the shared-array atomics, the
+# categorical ones the bucket index (ent.y), with empty buckets.
+HUB_TASKS = [((0, 2), 2048), ((0, 2), 4500), ((0, 6), 2049), ((0, 6), 4161),
+             ((1, 40), 2048), ((1, 40), 4300), ((1, 200), 2049), ((1, 200), 5000)]
+# "card_band": dataType-0 and categorical cardinalities of a 1-byte graph, all above the lanes of a warp
+# but 5 (and above NB_CAT_MAX_CARD); 128 - 255 are values of uint8_t with the top bit set
+CARD_BAND = ((5, 40, 255), (33, 64, 127, 128, 200, 255))
+
+
+def _check_spec(r):
+    """The property each of the larger replay graphs exists for, from the records."""
+    name, O = r.name, oracle.oracle
+    fm = r.fg.fmap
+    ninc = np.bincount(fm["vid"], minlength=r.V)
+    live = r.evid != 4
+    warp_path = np.isin(r.cls, (O.WARP, O.WIDE)) & live
+    if name in ("hub_tasks", "hub_mirror"):
+        hub = warp_path & (ninc >= 2048)
+        tasks = {(int(r.card[v]), -(-int(ninc[v]) // 64)) for v in np.nonzero(hub)[0]}
+        if name == "hub_tasks":
+            assert tasks == {(c, -(-n // 64)) for (_, c), n in HUB_TASKS}, tasks
+            assert {32, 33} <= {t for _, t in tasks} and max(t for _, t in tasks) > 64, tasks
+        else:                            # more than 32 tasks: the task sum wraps before the mirror update
+            assert (r.card == 2).all() and tasks and max(t for _, t in tasks) > 32, tasks
+    if name == "hub_tasks_wide":
+        assert r.info["value_bytes"] == 2
+        (hub,) = np.nonzero((r.card > 255) & warp_path)[0]
+        assert r.cls[hub] == O.WIDE and ninc[hub] > 2048
+        size = np.bincount(fm["dense_equal_to"][fm["vid"] == hub], minlength=r.card[hub])
+        assert (size == 0).any(), "no empty bucket"
+        end = np.cumsum(size[size > 0])          # buckets in value order, as the row holds them
+        assert ((end - size[size > 0]) // 32 != (end - 1) // 32).any(), "no bucket straddles 32 incidences"
+    if name == "card_band":
+        assert r.info["value_bytes"] == 1
+        dtype = r.fg.variable["dataType"]
+        for d, cards in enumerate(CARD_BAND):
+            for c in cards:
+                for cl in (O.GEN, O.WARP):
+                    assert ((dtype == d) & (r.card == c) & (r.cls == cl) & live).any(), (d, c, CLASS_NAMES[cl])
+    if name == "cat32":
+        assert ((r.cls == O.CAT) & (r.card == 32) & live).any()
+        c33 = (r.card == 33) & live
+        assert c33.any() and (r.cls[c33] != O.CAT).all()
+    if name == "thread_row_long":        # at least (1 + arity) words per incidence
+        fac = r.fg.factor
+        fidx = np.repeat(np.arange(len(fac)), fac["arity"])
+        hub = int(np.argmax(ninc))
+        assert (1 + fac["arity"][fidx[fm["vid"] == hub]]).sum() > 131071 and r.evid[hub] == 0
 
 
 def _sms():
@@ -377,6 +476,7 @@ class Replay(object):
         present = {CLASS_NAMES[c] for c in np.unique(cls[live])}
         for c in self.expect:
             assert c in present, (name, c, present, self.info)
+        _check_spec(self)
 
     # ---- state through the C ABI ----
     def _chk(self, rc):
@@ -560,7 +660,8 @@ def apply_update(w, G, cnt, reg, step, reg_param, trunc):
 
 # =========================================================================== GPU: Gibbs phases
 GIBBS_GRAPHS = ["pair_uniform", "pair_records", "fast", "gen_boolean", "gen_card", "gen_cat_empty", "cat", "warp",
-                "saturating", "wide_headers", "global_vid", "wide_card", "wide_card_thread"]
+                "saturating", "wide_headers", "global_vid", "wide_card", "wide_card_thread", "hub_tasks", "hub_tasks_wide",
+                "card_band", "cat32", "thread_row_long"]
 
 
 @pytest.mark.gpu
@@ -581,6 +682,13 @@ def test_gibbs_phases_replay_exactly(name):
             for c in range(r.info["n_colors"]):
                 n += r.gibbs_phase(c, burnin, sample_evidence, epoch + 7 * c * (i % 2))
     assert n > 0
+    if name == "card_band":
+        assert (r.get_vals(0)[r.sampled(True)] >= 128).any()
+    if name == "thread_row_long":
+        # too long for the 17-bit length of thread rows.  Only this class check catches a partly walked
+        # row here: the hub's energy saturates, so its draws match either way.  The LEARN cases of
+        # thread_row_long are the ones that see the wrong gradient sums of such a walk.
+        assert r.cls[np.argmax(np.bincount(r.fg.fmap["vid"], minlength=r.V))] == oracle.oracle.WARP
     r.finish()
 
 
@@ -593,7 +701,7 @@ def _whole_sweeps(name, sample_evidence):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name,mirror", [("fast", "-1"), ("fast", "0"), ("warp", "-1"), ("gen_cat_empty", "-1"),
-                                         ("wide_card", "-1")])
+                                         ("wide_card", "-1"), ("hub_mirror", "0"), ("hub_tasks", "-1")])
 def test_whole_sweeps_replay_with_fan_out(name, mirror, monkeypatch):
     """nb_gibbs_sweeps with the row classes of a colour on concurrent streams (the default); "0"
     forces the bit-packed value mirror on (all-Boolean graphs)."""
@@ -622,6 +730,9 @@ LEARN = [  # graph, regularization, learn_non_evidence
     ("big_table", 2, True), ("big_table", 1, False),
     ("wide_headers", 2, True), ("wide_headers", 1, False), ("global_vid", 1, True), ("global_vid", 2, False),
     ("saturating", 2, True), ("saturating", 0, True), ("pair_uniform", 1, True), ("pair_uniform", 2, False),
+    ("hub_tasks", 2, True), ("hub_tasks", 1, False), ("card_band", 1, True), ("card_band", 2, False),
+    ("cat32", 2, True), ("cat32", 1, False),
+    ("thread_row_long", 2, True), ("thread_row_long", 1, True),     # the hub's own gradient: learn_non_evidence
 ]
 
 
@@ -649,11 +760,13 @@ def test_learning_cells_replay_exactly(name, reg, lne, mode, monkeypatch):
     rng = np.random.default_rng(len(name) * 31 + reg)
     touched = _learn(r, reg, lne, (1, 3), rng)
     assert touched > 0
+    if name == "card_band":
+        assert all((r.get_vals(chain)[r.evid == 0] >= 128).any() for chain in (0, 1))
     r.finish()
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", ["wide_card", "wide_card_thread"])
+@pytest.mark.parametrize("name", ["wide_card", "wide_card_thread", "hub_tasks_wide"])
 def test_learning_cells_replay_on_a_two_byte_graph(name, monkeypatch):
     monkeypatch.setenv("NUMBSKULL_B200_LEARN_MODE", "2")
     r = Replay(name)
@@ -693,7 +806,9 @@ def learn_branches(r, color, cell, mode, sms):
       * a warp takes several rows when there are more rows than warps; a row of more than
         NB_ROW_STASH x 32 = 256 incidences re-reads its tail;
       * GEN (learn_thread_rows) and CAT (learn_cat_rows) threads take several rows when the cell
-        has more of them than the grid has threads.
+        has more of them than the grid has threads;
+      * a warp of learn_warp_rows takes several WARP rows when the cell has more of them than the
+        grid has warps.
     Slices whose learnable incidences all share one weight id reduce it warp-wide (the tied branch);
     with several ids the lanes can add one by one."""
     fm, fac, w = r.fg.fmap, r.fg.factor, r.fg.weight
@@ -704,14 +819,17 @@ def learn_branches(r, color, cell, mode, sms):
     cls = r.cls[cell]
     tt_ids = cell[np.isin(cls, tt_cls)]
     tt, cat, gen = len(tt_ids), int((cls == oracle.oracle.CAT).sum()), int((cls == oracle.oracle.GEN).sum())
+    warp = int(np.isin(cls, (oracle.oracle.WARP, oracle.oracle.WIDE)).sum())
     if mode == 1:
         rows_warps, threads = 16 * sms, 512 * sms
         slices = not long_rows and tt > 2 * rows_warps
+        warps = 16 * sms
     else:
         cap = sms * (8 if len(w) <= 2048 else 32)
         slices = not long_rows and tt > 2 * cap * 8
         rows_warps = min((tt + 7) // 8, cap) * 8
         threads = cap * 256          # a thread takes several rows once the grid is capped
+        warps = cap * 8              # k_cell_warp: at most cap CTAs of 8 warps
     out = set()
     if tt and slices:
         out.add("tt_slices")
@@ -730,6 +848,8 @@ def learn_branches(r, color, cell, mode, sms):
         out.add("gen_several_per_thread")
     if cat > threads:
         out.add("cat_several_per_thread")
+    if warp > warps:
+        out.add("warp_several_per_warp")
     return out
 
 
@@ -742,6 +862,8 @@ LARGE = [  # graph, mode, regularization, learn_non_evidence, branches that must
     ("lf_many", 2, 2, True, {"gen_several_per_thread"}),
     ("lf_long", 1, 2, True, {"tt_rows_tail"}), ("lf_long", 2, 1, True, {"tt_rows_tail"}),
     ("cat_many", 1, 1, True, {"cat_several_per_thread"}), ("cat_many", 1, 0, False, {"cat_several_per_thread"}),
+    ("warp_crowd", 1, 2, True, {"warp_several_per_warp"}), ("warp_crowd", 2, 1, False, {"warp_several_per_warp"}),
+    ("warp_crowd_untied", 2, 2, True, {"warp_several_per_warp"}),
 ]
 
 
@@ -799,13 +921,14 @@ def _visit_bound(fg, colors, lne):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("name", ["pair_blocks", "lf_many"])
+@pytest.mark.parametrize("name", ["pair_blocks", "lf_many", "warp_crowd"])
 def test_large_learning_modes_agree_bit_for_bit(name, monkeypatch):
     """Whole epochs (FactorGraph.learn, decaying step) of 3 blocks of large cells: the persistent
     launch (mode 1: rotating tables, next-cell range lookup, per-CTA weight copies) and the lean
     launches (mode 2) give identical weights and chains.  Both modes take the same truth-table
-    branch in every cell -- slices on the tied grid, rows on the long-row label colour -- since
-    the two branches sum the float64 energies in different orders."""
+    branch in every cell -- slices on the tied grid, rows on the long-row label colour and on the
+    corner rows of the warp grid -- since the two branches sum the float64 energies in different
+    orders.  The warp grid's Boolean warp rows reduce with shuffles, in the same order in both modes."""
     import ctypes as C
     import numbskull_b200 as nb
     lne, step = True, 0.01
