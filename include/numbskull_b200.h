@@ -203,7 +203,12 @@ int nb_get_marginals(nb_graph *g, double *marginals, double epochs);
 int nb_get_counts_compact(nb_graph *g, void *out, int64_t out_bytes, int32_t *elem_bytes);
 /* Install `counts` (int64, cstart layout) as the device tallies: callers that edit `count` between
  * calls.  The device tallies are CUMULATIVE like the reference's count array (factorgraph.py:30-31
- * is never re-zeroed by inference()); nb_reset_counts zeroes them (FactorGraph.clear). */
+ * is never re-zeroed by inference()); nb_reset_counts zeroes them (FactorGraph.clear).
+ * Limit: the device tallies are int32.  Entries must lie in [0, 2^31 - 1] (else NB_ERR_INVALID), and
+ * a tallying sweep or colour phase that could take a tally past 2^31 - 1 (the largest installed
+ * count plus the tallying launches of a colour since the last reset or nb_set_counts) is refused
+ * with NB_ERR_UNSUPPORTED before anything is launched; burn-in sweeps stay allowed.  Read the
+ * counts and reset them to go on. */
 int nb_set_counts(nb_graph *g, const int64_t *counts);
 /* page-locked host memory for result arrays the library fills by DMA */
 int nb_host_alloc(void **ptr, int64_t bytes);

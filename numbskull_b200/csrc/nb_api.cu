@@ -379,13 +379,14 @@ extern "C" int nb_reset_counts(nb_graph *g)
     NB_CUDA(cudaSetDevice(g->device));
     NB_CUDA(cudaMemsetAsync(g->d_count, 0, (size_t)g->count_entries * 4, g->stream));
     NB_CUDA(cudaMemsetAsync(g->d_count_b, 0, (size_t)g->Vn * 4, g->stream));
-    g->tally_bound = 0;
+    g->tally_bound = g->tally_base = 0;
+    g->tally_launches.clear();
     return NB_OK;
 }
 
-// new-order tallies -> reference cstart layout, narrowed on the fly: no tally exceeds the number of
-// tallying sweeps since the last reset (g->tally_bound, tracked on the host), so a short call's tallies
-// cross PCIe as one byte each (two up to 65535 sweeps).
+// new-order tallies -> reference cstart layout, narrowed on the fly: no tally exceeds g->tally_bound
+// (tallying launches per colour since the last reset, plus the largest installed count, tracked on the
+// host), so a short call's tallies cross PCIe as one byte each (two up to 65535 sweeps).
 // (Boolean rows sampled by the truth-table kernels tally into count_b[new id].)
 template <class T>
 __global__ void k_counts_to_old(int64_t V, const int32_t *count, const int32_t *count_b, const uint32_t *cstart_new,
@@ -560,7 +561,8 @@ extern "C" int nb_set_counts(nb_graph *g, const int64_t *counts)
                                                               g->d_old2new, g->d_v_card, (const int32_t *)g->d_xfer);
     NB_CUDA(cudaGetLastError());
     NB_CUDA(cudaStreamSynchronize(g->stream));
-    g->tally_bound = mx.load();
+    g->tally_bound = g->tally_base = mx.load();
+    g->tally_launches.clear();
     return NB_OK;
 }
 
@@ -609,6 +611,7 @@ extern "C" int nb_gibbs_sweeps(nb_graph *g, int64_t n_epochs, int burnin, int sa
 {
     NB_CUDA(cudaSetDevice(g->device));
     NB_TRY(check_runnable(g));
+    NB_TRY(nb_check_tally_room(g, burnin, n_epochs));
     NB_TRY(nb_refresh_inlined_weights(g));
     static const bool fan = [] { const char *e = getenv("NUMBSKULL_B200_FAN_OUT"); return !e || atoi(e) != 0; }();
     g->fan_out = fan && g->p2p == nullptr;

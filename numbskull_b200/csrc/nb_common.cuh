@@ -229,8 +229,12 @@ struct nb_graph {
     int64_t device_bytes = 0;
     int64_t launches = 0;
     uint64_t epoch_counter = 0;
-    int64_t tally_bound = 0;          // no tally exceeds this: tallying sweeps since the last reset (or max of nb_set_counts)
-    uint64_t last_tally_epoch = ~0ull;
+    // No tally exceeds tally_bound = tally_base + max over colours of tally_launches[c]: a variable is
+    // tallied at most once per tallying launch of its colour (of its phase on partitioned graphs).
+    // tally_base is the largest count installed by nb_set_counts (0 after nb_reset_counts).
+    int64_t tally_bound = 0;
+    int64_t tally_base = 0;
+    std::vector<int64_t> tally_launches;   // [n_colors] tallying launches since the last reset / nb_set_counts
     int warp_row_words = 1024;
     int sigma_shift = 12;
 
@@ -389,6 +393,8 @@ int nb_learn_cell_id_list(nb_graph *g, int color, int block, int n_blocks, int64
 // sweeps (nb_sweep.cu / nb_learn.cu)
 int nb_launch_gibbs_color(nb_graph *g, int color, int burnin, int sample_evidence, uint64_t seed,
                           uint64_t epoch);
+// NB_ERR_UNSUPPORTED when n_sweeps more tallying sweeps could take a tally past INT32_MAX
+int nb_check_tally_room(const nb_graph *g, int burnin, int64_t n_sweeps);
 int nb_run_learn(nb_graph *g, int64_t n_epochs, double *stepsize, double decay, int regularization,
                  double reg_param, double truncation, int learn_non_evidence, uint64_t seed,
                  int64_t batch_visits);

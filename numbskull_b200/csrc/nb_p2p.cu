@@ -301,6 +301,7 @@ extern "C" int nb_gibbs_sweeps_p2p(nb_graph *g, int64_t n_epochs, int burnin, in
     if (g->has_unknown_func)
         NB_FAIL(NB_ERR_NOT_IMPLEMENTED, "Error: Factor Function %d ( used in factor %lld ) is not implemented.",
                 g->unknown_func_id, (long long)g->unknown_func_factor);
+    NB_TRY(nb_check_tally_room(g, burnin, n_epochs));
     const int nowait = mode & 3;
     NB_TRY(nb_refresh_inlined_weights(g));   // before the streams fork
     if (mode & 2) {

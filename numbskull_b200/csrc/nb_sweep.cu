@@ -492,11 +492,27 @@ static int launch_gibbs_color_t(nb_graph *g, int color, int burnin, int sample_e
     return NB_OK;
 }
 
+int nb_check_tally_room(const nb_graph *g, int burnin, int64_t n_sweeps)
+{
+    if (!burnin && n_sweeps > 0 && g->tally_bound > (int64_t)INT32_MAX - n_sweeps)
+        NB_FAIL(NB_ERR_UNSUPPORTED, "%lld tallying sweeps could take a tally from %lld past 2^31 - 1 (the device tallies "
+                "are int32): read the counts and reset them first", (long long)n_sweeps, (long long)g->tally_bound);
+    return NB_OK;
+}
+
 int nb_launch_gibbs_color(nb_graph *g, int color, int burnin, int sample_evidence, uint64_t seed, uint64_t epoch)
 {
     if (color < 0) NB_FAIL(NB_ERR_INVALID, "negative colour %d", color);
     if (color >= g->n_colors) return NB_OK;   // partitioned graphs: a colour this rank does not own
-    if (!burnin && epoch != g->last_tally_epoch) { g->tally_bound++; g->last_tally_epoch = epoch; }
+    if (!burnin) {
+        if (g->tally_launches.size() != (size_t)g->n_colors) g->tally_launches.assign((size_t)g->n_colors, 0);
+        int64_t &n = g->tally_launches[(size_t)color];
+        if (g->tally_base + n + 1 > INT32_MAX)
+            NB_FAIL(NB_ERR_UNSUPPORTED, "a tally of colour %d could pass 2^31 - 1 (the device tallies are int32): "
+                    "read the counts and reset them first", color);
+        n++;
+        g->tally_bound = std::max(g->tally_bound, g->tally_base + n);
+    }
     return g->value_bytes == 1 ? launch_gibbs_color_t<nb_val_t>(g, color, burnin, sample_evidence, seed, epoch)
                                : launch_gibbs_color_t<nb_val16_t>(g, color, burnin, sample_evidence, seed, epoch);
 }

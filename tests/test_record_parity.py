@@ -221,6 +221,31 @@ def test_record_energies_on_reference_golden_graphs(oracle, name):
     fg.clear()
 
 
+@pytest.mark.parametrize("name", ["wid_compact_top", "wid_wide", "wid_pair_top", "wid_pair_alias", "wid_fast",
+                                  "wid_cat"])
+def test_energies_at_the_weight_id_limits(oracle, name):
+    """Graphs whose weight ids sit at the limits of the record fields (test_sweep_replay's wid_*
+    graphs, tables of 2^20 to 2^22 + 512 weights): nb_potentials bit-exact, the record energies as
+    on the golden graphs."""
+    from test_sweep_replay import _spec
+    g, attrs, _ = _spec(name)
+    fg = _fg(g, **attrs)
+    og = _oracle_of(oracle, fg)
+    card = fg.variable["cardinality"].astype(np.int64)
+    ids = np.arange(len(card))
+    rng = np.random.default_rng(4)
+    n_rec = 0
+    for trial in range(3):
+        state = rng.integers(0, 1 << 30, len(card)) % card
+        w = rng.normal(size=len(fg.weight)).astype(np.float32).astype(np.float64)
+        _set_state(fg, og, state, evid_state=state[::-1] % card, weights=w)
+        for evid in (False, True):
+            assert np.array_equal(fg.potentials(evid_chain=evid), og.energies(ids, evid)), "potential() parity"
+            n_rec += sum(_check(fg, og, ids, evid=evid).values())
+    assert n_rec > 0
+    fg.clear()
+
+
 def test_fp32_inlined_weights_meet_the_energy_bar(oracle):
     """FAST quads carry the weight as fp32: with weights that are NOT fp32-representable the
     difference to the float64 oracle stays within 1e-5 of the variable's energies."""

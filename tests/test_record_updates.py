@@ -22,7 +22,7 @@ from test_sweep_replay import _graph, _spec   # noqa: E402
 
 SEED = 0x2468_ACE0_1357_9BDF
 SPECS = ["pair_uniform", "pair_records", "fast", "cat", "gen_boolean", "gen_cat_empty", "warp", "wide_headers",
-         "wide_card", "wide_card_thread"]
+         "wide_card", "wide_card_thread", "wid_wide", "wid_pair_top", "wid_pair_alias"]
 EDITS = ["query_to_evidence", "evidence_to_query", "initial_value", "fix", "unfix", "all"]
 
 
@@ -163,7 +163,9 @@ def _edit(kind, records, rng):
         var.append(dict(var_ids=ids, initialValue=x))
     if kind in ("fix", "all") and (fixed == 0).any():
         ids = np.nonzero(fixed == 0)[0]
-        ids = rng.choice(ids, max(1, len(ids) // 3), replace=False)
+        # and the largest free id a factor uses: the one at a record field's limit in the wid_* graphs
+        used = np.intersect1d(ids, records[2]["weightId"])
+        ids = np.union1d(rng.choice(ids, max(1, len(ids) // 3), replace=False), used[-1:])
         wts.append(dict(weight_ids=ids, isFixed=np.ones(len(ids), np.uint8)))
     if kind in ("unfix", "all"):
         ids = np.nonzero(fixed == 1)[0]

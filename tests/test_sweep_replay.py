@@ -336,6 +336,32 @@ def _spec(name):
     if name == "thread_row_long":    # one Boolean hub of > NB_META_MAX_ROWLEN words, as long as thread rows may be
         return (_graph(23, dt0_cards=(2,), feature_values=True, hub_rows=[(0, 2, 46000)]), {"warp_row_words": 1 << 20},
                 ("GEN",))
+    if name == "tally_chunks":       # > 3 x 2^18 tallies (test_tally_widths): Boolean record rows, cardinality-40 GEN rows
+        return _graph(30, nvar=60001, nfac=60000, dt0_cards=(2, 2, 40), max_arity=3), {}, ("PAIR", "FAST", "GEN")
+    # weight ids at the limits of the record fields (WID_COMPACT, WID_PAIR): fixtures above with their
+    # weights moved into large tables
+    if name in ("wid_compact_top", "wid_wide"):   # every row class; weight 0 tied to a tenth of the factors
+        g = _every_class()
+        n = len(g[0])
+        if name == "wid_compact_top":             # W = 2^20: the last compact id, headers stay compact
+            ids = _wid_targets(n, WID_COMPACT, WID_COMPACT, [WID_COMPACT - 1], 24)
+            return _move_weights(g, WID_COMPACT, ids, 24), {"warp_row_words": 40}, CLASS_NAMES[:5]
+        # W = 2^20 + 1: the table alone makes the headers wide, and only weight 0 sits at 2^20
+        ids = _wid_targets(n, WID_COMPACT + 1, WID_COMPACT, [WID_COMPACT, 0, WID_COMPACT - 1], 25)
+        return _move_weights(g, WID_COMPACT + 1, ids, 25), {"warp_row_words": 40}, CLASS_NAMES[:5]
+    if name == "wid_pair_top":       # pair_uniform's one weight at 2^22 - 1 (W = 2^22)
+        g, _, cls = _spec("pair_uniform")
+        return _move_weights(g, WID_PAIR, np.array([WID_PAIR - 1]), 26), {}, cls
+    if name == "wid_pair_alias":     # ids 0 and 2^22 (W = 2^22 + 1): the same 22-bit field, different weights
+        g = list(_grid(48))
+        g[2]["weightId"] = np.where(np.random.default_rng(27).random(len(g[2])) < 0.2, 1, 0)
+        g[0] = np.concatenate([g[0], g[0]])
+        g[0]["initialValue"][1] = -0.81
+        return _move_weights(tuple(g), WID_PAIR + 1, np.array([0, WID_PAIR]), 27), {}, ("PAIR", "FAST")
+    if name in ("wid_fast", "wid_cat"):   # FAST / CAT records with ids on both sides of 2^22 (W = 2^22 + 512)
+        g, attrs, cls = _spec(name[4:])
+        ids = _wid_targets(len(g[0]), WID_PAIR + 512, WID_PAIR, [WID_PAIR - 1, WID_PAIR, WID_PAIR + 511], 28)
+        return _move_weights(g, WID_PAIR + 512, ids, 28), attrs, cls
     # Large cells, sized from the SM count S to about twice the threshold of the branch they are for
     # (learn_branches; the grids' two colours hold n^2 / 2 rows each)
     S = _sms()
@@ -373,6 +399,66 @@ HUB_TASKS = [((0, 2), 2048), ((0, 2), 4500), ((0, 6), 2049), ((0, 6), 4161),
 # "card_band": dataType-0 and categorical cardinalities of a 1-byte graph, all above the lanes of a warp
 # but 5 (and above NB_CAT_MAX_CARD); 128 - 255 are values of uint8_t with the top bit set
 CARD_BAND = ((5, 40, 255), (33, 64, 127, 128, 200, 255))
+
+# Weight ids are packed into fixed-width fields: 20 bits in compact generic headers (a larger table
+# makes the whole graph take 2-word headers), 22 bits in the 8-byte pair records and the hoisted
+# tt2_common word (a row with a larger id is FAST instead of PAIR)
+WID_COMPACT, WID_PAIR = 1 << 20, 1 << 22
+
+
+def _union(*gs):
+    """Disjoint union of graphs (weight, variable, factor, fmap, domain_mask, edges)."""
+    w, v, f, m = [], [], [], []
+    nw = nv = nm = 0
+    for g in gs:
+        fac, fmap = g[2].copy(), g[3].copy()
+        fac["weightId"] += nw
+        fac["ftv_offset"] += nm
+        fmap["vid"] += nv
+        w.append(g[0])
+        v.append(g[1])
+        f.append(fac)
+        m.append(fmap)
+        nw, nv, nm = nw + len(g[0]), nv + len(g[1]), nm + len(fmap)
+    return np.concatenate(w), np.concatenate(v), np.concatenate(f), np.concatenate(m), np.zeros(nv, np.bool_), nm
+
+
+def _every_class():
+    """PAIR, FAST, CAT, GEN (categorical ones with MARK words) and WARP rows in one graph, with
+    weight 0 tied to a tenth of the factors, so that one weight id reaches every row class."""
+    g = _union(_spec("fast")[0], _spec("cat")[0], _spec("warp")[0], _spec("pair_records")[0])
+    g[2]["weightId"][np.random.default_rng(29).random(len(g[2])) < 0.1] = 0
+    return g
+
+
+def _wid_targets(n, W, limit, pinned, seed):
+    """n distinct weight ids below W: old id i < len(pinned) goes to pinned[i]; of the others, half go
+    to [limit - 4n, limit) and half to [limit, W) (all of them below `limit` when W <= limit)."""
+    rng = np.random.default_rng(seed)
+    pinned = np.asarray(pinned, np.int64)
+    k = n - len(pinned)
+    above = np.setdiff1d(np.arange(limit, W), pinned)
+    n_above = min(len(above), k // 2)
+    below = np.setdiff1d(np.arange(max(0, limit - 4 * n), min(limit, W)), pinned)
+    rest = np.concatenate([rng.choice(above, n_above, replace=False), rng.choice(below, k - n_above, replace=False)])
+    return np.concatenate([pinned, rng.permutation(rest)])
+
+
+def _move_weights(g, W, ids, seed):
+    """g with its weights moved into a table of W: old weight i becomes weight ids[i] (ids distinct, so
+    the tying, isFixed and initialValue of every used weight are kept).  The unused weights get random
+    values and flags: an incidence that reads a wrong id reads a different weight."""
+    from numbskull_b200.numbskulltypes import Weight
+    rng = np.random.default_rng(seed)
+    ids = np.asarray(ids, np.int64)
+    assert len(ids) == len(g[0]) and len(np.unique(ids)) == len(ids) and ids.max() < W
+    weight = np.zeros(W, Weight)
+    weight["isFixed"] = rng.random(W) < 0.2
+    weight["initialValue"] = rng.normal(0.0, 1.0, W)
+    weight[ids] = g[0]
+    factor = g[2].copy()
+    factor["weightId"] = ids[factor["weightId"]]
+    return (weight, g[1], factor) + tuple(g[3:])
 
 
 def _check_spec(r):
@@ -414,6 +500,47 @@ def _check_spec(r):
         fidx = np.repeat(np.arange(len(fac)), fac["arity"])
         hub = int(np.argmax(ninc))
         assert (1 + fac["arity"][fidx[fm["vid"] == hub]]).sum() > 131071 and r.evid[hub] == 0
+    if name.startswith("wid_"):
+        W = len(r.fg.weight)
+        fac = r.fg.factor
+        wid = fac["weightId"][np.repeat(np.arange(len(fac)), fac["arity"])].astype(np.int64)
+        top = np.zeros(r.V, np.int64)            # largest weight id among a row's incidences
+        np.maximum.at(top, fm["vid"], wid)
+
+        def rows_with(ids):
+            has = np.zeros(r.V, bool)
+            has[fm["vid"][np.isin(wid, ids)]] = True
+            return has & live
+
+        assert r.info["max_arity"] <= 31
+        if name in ("wid_compact_top", "wid_wide"):
+            at = WID_COMPACT - 1 if name == "wid_compact_top" else WID_COMPACT
+            assert W == at + 1 and r.info["wide_headers"] == int(name == "wid_wide")
+            for c in range(5):                   # the id at the limit in every row class
+                assert (rows_with([at]) & (r.cls == c)).any(), CLASS_NAMES[c]
+            gen = np.isin(r.cls, (O.GEN, O.WARP)) & (r.fg.variable["dataType"] == 1)
+            assert (rows_with([at]) & gen).any(), "no categorical generic row (MARK words) at the limit"
+        if name == "wid_pair_top":
+            assert W == WID_PAIR and (wid == WID_PAIR - 1).all() and (r.cls[live] == O.PAIR).all()
+            import numbskull_b200 as nb
+            ns = nb.NumbSkull(quiet=True)
+            ns.loadFactorGraph(*_spec("pair_uniform")[0])
+            fg = ns.factorGraphs[0]
+            quads = fg.device_info()["tt2_quads"]
+            fg.clear()
+            assert r.info["tt2_quads"] == quads, "the grid's slices are no longer uniform"
+        if name == "wid_pair_alias":             # a row reading id 2^22 cannot take a pair record
+            assert W == WID_PAIR + 1 and set(np.unique(wid)) == {0, WID_PAIR}
+            w = r.fg.weight
+            assert w["initialValue"][0] != w["initialValue"][WID_PAIR] and w["isFixed"][0] == w["isFixed"][WID_PAIR]
+            alias = rows_with([WID_PAIR])
+            assert alias.any() and (live & ~alias).any()
+            assert (r.cls[alias] == O.FAST).all() and (r.cls[live & ~alias] == O.PAIR).all()
+        if name in ("wid_fast", "wid_cat"):      # records on both sides of 2^22, and at W - 1
+            c = O.FAST if name == "wid_fast" else O.CAT
+            assert W == WID_PAIR + 512 and (rows_with([W - 1, WID_PAIR]) & (r.cls == c)).any()
+            assert ((top >= WID_PAIR) & (r.cls == c) & live).any() and ((top < WID_PAIR) & (r.cls == c) & live).any()
+            assert not ((top >= WID_PAIR) & (r.cls == O.PAIR) & live).any()
 
 
 def _sms():
@@ -661,7 +788,8 @@ def apply_update(w, G, cnt, reg, step, reg_param, trunc):
 # =========================================================================== GPU: Gibbs phases
 GIBBS_GRAPHS = ["pair_uniform", "pair_records", "fast", "gen_boolean", "gen_card", "gen_cat_empty", "cat", "warp",
                 "saturating", "wide_headers", "global_vid", "wide_card", "wide_card_thread", "hub_tasks", "hub_tasks_wide",
-                "card_band", "cat32", "thread_row_long"]
+                "card_band", "cat32", "thread_row_long", "wid_compact_top", "wid_wide", "wid_pair_top", "wid_pair_alias",
+                "wid_fast", "wid_cat"]
 
 
 @pytest.mark.gpu
@@ -701,7 +829,10 @@ def _whole_sweeps(name, sample_evidence):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name,mirror", [("fast", "-1"), ("fast", "0"), ("warp", "-1"), ("gen_cat_empty", "-1"),
-                                         ("wide_card", "-1"), ("hub_mirror", "0"), ("hub_tasks", "-1")])
+                                         ("wide_card", "-1"), ("hub_mirror", "0"), ("hub_tasks", "-1"),
+                                         ("wid_compact_top", "-1"), ("wid_wide", "-1"), ("wid_pair_top", "-1"),
+                                         ("wid_pair_top", "0"), ("wid_pair_alias", "-1"), ("wid_pair_alias", "0"),
+                                         ("wid_fast", "0"), ("wid_cat", "-1")])
 def test_whole_sweeps_replay_with_fan_out(name, mirror, monkeypatch):
     """nb_gibbs_sweeps with the row classes of a colour on concurrent streams (the default); "0"
     forces the bit-packed value mirror on (all-Boolean graphs)."""
@@ -733,6 +864,8 @@ LEARN = [  # graph, regularization, learn_non_evidence
     ("hub_tasks", 2, True), ("hub_tasks", 1, False), ("card_band", 1, True), ("card_band", 2, False),
     ("cat32", 2, True), ("cat32", 1, False),
     ("thread_row_long", 2, True), ("thread_row_long", 1, True),     # the hub's own gradient: learn_non_evidence
+    ("wid_compact_top", 2, True), ("wid_wide", 1, True), ("wid_wide", 2, False), ("wid_pair_top", 1, True),
+    ("wid_pair_alias", 2, True), ("wid_fast", 1, True), ("wid_cat", 2, True),
 ]
 
 
